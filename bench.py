@@ -5,6 +5,7 @@ audio-hours/sec at 1/2/4/8 B200).
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload sweep|filter|crnn|wavenet]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # CPU restatement of the reference path, host cores
+    python bench.py ... --dump-outputs DIR    # + what the last timed step computed, as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic 16 kHz int16 PCM.
 Default workload "sweep" (BASELINE config 5, one time-chunk of it): S streams x T s ->
@@ -217,6 +218,27 @@ def cpu_filter_rate(processes, seconds_per_stream):
     return processes * seconds_per_stream / 3600.0 / dt, dt
 
 
+DUMP_BUDGET = 60 << 20        # bytes of sampled rows over all dumped arrays (the rest stays far below 64 MB)
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes {name: tensor} as out_dir/<name>.npy: floating point as float32, integer counters as float64 (exact
+    below 2**53).  A [rows, ...] array larger than its share of DUMP_BUDGET keeps a fixed seeded sample of rows
+    (streams), whose indices go to out_dir/<name>_rows.npy, so that two builds are compared on the same rows."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BUDGET // max(1, sum(t.dim() >= 2 for t in outputs.values()))
+    for name, t in outputs.items():
+        a = t.detach()
+        if a.dim() >= 2 and a.numel() * 4 > share:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], max(1, share // (a[0].numel() * 4)), replace=False))
+            a = a[torch.as_tensor(rows, device=a.device)]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        a = a.cpu().numpy()
+        a = a.astype(np.float32) if np.issubdtype(a.dtype, np.floating) else a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def config_dict(args, S, N):
     names = {"sweep": "config5-step: FAR/FRR sweep time-chunk, filter->encode->detect, CRNN + WaveNet, hop-2 windows",
              "crnn": "filter->encode->detect, CRNN, hop-2 windows", "wavenet": "filter->encode->detect, WaveNet, hop-2 windows",
@@ -421,7 +443,11 @@ def main():
     ap.add_argument("--precision", default="tc", choices=["f32", "tc", "tc_fast"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip extra.configs / extra.parity (kernel work only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy; same arguments, same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         sys.stderr.write("bench.py: --warmup %d is below the 3 warm-up steps the timing rules require; using 3\n" % args.warmup)
         args.warmup = 3
@@ -518,9 +544,18 @@ def main():
     if rank == 0:
         sampler.start()
     stages = []
-    total_ms = timed(lambda: dev_step(stages), args.steps)
+    try:
+        total_ms = timed(lambda: dev_step(stages), args.steps)
+    finally:
+        clocks = sampler.stop() if rank == 0 else None       # never leave the nvidia-smi sampler running
     launches = sum(e.launch_count() for e in engines.values()) - launches0
-    clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before anything below reuses post / mel: posteriors and FAR / FRR counters per model (what
+        # wwb_sweep_wait hands back), or the mel features of the filter-only workload
+        outs = {m + "_posteriors": post[m] for m in models} if models else {"mel": mel}
+        for k, m in enumerate(models):
+            outs[m + "_far_edges"], outs[m + "_frr_accepts"] = last_counters["c"][2 * k:2 * k + 2]
+        dump_outputs(args.dump_outputs, outs)
     for marks in stages:
         names = ["filter"] + models + ["counts"]
         for i, nme in enumerate(names):

@@ -34,16 +34,29 @@ def _drive(rb, ops, log):
             log.append(("IndexError", str(e)))
 
 
+def _check_log(mine, theirs):
+    assert len(mine) == len(theirs)
+    for a, b in zip(mine, theirs):
+        assert a[0] == b[0]
+        if isinstance(a[1], np.ndarray):      # the data a read / read_all returned
+            assert isinstance(b[1], (list, np.ndarray))
+            np.testing.assert_array_equal(a[1].reshape(-1), np.asarray(b[1], np.float32).reshape(-1))
+        else:                                 # (is_empty, is_full) after the operation, or the IndexError message
+            assert tuple(a[1:]) == tuple(b[1:])
+
+
 def test_ring_buffer_matches_reference_semantics():
-    rng = np.random.default_rng(0)
-    ops = [("fill", 0.0)]
-    for _ in range(400):
-        k = rng.integers(0, 10)
-        ops.append([("write", float(rng.random())), ("write", float(rng.random())), ("read", None),
-                    ("read_all", None), ("seek", int(rng.integers(0, 3))), ("rewind", None), ("reset", None),
-                    ("write", float(rng.random())), ("write", float(rng.random())), ("fill", float(k))][k])
+    """The RingBuffer replays the stored operation log of tests/golden/ring_buffer_log.json
+    (make_golden_ring_buffer.py); with WWB_REFERENCE pointing at a checkout of the reference, its own
+    spokestack/ring_buffer.py is driven through the same operations as well."""
+    import json
+    from conftest import GOLDEN
+    g = json.load(open(os.path.join(GOLDEN, "ring_buffer_log.json")))
+    ops = [tuple(o) for o in g["ops"]]
     mine = []
-    _drive(RingBuffer(shape=[5]), ops, mine)
+    _drive(RingBuffer(shape=[g["capacity"]]), ops, mine)
+    assert len(ops) == 401 and sum(e[0] == "IndexError" for e in mine) > 0   # the log does exercise misuse
+    _check_log(mine, g["log"])
     # invariants that hold without the reference
     rb = RingBuffer(shape=[3])
     assert rb.capacity == 3 and rb.is_empty and not rb.is_full
@@ -58,22 +71,15 @@ def test_ring_buffer_matches_reference_semantics():
     assert rb.is_empty
     with pytest.raises(IndexError):
         rb.read()
-    path = os.path.join(REFERENCE, "spokestack", "ring_buffer.py")
-    if not os.path.exists(path):
+    if not REFERENCE:
         return
     import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_ring_buffer", path)
+    spec = importlib.util.spec_from_file_location("ref_ring_buffer", os.path.join(REFERENCE, "spokestack", "ring_buffer.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     theirs = []
-    _drive(mod.RingBuffer(shape=[5]), ops, theirs)
-    assert len(mine) == len(theirs)
-    for a, b in zip(mine, theirs):
-        assert a[0] == b[0]
-        if a[0] in ("read", "all"):
-            np.testing.assert_array_equal(a[1], b[1])
-        else:
-            assert a[1:] == b[1:]
+    _drive(mod.RingBuffer(shape=[g["capacity"]]), ops, theirs)
+    _check_log(mine, theirs)
 
 
 def test_shard_range_partitions():

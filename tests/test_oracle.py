@@ -8,7 +8,8 @@ import pytest
 from conftest import REFERENCE, WEIGHTS, load_weights
 from oracle import restated as R
 
-HAVE_REF = os.path.isdir(os.path.join(REFERENCE, "tf_lite_models"))
+HAVE_REF = bool(REFERENCE) and os.path.isdir(os.path.join(REFERENCE, "tf_lite_models"))
+NO_REF = "needs the reference's .tflite files: set WWB_REFERENCE to a checkout of the reference project"
 
 
 def test_known_answers(w_crnn, w_crnn_softmax, w_wavenet):
@@ -90,7 +91,7 @@ def test_window_counts():
     assert R.num_frames(511) == 0 and R.num_frames(512) == 1 and R.eval_windows(150, 151) == 0
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
+@pytest.mark.skipif(not HAVE_REF, reason=NO_REF)
 def test_restated_equals_literal():
     from oracle.tflite_literal import LiteralInterpreter
     ref = os.path.join(REFERENCE, "tf_lite_models")
@@ -112,7 +113,7 @@ def test_restated_equals_literal():
     np.testing.assert_allclose(R.mel_from_magnitude(mag, w), np.stack([f(m[None])[0][0] for m in mag]), atol=2e-6)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
+@pytest.mark.skipif(not HAVE_REF, reason=NO_REF)
 def test_committed_weights_match_reference_files():
     from wakeword_detection_b200 import weights as W
     for name, sub, typ in (("CRNN", "tf_lite_models/CRNN", "CRNN"), ("Wavenet", "tf_lite_models/Wavenet", "Wavenet")):
