@@ -209,6 +209,25 @@ int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm_dev, int64_t n_streams, int
                     const uint8_t* is_speech_dev, const uint8_t* is_active_dev, float pre_emphasis,
                     float threshold, float* post_out_dev, int32_t* n_post_out_dev,
                     uint8_t* trigger_out_dev, float* post_max_out_dev, void* stream);
+/* The same for a server's traffic: one chunk for each of n_ids streams, named by slot id, each
+ * chunk of its own length.  Only the named slots advance, and the work is proportional to n_ids,
+ * not to max_streams.
+ * ids_host int32 [n_ids] (host): distinct slots in [0, max_streams), any order.  A slot may appear
+ *   once per call: to feed a stream more samples, push again.
+ * len_host int32 [n_ids] (host): chunk lengths, each in [1, max_chunk_samples].
+ * pcm_dev int16: the chunks packed back to back in ids order (chunk i starts at sum(len[:i])).
+ * is_speech_dev / is_active_dev uint8 [n_ids], per entry (NULL = speech / inactive, as above).
+ * Outputs are per ENTRY i, not per slot: post_out [n_ids, max_frames] (NaN tail), n_post_out,
+ * trigger_out, post_max_out [n_ids].  Slots not named are not touched.
+ * The tables are checked before any device work; a rejected call changes no state (WWB_ERR_STATE:
+ * no wwb_stream_alloc, n_ids outside [1, max_streams], an id out of range or repeated, a length out
+ * of range, a filter-only ctx; WWB_ERR_ARG: NULL tables or PCM).  The library turns the lengths
+ * into offsets and copies ids and offsets to the device on `stream` through page-locked staging
+ * owned by ctx, so the call does not wait for earlier pushes. */
+int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                            const int16_t* pcm_dev, const uint8_t* is_speech_dev, const uint8_t* is_active_dev,
+                            float pre_emphasis, float threshold, float* post_out_dev, int32_t* n_post_out_dev,
+                            uint8_t* trigger_out_dev, float* post_max_out_dev, void* stream);
 int wwb_stream_max_frames(const wwb_ctx* ctx);
 /* WakewordTrigger.reset (:241-246) for the streams whose mask byte is non-zero (NULL = all). */
 int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask_dev, int64_t n_streams, void* stream);
@@ -231,6 +250,15 @@ int wwb_context_step(wwb_ctx* ctx, const int16_t* pcm_dev, int64_t n_streams, in
                      float* post_out_dev, int32_t* n_post_out_dev, float* post_max_out_dev,
                      uint8_t* is_speech_out_dev, uint8_t* is_active_out_dev,
                      uint8_t* activated_out_dev, uint8_t* deactivated_out_dev, void* stream);
+/* wwb_context_step for the slots named in ids_host, with the tables, their checks and the per-entry
+ * outputs of wwb_stream_push_indexed: one SpeechPipeline dispatch for each named slot, vad_raw_dev
+ * uint8 [n_ids] per entry (NULL = speech), every output per entry.  Slots not named are not
+ * touched.  Needs wwb_context_alloc (else WWB_ERR_STATE). */
+int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                             const int16_t* pcm_dev, const uint8_t* vad_raw_dev, float pre_emphasis, float threshold,
+                             float* post_out_dev, int32_t* n_post_out_dev, float* post_max_out_dev,
+                             uint8_t* is_speech_out_dev, uint8_t* is_active_out_dev,
+                             uint8_t* activated_out_dev, uint8_t* deactivated_out_dev, void* stream);
 /* all stages of all streams back to their initial state */
 int wwb_context_reset(wwb_ctx* ctx, void* stream);
 

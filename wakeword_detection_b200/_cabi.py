@@ -66,10 +66,14 @@ PROTOTYPES = {
     "wwb_eval_counts": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp, C.c_int, C.c_int, C.c_int, _vp, _vp]),
     "wwb_stream_alloc": (C.c_int, [_vp, _i64, _i64]),
     "wwb_stream_push": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp]),
+    "wwb_stream_push_indexed": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp,
+                                          _vp]),
     "wwb_stream_max_frames": (C.c_int, [_vp]),
     "wwb_stream_reset": (C.c_int, [_vp, _vp, _i64, _vp]),
     "wwb_context_alloc": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "wwb_context_step": (C.c_int, [_vp, _vp, _i64, _i64, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "wwb_context_step_indexed": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp,
+                                           _vp, _vp, _vp]),
     "wwb_context_reset": (C.c_int, [_vp, _vp]),
     "wwb_launch_count": (_i64, [_vp]),
     "wwb_debug_buffer": (C.c_int, [_vp, _vp]),
@@ -503,6 +507,45 @@ class Engine:
             post.data_ptr(), npost.data_ptr(), trig.data_ptr(), pmax.data_ptr(), self._stream()))
         return post, npost, trig, pmax
 
+    def _flags(self, a):
+        """optional per-stream uint8 flags -> device tensor (or None)"""
+        t = self.torch
+        if a is None:
+            return None
+        return a.to(self.device, t.uint8) if isinstance(a, t.Tensor) else self._dev(np.asarray(a), t.uint8)
+
+    def _indexed(self, ids, pcm_packed, lengths):
+        """host int32 id / length tables and the packed int16 PCM on the device, checked for shape (the library checks
+        the values)"""
+        ids = np.ascontiguousarray(ids, np.int32)
+        lengths = np.ascontiguousarray(lengths, np.int32)
+        if ids.ndim != 1 or lengths.shape != ids.shape:
+            raise ValueError("ids and lengths must be 1-D and of the same length")
+        x = self._dev(pcm_packed, self.torch.int16)
+        if x.dim() != 1 or x.numel() != int(lengths.astype(np.int64).sum()):
+            raise ValueError("pcm_packed must be 1-D with sum(lengths) = %d samples, got %s"
+                             % (int(lengths.astype(np.int64).sum()), list(x.shape)))
+        return ids, lengths, x
+
+    def stream_push_indexed(self, ids, pcm_packed, lengths, is_speech=None, is_active=None, pre_emphasis: float = 0.0,
+                            threshold: float = 0.5):
+        """One chunk for each slot in `ids` (distinct, any order), chunk i of lengths[i] samples, packed back to back in
+        `pcm_packed` (1-D int16) -> (post [n_ids, max_frames] (NaN = none), n_post [n_ids] int32, trigger [n_ids] uint8,
+        post_max [n_ids] float32) device tensors, one row per entry of `ids`.  is_speech / is_active per entry."""
+        t = self.torch
+        ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
+        K = ids.size
+        sp, ac = self._flags(is_speech), self._flags(is_active)
+        post = t.empty((K, self.stream_max_frames()), dtype=t.float32, device=self.device)
+        npost = t.empty((K,), dtype=t.int32, device=self.device)
+        trig = t.empty((K,), dtype=t.uint8, device=self.device)
+        pmax = t.empty((K,), dtype=t.float32, device=self.device)
+        self._check(self.lib.wwb_stream_push_indexed(
+            self.ctx, ids.ctypes.data, K, lengths.ctypes.data, x.data_ptr(), sp.data_ptr() if sp is not None else None,
+            ac.data_ptr() if ac is not None else None, float(pre_emphasis), float(threshold),
+            post.data_ptr(), npost.data_ptr(), trig.data_ptr(), pmax.data_ptr(), self._stream()))
+        return post, npost, trig, pmax
+
     def context_alloc(self, frame_width: int = 20, vad_rise_delay: int = 0, vad_fall_delay: int = 0, min_active: int = 500,
                       max_active: int = 5000) -> None:
         """Per-stream VAD debounce + ActivationTimeout state next to the streaming trigger (wwb_context_alloc)."""
@@ -531,6 +574,26 @@ class Engine:
             self.ctx, x.data_ptr(), S, n, raw.data_ptr() if raw is not None else None, float(pre_emphasis), float(threshold),
             out["post"].data_ptr(), out["n_post"].data_ptr(), out["post_max"].data_ptr(), out["is_speech"].data_ptr(),
             out["is_active"].data_ptr(), out["activated"].data_ptr(), out["deactivated"].data_ptr(), self._stream()))
+        return out
+
+    def context_step_indexed(self, ids, pcm_packed, lengths, vad_raw=None, pre_emphasis: float = 0.0,
+                             threshold: float = 0.5):
+        """context_step for the slots in `ids` only, tables and packing as in stream_push_indexed; vad_raw per entry ->
+        the dict of context_step with one row per entry of `ids`."""
+        t = self.torch
+        ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
+        K = ids.size
+        raw = self._flags(vad_raw)
+        out = {"post": t.empty((K, self.stream_max_frames()), dtype=t.float32, device=self.device),
+               "n_post": t.empty((K,), dtype=t.int32, device=self.device),
+               "post_max": t.empty((K,), dtype=t.float32, device=self.device)}
+        for k in ("is_speech", "is_active", "activated", "deactivated"):
+            out[k] = t.empty((K,), dtype=t.uint8, device=self.device)
+        self._check(self.lib.wwb_context_step_indexed(
+            self.ctx, ids.ctypes.data, K, lengths.ctypes.data, x.data_ptr(), raw.data_ptr() if raw is not None else None,
+            float(pre_emphasis), float(threshold), out["post"].data_ptr(), out["n_post"].data_ptr(),
+            out["post_max"].data_ptr(), out["is_speech"].data_ptr(), out["is_active"].data_ptr(),
+            out["activated"].data_ptr(), out["deactivated"].data_ptr(), self._stream()))
         return out
 
     def context_reset(self) -> None:

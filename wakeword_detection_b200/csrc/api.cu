@@ -313,6 +313,10 @@ int wwb_destroy(wwb_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaDeviceSynchronize();
   host_pipe_destroy(ctx);
+  for (int k = 0; k < 2; ++k) {
+    if (ctx->stage_host[k]) cudaFreeHost(ctx->stage_host[k]);
+    if (ctx->stage_done[k]) cudaEventDestroy(ctx->stage_done[k]);
+  }
   for (void* p : ctx->owned) cudaFree(p);
   for (int i = 0; i < 8; ++i)
     if (ctx->ws[i]) cudaFree(ctx->ws[i]);
@@ -432,11 +436,13 @@ int wwb_eval_counts(wwb_ctx* ctx, const float* post, const int64_t* seg_off, int
                             (cudaStream_t)stream);
 }
 
-// the explicit window lists of a streaming push over the first S streams (filled by the plan kernel, filter.cu)
-static WinMap stream_map(const wwb_ctx* ctx, int64_t S) {
+// the explicit window lists of a streaming push over S entries (filled by the plan kernel, filter.cu); entry i is stream
+// ids[i] of the ring (device table, NULL = i)
+static WinMap stream_map(const wwb_ctx* ctx, int64_t S, const int32_t* ids) {
   WinMap wm;
   memset(&wm, 0, sizeof(wm));
   wm.mel = ctx->st.mel_ring;
+  wm.stream_slot = ids;
   wm.win_stream = ctx->st.win_stream;
   wm.win_start = ctx->st.win_start;
   wm.n_win_dev = ctx->st.n_win;
@@ -476,12 +482,18 @@ int wwb_stream_alloc(wwb_ctx* ctx, int64_t max_streams, int64_t max_chunk) {
   if ((rc = dalloc(ctx, S, &s.win_slot))) return rc;
   if ((rc = dalloc(ctx, 1, &s.n_win))) return rc;
   if ((rc = dalloc(ctx, S * s.max_frames, &s.win_post))) return rc;
+  if ((rc = dalloc(ctx, 2 * S + 1, &s.tables))) return rc;
+  for (int k = 0; k < 2; ++k) {
+    if (!ctx->stage_host[k]) WWB_CUDA(ctx, cudaHostAlloc((void**)&ctx->stage_host[k], (2 * S + 1) * sizeof(int32_t), cudaHostAllocDefault));
+    if (!ctx->stage_done[k]) WWB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->stage_done[k], cudaEventDisableTiming));
+  }
+  ctx->id_seen.assign(S, 0);
   s.max_streams = max_streams;
   // Size the encoder's workspaces for the largest push now (a dry run over zero windows: n_win is 0 after dalloc), so that
   // wwb_stream_push cannot fail on an allocation AFTER its filter stage has consumed the chunk and advanced the
   // per-stream state.
   if (ctx->kind != WWB_MODEL_NONE) {
-    WinMap wm = stream_map(ctx, max_streams);
+    WinMap wm = stream_map(ctx, max_streams, nullptr);
     if ((rc = run_posteriors(ctx, wm, nullptr, nullptr, s.win_post, 0))) { s.max_streams = 0; return rc; }
     WWB_CUDA(ctx, cudaStreamSynchronize(0));
   }
@@ -489,6 +501,67 @@ int wwb_stream_alloc(wwb_ctx* ctx, int64_t max_streams, int64_t max_chunk) {
 }
 
 int wwb_stream_max_frames(const wwb_ctx* ctx) { return ctx ? ctx->st.max_frames : 0; }
+
+// filter -> encoder -> trigger bookkeeping over S entries (ids / off as in launch_stream_filter; NULL = dense push)
+static int stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids, const int32_t* off,
+                       const uint8_t* is_speech, const uint8_t* is_active, float a, float threshold, float* post_out,
+                       int32_t* n_post_out, uint8_t* trigger_out, float* post_max_out, cudaStream_t st) {
+  int rc = launch_stream_filter(ctx, pcm, S, n, ids, off, is_speech, is_active, a, st);
+  if (rc) return rc;
+  WinMap wm = stream_map(ctx, S, ids);
+  if ((rc = run_posteriors(ctx, wm, nullptr, nullptr, ctx->st.win_post, st))) return rc;
+  return launch_stream_finish(ctx, S, ids, is_speech, is_active, threshold, post_out, n_post_out, trigger_out,
+                              post_max_out, st);
+}
+
+// Checks the host tables of an indexed push (nothing is touched if they are rejected), then copies the slot ids and the
+// chunk offsets to st.tables on `st` through the next page-locked staging slot.  Waiting only for that slot's previous
+// copy keeps the host from blocking behind the push before.
+static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, const int16_t* pcm,
+                        cudaStream_t st) {
+  StreamState& s = ctx->st;
+  if (n_ids < 1 || n_ids > s.max_streams)
+    return fail(ctx, WWB_ERR_STATE, "n_ids %lld outside [1, %lld]", (long long)n_ids, (long long)s.max_streams);
+  if (!ids || !len) return fail(ctx, WWB_ERR_ARG, "NULL id or length table");
+  if (!pcm) return fail(ctx, WWB_ERR_ARG, "NULL pcm");
+  if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
+  int64_t marked = 0;
+  char why[160] = "";
+  for (int64_t i = 0; i < n_ids; ++i) {
+    const int32_t id = ids[i];
+    if (id < 0 || id >= s.max_streams) {
+      snprintf(why, sizeof(why), "id %d of entry %lld outside [0, %lld)", id, (long long)i, (long long)s.max_streams);
+      break;
+    }
+    if (ctx->id_seen[id]) {
+      snprintf(why, sizeof(why), "id %d named twice (entry %lld): push again to feed a stream more samples", id, (long long)i);
+      break;
+    }
+    ctx->id_seen[id] = 1;
+    ++marked;
+    if (len[i] < 1 || len[i] > s.max_chunk) {
+      snprintf(why, sizeof(why), "chunk of %d samples (entry %lld) outside [1, %lld]", len[i], (long long)i,
+               (long long)s.max_chunk);
+      break;
+    }
+  }
+  for (int64_t i = 0; i < marked; ++i) ctx->id_seen[ids[i]] = 0;
+  if (why[0]) return fail(ctx, WWB_ERR_STATE, "%s", why);
+  const int k = ctx->stage_next;
+  WWB_CUDA(ctx, cudaEventSynchronize(ctx->stage_done[k]));
+  int32_t* h = ctx->stage_host[k];
+  memcpy(h, ids, (size_t)n_ids * sizeof(int32_t));
+  int32_t at = 0;
+  for (int64_t i = 0; i < n_ids; ++i) {
+    h[n_ids + i] = at;
+    at += len[i];
+  }
+  h[2 * n_ids] = at;
+  WWB_CUDA(ctx, cudaMemcpyAsync(s.tables, h, (size_t)(2 * n_ids + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  WWB_CUDA(ctx, cudaEventRecord(ctx->stage_done[k], st));
+  ctx->stage_next = 1 - k;
+  return WWB_OK;
+}
 
 int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* is_speech,
                     const uint8_t* is_active, float a, float threshold, float* post_out, int32_t* n_post_out,
@@ -499,14 +572,24 @@ int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, cons
   if (n < 1 || n > ctx->st.max_chunk) return fail(ctx, WWB_ERR_STATE, "chunk of %lld samples exceeds capacity %lld", (long long)n, (long long)ctx->st.max_chunk);
   if (!pcm) return fail(ctx, WWB_ERR_ARG, "NULL pcm");
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = (cudaStream_t)stream;
   if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
-  int rc = launch_stream_filter(ctx, pcm, S, n, is_speech, is_active, a, st);
+  return stream_push(ctx, pcm, S, n, nullptr, nullptr, is_speech, is_active, a, threshold, post_out, n_post_out,
+                     trigger_out, post_max_out, (cudaStream_t)stream);
+}
+
+int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                            const int16_t* pcm, const uint8_t* is_speech, const uint8_t* is_active, float a,
+                            float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
+                            float* post_max_out, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = stage_tables(ctx, ids_host, n_ids, len_host, pcm, st);
   if (rc) return rc;
-  WinMap wm = stream_map(ctx, S);
-  if ((rc = run_posteriors(ctx, wm, nullptr, nullptr, ctx->st.win_post, st))) return rc;
-  return launch_stream_finish(ctx, S, is_speech, is_active, threshold, post_out, n_post_out, trigger_out,
-                              post_max_out, st);
+  const int32_t* ids = ctx->st.tables;
+  return stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, is_speech, is_active, a, threshold, post_out, n_post_out,
+                     trigger_out, post_max_out, st);
 }
 
 int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, void* stream) {
@@ -539,6 +622,8 @@ int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, i
   if ((rc = dalloc(ctx, S, &c.active_length))) return rc;
   if ((rc = dalloc(ctx, S, &c.t_is_speech))) return rc;
   if ((rc = dalloc(ctx, S, &c.trigger))) return rc;
+  if ((rc = dalloc(ctx, S, &c.e_is_speech))) return rc;
+  if ((rc = dalloc(ctx, S, &c.e_is_active))) return rc;
   c.max_streams = (int64_t)S;
   return WWB_OK;
 }
@@ -551,11 +636,31 @@ int wwb_context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, con
   if (S < 1 || S > ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "n_streams %lld exceeds capacity %lld", (long long)S, (long long)ctx->cs.max_streams);
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = launch_context_vad(ctx, vad_raw, S, st);
+  int rc = launch_context_vad(ctx, nullptr, vad_raw, S, st);
   if (rc) return rc;
-  if ((rc = wwb_stream_push(ctx, pcm, S, n, ctx->cs.is_speech, ctx->cs.is_active, a, threshold, post_out, n_post_out,
+  if ((rc = wwb_stream_push(ctx, pcm, S, n, ctx->cs.e_is_speech, ctx->cs.e_is_active, a, threshold, post_out, n_post_out,
                             ctx->cs.trigger, post_max_out, stream))) return rc;
-  return launch_context_timeout(ctx, ctx->cs.trigger, S, is_speech_out, is_active_out, activated_out, deactivated_out, st);
+  return launch_context_timeout(ctx, nullptr, ctx->cs.trigger, S, is_speech_out, is_active_out, activated_out,
+                                deactivated_out, st);
+}
+
+int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                             const int16_t* pcm, const uint8_t* vad_raw, float a, float threshold, float* post_out,
+                             int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
+                             uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  if (!ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = stage_tables(ctx, ids_host, n_ids, len_host, pcm, st);
+  if (rc) return rc;
+  const int32_t* ids = ctx->st.tables;
+  ContextState& c = ctx->cs;
+  if ((rc = launch_context_vad(ctx, ids, vad_raw, n_ids, st))) return rc;
+  if ((rc = stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, c.e_is_speech, c.e_is_active, a, threshold, post_out,
+                        n_post_out, c.trigger, post_max_out, st))) return rc;
+  return launch_context_timeout(ctx, ids, c.trigger, n_ids, is_speech_out, is_active_out, activated_out, deactivated_out,
+                                st);
 }
 
 int wwb_context_reset(wwb_ctx* ctx, void* stream) {

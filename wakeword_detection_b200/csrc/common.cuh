@@ -91,6 +91,9 @@ struct StreamState {
   int32_t* win_slot = nullptr;  // [S] first window slot of the stream in this push
   int32_t* n_win = nullptr;     // [1]
   float* win_post = nullptr;    // [S*max_frames]
+  // tables of an indexed push of n entries (wwb_stream_push_indexed): [0, n) slot of each entry, [n, 2n] exclusive
+  // prefix sum of the chunk lengths
+  int32_t* tables = nullptr;    // [2S+1]
 };
 
 // per-stream state of the pipeline stages around the trigger (context.cu)
@@ -105,6 +108,8 @@ struct ContextState {
   int32_t* active_length = nullptr;  // [S] ActivationTimeout._active_length
   uint8_t* t_is_speech = nullptr;    // [S] ActivationTimeout._is_speech
   uint8_t* trigger = nullptr;        // [S] scratch: the push's trigger output
+  uint8_t* e_is_speech = nullptr;    // [S] scratch: is_speech / is_active per entry of the push (context_vad_kernel)
+  uint8_t* e_is_active = nullptr;
 };
 
 }  // namespace wwb
@@ -131,6 +136,12 @@ struct wwb_ctx {
   int64_t launches = 0;
   void* debug_buf = nullptr;   // optional device buffer for kernel timeline dumps (wwb_debug_buffer)
   void* host_pipe = nullptr;   // host-buffer pipeline state (host_pipeline.cu), created on first use
+  // host side of the indexed-push tables: two page-locked staging slots laid out like st.tables, each guarded by an event
+  // recorded after its copy, and the duplicate-id marks (all 0 between calls)
+  int32_t* stage_host[2] = {};
+  cudaEvent_t stage_done[2] = {};
+  int stage_next = 0;
+  std::vector<uint8_t> id_seen;
   std::string err;
   std::vector<void*> owned;    // device allocations to free
 };
@@ -166,16 +177,18 @@ int workspace(wwb_ctx* ctx, int i, size_t bytes, void** out);
 int launch_filter(wwb_ctx* ctx, const void* pcm, int dtype, int64_t S, int64_t N, int64_t pitch,
                   float a, float* mel, cudaStream_t st);
 int launch_mel_from_mag(wwb_ctx* ctx, const float* mag, int64_t B, float* mel, cudaStream_t st);
-int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n,
+// Streaming kernels run over the entries i of a push.  ids (device, NULL = identity) names entry i's stream slot; off
+// (device, NULL = i * n) is where its chunk starts in pcm, of length off[i+1] - off[i].
+int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids, const int32_t* off,
                          const uint8_t* is_speech, const uint8_t* is_active, float a,
                          cudaStream_t st);
-int launch_stream_finish(wwb_ctx* ctx, int64_t S, const uint8_t* is_speech, const uint8_t* is_active,
+int launch_stream_finish(wwb_ctx* ctx, int64_t S, const int32_t* ids, const uint8_t* is_speech, const uint8_t* is_active,
                          float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
                          float* post_max_out, cudaStream_t st);
 int launch_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, cudaStream_t st);
-int launch_context_vad(wwb_ctx* ctx, const uint8_t* vad_raw, int64_t S, cudaStream_t st);
-int launch_context_timeout(wwb_ctx* ctx, const uint8_t* trigger, int64_t S, uint8_t* is_speech_out, uint8_t* is_active_out,
-                           uint8_t* activated_out, uint8_t* deactivated_out, cudaStream_t st);
+int launch_context_vad(wwb_ctx* ctx, const int32_t* ids, const uint8_t* vad_raw, int64_t S, cudaStream_t st);
+int launch_context_timeout(wwb_ctx* ctx, const int32_t* ids, const uint8_t* trigger, int64_t S, uint8_t* is_speech_out,
+                           uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out, cudaStream_t st);
 
 // window addressing shared by the encoders: window b reads rows
 //   mel + (stream(b)*ring + (start(b)+t) % ring) * 40,  t = 0..L-1
@@ -189,7 +202,8 @@ struct WinMap {
   int win_per_stream;         // regular grid: stream = b / wps, start = (b % wps)*hop
   int hop;
   int ring;                   // rows per stream
-  int64_t n_streams;          // streams behind `mel` (rows = n_streams * ring)
+  int64_t n_streams;          // streams the windows name (x0 of the WaveNet tensor-core path has n_streams * ring rows)
+  const int32_t* stream_slot; // optional: stream s of the windows is stream stream_slot[s] of `mel` (indexed pushes)
 };
 
 int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* det_out,
@@ -231,23 +245,8 @@ int launch_eval_counts(wwb_ctx* ctx, const float* post, const int64_t* seg_off, 
                        const double* thr, int n_thr, int mode, int smooth, int64_t* counts,
                        cudaStream_t st);
 
-__device__ __forceinline__ const float* win_row(const WinMap& wm, int64_t b, int t) {
-  int64_t s;
-  int start;
-  b += wm.b0;
-  if (wm.win_stream) {
-    s = wm.win_stream[b];
-    start = wm.win_start[b];
-  } else {
-    s = b / wm.win_per_stream;
-    start = (int)(b % wm.win_per_stream) * wm.hop;
-  }
-  int r = start + t;
-  if (r >= wm.ring) r -= wm.ring;
-  return wm.mel + (s * wm.ring + r) * (int64_t)kMel;
-}
-
-// win_row split in two: the window's stream / first mel row, and a row of that stream (ring-wrapped)
+// win_row split in two: the window's stream / first mel row, and a row of that stream (ring-wrapped).  win_origin
+// returns the stream as the windows name it (the compact entry of an indexed push); stream_row maps it to its slot.
 __device__ __forceinline__ void win_origin(const WinMap& wm, int64_t b, int64_t& s, int& start) {
   b += wm.b0;
   if (wm.win_stream) {
@@ -260,7 +259,15 @@ __device__ __forceinline__ void win_origin(const WinMap& wm, int64_t b, int64_t&
 }
 __device__ __forceinline__ const float* stream_row(const WinMap& wm, int64_t s, int r) {
   if (r >= wm.ring) r -= wm.ring;
+  if (wm.stream_slot) s = wm.stream_slot[s];
   return wm.mel + (s * wm.ring + r) * (int64_t)kMel;
+}
+
+__device__ __forceinline__ const float* win_row(const WinMap& wm, int64_t b, int t) {
+  int64_t s;
+  int start;
+  win_origin(wm, b, s, start);
+  return stream_row(wm, s, start + t);
 }
 
 }  // namespace wwb

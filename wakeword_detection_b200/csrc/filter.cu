@@ -325,10 +325,14 @@ int launch_filter(wwb_ctx* ctx, const void* pcm, int dtype, int64_t S, int64_t N
 //          into the stream's ring; with one new frame per stream and push (hop 1, BASELINE config 4) 16 streams share a
 //          CTA instead of one CTA per stream
 //   tail   (one CTA per stream)  unread PCM tail, previous sample, ring head
+// Each kernel runs over the entries i of the push: per-stream state is at slot ids[i], the chunk at pcm + off[i], and the
+// per-push scratch (n_new, win_slot, window lists) and every output at i.  A dense push passes ids = off = NULL.
 struct StreamFilterParams {
   const int16_t* pcm;
   int64_t n;
-  int64_t n_streams;
+  int64_t n_streams;      // entries
+  const int32_t* ids;     // [n_streams] slot of entry i (NULL = i)
+  const int32_t* off;     // [n_streams + 1] chunk offsets (NULL = i * n)
   const uint8_t* is_speech;
   const uint8_t* is_active;
   float a;
@@ -342,27 +346,43 @@ struct StreamFilterParams {
 
 __device__ __forceinline__ int stream_total_frames(int total) { return total >= kFFT ? (total - kFFT) / kHop + 1 : 0; }
 
+__device__ __forceinline__ int64_t entry_slot(const int32_t* ids, int64_t i) { return ids ? (int64_t)ids[i] : i; }
+
+// entry i's chunk and its length
+__device__ __forceinline__ const int16_t* entry_chunk(const StreamFilterParams& P, int64_t i, int& n) {
+  if (P.off) {
+    const int o = P.off[i];
+    n = P.off[i + 1] - o;
+    return P.pcm + o;
+  }
+  n = (int)P.n;
+  return P.pcm + i * P.n;
+}
+
 __global__ void __launch_bounds__(128) stream_plan_kernel(const StreamFilterParams P) {
   const StreamState& S = P.st;
-  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= P.n_streams) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n_streams) return;
+  const int64_t s = entry_slot(P.ids, i);
   int n_new = 0;
-  const bool active = P.is_active && P.is_active[s];   // "if not context.is_active: self._sample(...)" (:139-140)
-  const bool speech = P.is_speech ? (P.is_speech[s] != 0) : true;
+  const bool active = P.is_active && P.is_active[i];   // "if not context.is_active: self._sample(...)" (:139-140)
+  const bool speech = P.is_speech ? (P.is_speech[i] != 0) : true;
   if (!active && speech) {
-    const int n_frames = stream_total_frames(S.n_pending[s] + (int)P.n);
+    int n;
+    entry_chunk(P, i, n);
+    const int n_frames = stream_total_frames(S.n_pending[s] + n);
     if (n_frames > 0) {
       const int head = S.ring_head[s];
       const int slot = atomicAdd(S.n_win, n_frames);
       for (int q = 0; q < n_frames; ++q) {
-        S.win_stream[slot + q] = (int32_t)s;
+        S.win_stream[slot + q] = (int32_t)i;
         S.win_start[slot + q] = (head + 1 + q) % S.ring;
       }
-      S.win_slot[s] = slot;
+      S.win_slot[i] = slot;
       n_new = n_frames;
     }
   }
-  S.n_new[s] = n_new;
+  S.n_new[i] = n_new;
 }
 
 __global__ void __launch_bounds__(F_THREADS, 1) stream_frames_kernel(const StreamFilterParams P) {
@@ -381,15 +401,17 @@ __global__ void __launch_bounds__(F_THREADS, 1) stream_frames_kernel(const Strea
   // a warp takes two items (stream, frame) per iteration, one per half
   for (int64_t it0 = ((int64_t)blockIdx.x * F_WARPS + warp) * 2; it0 < n_items; it0 += (int64_t)gridDim.x * F_WARPS * 2) {
     const int64_t it = it0 + h;
-    const int64_t s = it < n_items ? it / S.max_frames : 0;
-    const int q = (int)(it - s * S.max_frames);
-    const bool live = it < n_items && q < S.n_new[s];
+    const int64_t e = it < n_items ? it / S.max_frames : 0;   // entry
+    const int q = (int)(it - e * S.max_frames);
+    const bool live = it < n_items && q < S.n_new[e];
+    const int64_t s = live ? entry_slot(P.ids, e) : 0;
     float* frame = ws.ring + h * kFFT;   // the ring doubles as two frame buffers
     __syncwarp();
     if (live) {
       const int np = S.n_pending[s];
       const float* pend = S.pending + s * S.pend_cap;
-      const int16_t* chunk = P.pcm + s * P.n;
+      int n;
+      const int16_t* chunk = entry_chunk(P, e, n);
       const float prev = S.prev_sample[s];
       for (int i = j; i < kFFT; i += 16) {
         const int p = q * kHop + i;
@@ -424,15 +446,17 @@ __global__ void __launch_bounds__(F_THREADS, 1) stream_frames_kernel(const Strea
 
 __global__ void __launch_bounds__(128) stream_tail_kernel(const StreamFilterParams P) {
   const StreamState& S = P.st;
-  const int64_t s = blockIdx.x;
+  const int64_t i = blockIdx.x;
   const int tid = threadIdx.x;
-  if (P.is_active && P.is_active[s]) return;
+  if (P.is_active && P.is_active[i]) return;
+  const int64_t s = entry_slot(P.ids, i);
+  int n;
+  const int16_t* chunk = entry_chunk(P, i, n);
   const int np = S.n_pending[s];
-  const int total = np + (int)P.n;
+  const int total = np + n;
   const int n_frames = stream_total_frames(total);
   float* pend = S.pending + s * S.pend_cap;
   const float prev = S.prev_sample[s];
-  const int16_t* chunk = P.pcm + s * P.n;
   // new pending tail = samples [n_frames*hop, total) (< 512 + 160); moved through registers (overlapping ranges)
   const int keep0 = n_frames * kHop;
   const int keep = total - keep0;
@@ -456,8 +480,8 @@ __global__ void __launch_bounds__(128) stream_tail_kernel(const StreamFilterPara
   for (int i = tid; i < keep && c < 6; i += 128, ++c) pend[i] = tmp[c];
   if (tid == 0) {
     S.n_pending[s] = keep;
-    if (P.n > 0) S.prev_sample[s] = pcm_to_float(chunk[P.n - 1]);
-    if (S.n_new[s] > 0) S.ring_head[s] = (S.ring_head[s] + S.n_new[s]) % S.ring;
+    if (n > 0) S.prev_sample[s] = pcm_to_float(chunk[n - 1]);
+    if (S.n_new[i] > 0) S.ring_head[s] = (S.ring_head[s] + S.n_new[i]) % S.ring;
   }
 }
 
@@ -466,27 +490,29 @@ __global__ void __launch_bounds__(128) stream_tail_kernel(const StreamFilterPara
 struct StreamFinishParams {
   StreamState st;
   int L;
+  const int32_t* ids;     // [n_streams] slot of entry i (NULL = i)
   const uint8_t* is_speech;
   const uint8_t* is_active;
   float threshold;
-  float* post_out;        // [S, max_frames]
-  int32_t* n_post_out;    // [S]
-  uint8_t* trigger_out;   // [S]
-  float* post_max_out;    // [S]
-  int64_t n_streams;
+  float* post_out;        // [entries, max_frames]
+  int32_t* n_post_out;    // [entries]
+  uint8_t* trigger_out;   // [entries]
+  float* post_max_out;    // [entries]
+  int64_t n_streams;      // entries
 };
 
 __global__ void stream_finish_kernel(const StreamFinishParams P) {
   const StreamState& S = P.st;
-  const int64_t s = blockIdx.x;
-  if (s >= P.n_streams) return;
+  const int64_t i = blockIdx.x;
+  if (i >= P.n_streams) return;
+  const int64_t s = entry_slot(P.ids, i);
   __shared__ int do_reset;
   if (threadIdx.x == 0) {
-    const int n = S.n_new[s];
-    const int slot = n > 0 ? S.win_slot[s] : 0;
+    const int n = S.n_new[i];
+    const int slot = n > 0 ? S.win_slot[i] : 0;
     float pm = S.post_max[s];
     bool trig = false;
-    const bool active = P.is_active && P.is_active[s];
+    const bool active = P.is_active && P.is_active[i];
     for (int q = 0; q < S.max_frames; ++q) {
       float p = nanf("");
       if (q < n) {
@@ -494,12 +520,12 @@ __global__ void stream_finish_kernel(const StreamFinishParams P) {
         if (p > pm) pm = p;
         if (p > P.threshold && !active) trig = true;
       }
-      if (P.post_out) P.post_out[s * S.max_frames + q] = p;
+      if (P.post_out) P.post_out[i * S.max_frames + q] = p;
     }
-    if (P.n_post_out) P.n_post_out[s] = n;
-    if (P.trigger_out) P.trigger_out[s] = trig ? 1 : 0;
-    if (P.post_max_out) P.post_max_out[s] = pm;
-    const bool speech = P.is_speech ? (P.is_speech[s] != 0) : true;
+    if (P.n_post_out) P.n_post_out[i] = n;
+    if (P.trigger_out) P.trigger_out[i] = trig ? 1 : 0;
+    if (P.post_max_out) P.post_max_out[i] = pm;
+    const bool speech = P.is_speech ? (P.is_speech[i] != 0) : true;
     const bool fall = S.was_speech[s] && !speech;
     S.was_speech[s] = speech ? 1 : 0;
     S.post_max[s] = fall ? 0.0f : pm;
@@ -558,11 +584,11 @@ int launch_mel_from_mag(wwb_ctx* ctx, const float* mag, int64_t B, float* mel, c
   return WWB_OK;
 }
 
-int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n,
+int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids, const int32_t* off,
                          const uint8_t* is_speech, const uint8_t* is_active, float a,
                          cudaStream_t st) {
   StreamFilterParams P;
-  P.pcm = pcm; P.n = n; P.n_streams = S; P.is_speech = is_speech; P.is_active = is_active; P.a = a;
+  P.pcm = pcm; P.n = n; P.n_streams = S; P.ids = ids; P.off = off; P.is_speech = is_speech; P.is_active = is_active; P.a = a;
   P.st = ctx->st; P.L = ctx->L;
   P.hann_half = ctx->hann; P.tw256 = ctx->tw256; P.tw512 = ctx->tw512;
   P.mp = mel_params(ctx);
@@ -580,11 +606,11 @@ int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n,
   return WWB_OK;
 }
 
-int launch_stream_finish(wwb_ctx* ctx, int64_t S, const uint8_t* is_speech, const uint8_t* is_active,
+int launch_stream_finish(wwb_ctx* ctx, int64_t S, const int32_t* ids, const uint8_t* is_speech, const uint8_t* is_active,
                          float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
                          float* post_max_out, cudaStream_t st) {
   StreamFinishParams P;
-  P.st = ctx->st; P.L = ctx->L; P.is_speech = is_speech; P.is_active = is_active;
+  P.st = ctx->st; P.L = ctx->L; P.ids = ids; P.is_speech = is_speech; P.is_active = is_active;
   P.threshold = threshold; P.post_out = post_out; P.n_post_out = n_post_out;
   P.trigger_out = trigger_out; P.post_max_out = post_max_out; P.n_streams = S;
   stream_finish_kernel<<<(unsigned)S, 128, 0, st>>>(P);

@@ -773,9 +773,11 @@ std::vector<unsigned char> wavenet_pack_head(const float* bn_mul0, const float* 
 
 // Input layer (Wavenet/encode.tflite op 0: 1x1 conv 40 -> 16 + ReLU, SURVEY.md Appendix A3) once per mel row, fp32:
 // x0[row, c] = ReLU(b[c] + sum_k w[k][c] * mel[row, k]).  4 threads per row, 4 channels each; stored as 4 column planes
-// of n_rows float4 (the rows a warp of the main kernel reads are a handful of consecutive frames).
-__global__ void __launch_bounds__(256) wn_input_kernel(const float* __restrict__ mel, const float* __restrict__ w_kc,
-                                                       const float* __restrict__ b, float* __restrict__ x0, int64_t n_rows) {
+// of n_rows float4 (the rows a warp of the main kernel reads are a handful of consecutive frames).  With a stream_slot
+// table (indexed push), row s * ring + r of x0 is row r of stream stream_slot[s] of mel: x0 stays compact.
+__global__ void __launch_bounds__(256) wn_input_kernel(const float* __restrict__ mel, const int32_t* __restrict__ stream_slot,
+                                                       int ring, const float* __restrict__ w_kc, const float* __restrict__ b,
+                                                       float* __restrict__ x0, int64_t n_rows) {
   __shared__ float ws[kMel * 16];
   __shared__ float bs[16];
   for (int i = threadIdx.x; i < kMel * 16; i += 256) ws[i] = w_kc[i];
@@ -783,7 +785,12 @@ __global__ void __launch_bounds__(256) wn_input_kernel(const float* __restrict__
   __syncthreads();
   const int c4 = threadIdx.x & 3;
   for (int64_t row = (int64_t)blockIdx.x * 64 + (threadIdx.x >> 2); row < n_rows; row += (int64_t)gridDim.x * 64) {
-    const float4* m4 = reinterpret_cast<const float4*>(mel + row * kMel);
+    int64_t src = row;
+    if (stream_slot) {   // streaming rings: n_rows < 2^31 (wwb_stream_alloc bounds streams x frames)
+      const int s = (int)row / ring;
+      src = (int64_t)stream_slot[s] * ring + ((int)row - s * ring);
+    }
+    const float4* m4 = reinterpret_cast<const float4*>(mel + src * kMel);
     float a0 = bs[4 * c4], a1 = bs[4 * c4 + 1], a2 = bs[4 * c4 + 2], a3 = bs[4 * c4 + 3];
 #pragma unroll
     for (int k4 = 0; k4 < kMel / 4; ++k4) {
@@ -836,7 +843,7 @@ int wavenet_tc_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float*
   int rc = workspace(ctx, 1, (size_t)std::max<int64_t>(n_rows, 1) * 16 * sizeof(float), &x0);
   if (rc) return rc;
   wn_input_kernel<<<(unsigned)std::min<int64_t>((n_rows + 63) / 64, (int64_t)ctx->sm_count * 8), 256, 0, st>>>(
-      wm.mel, ctx->wn.in_w, ctx->wn.in_b, (float*)x0, n_rows);
+      wm.mel, wm.stream_slot, wm.ring, ctx->wn.in_w, ctx->wn.in_b, (float*)x0, n_rows);
   WWB_CHECK_LAUNCH(ctx);
   WnTcParams P;
   memset(&P, 0, sizeof(P));

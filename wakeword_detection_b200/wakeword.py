@@ -20,13 +20,29 @@ from .ring_buffer import RingBuffer
 _LOG = logging.getLogger(__name__)
 
 
+def _pack(chunks):
+    """list of 1-D int16 chunks (numpy arrays or torch tensors) -> (one packed 1-D array or tensor, lengths)"""
+    if any(len(c.shape) != 1 for c in chunks):
+        raise ValueError("every chunk must be 1-D")
+    lengths = [int(c.shape[0]) for c in chunks]
+    if all(isinstance(c, np.ndarray) for c in chunks):
+        return np.concatenate([np.zeros(0, np.int16)] + [c.astype(np.int16, copy=False) for c in chunks]), lengths
+    import torch
+    dev = next(c.device for c in chunks if isinstance(c, torch.Tensor))
+    return torch.cat([torch.as_tensor(c).to(dev, torch.int16) for c in chunks]), lengths
+
+
 class MultiStreamTrigger:
     """S independent WakewordTrigger state machines advanced by one call.
 
     push(pcm[S, n] int16, is_speech[S], is_active[S]) -> dict of device tensors:
       post [S, max_frames] (NaN where no frame was analysed), n_post [S], trigger [S],
       post_max [S].  The caller owns the `is_active` latch exactly like
-      SpeechContext.is_active in the reference (:139,:236-239)."""
+      SpeechContext.is_active in the reference (:139,:236-239).
+
+    push_streams(ids, chunks, is_speech, is_active) advances only the slots in `ids` (distinct, any order), each
+    by its own chunk (a list of 1-D int16 arrays or tensors, any lengths up to chunk_samples): the way a server
+    receives audio.  Same dict, one row per entry of `ids`."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, chunk_samples: int = 320,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, device: int = 0,
@@ -43,6 +59,12 @@ class MultiStreamTrigger:
                                                            self.threshold)
         return {"post": post, "n_post": n_post, "trigger": trig, "post_max": pmax}
 
+    def push_streams(self, ids, chunks, is_speech=None, is_active=None):
+        pcm, lengths = _pack(chunks)
+        post, n_post, trig, pmax = self.engine.stream_push_indexed(ids, pcm, lengths, is_speech, is_active,
+                                                                   self.pre_emphasis, self.threshold)
+        return {"post": post, "n_post": n_post, "trigger": trig, "post_max": pmax}
+
     def reset(self, mask=None) -> None:
         self.engine.stream_reset(mask)
 
@@ -57,7 +79,8 @@ class MultiStreamPipeline:
     input (the webrtcvad C extension is outside the path).
 
     step(pcm[S, n] int16, vad_raw[S]) -> dict of device tensors: post, n_post, post_max, is_speech, is_active,
-    activated, deactivated."""
+    activated, deactivated.  step_streams(ids, frames, vad_raw) dispatches only the slots in `ids`, each with its own
+    frame (list of 1-D int16 arrays or tensors); same dict, one row per entry of `ids`."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, frame_width: int = 20, sample_rate: int = 16000,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, vad_rise_delay: int = 0,
@@ -74,6 +97,10 @@ class MultiStreamPipeline:
 
     def step(self, pcm, vad_raw=None):
         return self.engine.context_step(pcm, vad_raw, self.pre_emphasis, self.threshold)
+
+    def step_streams(self, ids, frames, vad_raw=None):
+        pcm, lengths = _pack(frames)
+        return self.engine.context_step_indexed(ids, pcm, lengths, vad_raw, self.pre_emphasis, self.threshold)
 
     def reset(self) -> None:
         self.engine.context_reset()
