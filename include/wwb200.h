@@ -262,6 +262,64 @@ int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_id
 /* all stages of all streams back to their initial state */
 int wwb_context_reset(wwb_ctx* ctx, void* stream);
 
+/* ---- stream state records: a stream's state out of its slot and back, to park an idle session, move it to another
+ * slot, context or GPU, or rewind it.  One record per stream, of wwb_stream_state_bytes(ctx) bytes; its layout does not
+ * depend on the capacity, max_chunk, precision or device of the ctx that wrote it:
+ *   wwb_stream_state_header                       48 bytes
+ *   float pending[WWB_STREAM_STATE_PENDING]       the pre-emphasised samples not yet consumed (WakewordTrigger's sample
+ *                                                 ring); entries n_pending and beyond are 0
+ *   float mel[mel_length][40]                     the frame window (frame_window), oldest row first; all 0 for a stream
+ *                                                 never pushed or just reset
+ * Record size: 48 + 4*512 + 160*mel_length bytes (26 256 for CRNN, 31 216 for WaveNet). */
+#define WWB_STREAM_STATE_MAGIC 0x53425757u /* "WWBS" */
+#define WWB_STREAM_STATE_VERSION 1         /* of the record layout (not WWB_VERSION) */
+#define WWB_STREAM_STATE_PENDING 512
+#define WWB_STREAM_STATE_PIPELINE 1u /* flags bit 0: the pipeline fields hold state (wwb_context_alloc) */
+typedef struct {
+  uint32_t magic;       /* WWB_STREAM_STATE_MAGIC */
+  uint16_t version;     /* WWB_STREAM_STATE_VERSION */
+  uint16_t flags;       /* WWB_STREAM_STATE_PIPELINE or 0; other bits 0 */
+  int32_t kind;         /* WWB_MODEL_* of the ctx that wrote it */
+  int32_t mel_length;   /* L */
+  int32_t n_pending;    /* [0, 511] */
+  float prev_sample;    /* last sample consumed, raw (int16 / 32767, clipped): the pre-emphasis state */
+  float post_max;       /* running posterior maximum */
+  uint8_t was_speech;   /* is_speech of the stream's last push */
+  uint8_t is_speech;    /* pipeline: SpeechContext.is_speech (VAD debounce output) */
+  uint8_t is_active;    /* pipeline: SpeechContext.is_active */
+  uint8_t t_is_speech;  /* pipeline: ActivationTimeout._is_speech */
+  int32_t run_value;    /* pipeline: VoiceActivityDetector._run_value */
+  int32_t run_length;   /* pipeline: VoiceActivityDetector._run_length */
+  int32_t active_length;/* pipeline: ActivationTimeout._active_length */
+  uint32_t reserved;    /* 0 */
+} wwb_stream_state_header;
+/* wwb_stream_import's reason codes (status_dev[1]) */
+enum {
+  WWB_RECORD_OK = 0,
+  WWB_RECORD_BAD_MAGIC = 1,
+  WWB_RECORD_BAD_VERSION = 2,
+  WWB_RECORD_BAD_FLAGS = 3,   /* an unknown flag bit */
+  WWB_RECORD_BAD_KIND = 4,    /* written by a ctx of another model kind */
+  WWB_RECORD_BAD_LENGTH = 5,  /* mel_length differs from this ctx's */
+  WWB_RECORD_BAD_PENDING = 6  /* n_pending outside [0, 511] */
+};
+/* record size in bytes; 0 without wwb_stream_alloc or on a filter-only ctx */
+int64_t wwb_stream_state_bytes(const wwb_ctx* ctx);
+/* Gathers the state of the slots named in ids_host (host table, the rules of wwb_stream_push_indexed: distinct, in
+ * [0, max_streams), 1 <= n_ids <= max_streams) into records_dev (16-byte aligned): entry i's record at
+ * records_dev + i * wwb_stream_state_bytes(ctx).  Stream-ordered like the pushes; the slots are not modified.  Without
+ * wwb_context_alloc the flags are 0 and the pipeline fields 0.  A rejected call changes nothing (WWB_ERR_STATE: the id
+ * checks of the pushes, no wwb_stream_alloc, a filter-only ctx; WWB_ERR_ARG: NULL or misaligned buffers). */
+int wwb_stream_export(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, void* records_dev, void* stream);
+/* Scatters n_ids records (as written by wwb_stream_export, on this ctx's device) into the slots named in ids_host, all or
+ * nothing: every record's magic, version, flags, kind, mel_length and n_pending are checked on the device first, and
+ * status_dev int32[2] receives {0, 0} when the records were applied, else {1 + the lowest bad entry, WWB_RECORD_*} and no
+ * slot is touched.  An applied record's window becomes ring rows 0..L-1 of its slot (the rest of the ring is zeroed); the
+ * pipeline fields are applied when the ctx has pipeline state, and set to their initial values there when the record has
+ * none.  The pipeline's delays are per ctx and not carried.  Host-side checks as wwb_stream_export. */
+int wwb_stream_import(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const void* records_dev, int32_t* status_dev,
+                      void* stream);
+
 /* number of kernels this library has launched on ctx since creation (bench accounting) */
 int64_t wwb_launch_count(const wwb_ctx* ctx);
 /* development aid: device buffer (>= 8 KB, zeroed) that instrumented kernels fill with

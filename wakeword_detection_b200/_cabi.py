@@ -75,9 +75,52 @@ PROTOTYPES = {
     "wwb_context_step_indexed": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp,
                                            _vp, _vp, _vp]),
     "wwb_context_reset": (C.c_int, [_vp, _vp]),
+    "wwb_stream_state_bytes": (_i64, [_vp]),
+    "wwb_stream_export": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
+    "wwb_stream_import": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),
     "wwb_launch_count": (_i64, [_vp]),
     "wwb_debug_buffer": (C.c_int, [_vp, _vp]),
 }
+
+# ---- stream state records (include/wwb200.h, wwb_stream_export / wwb_stream_import): the only Python code that knows
+# the layout.  A record is the 48-byte header, the pending samples and the [L, 40] frame window, oldest row first.
+STREAM_STATE_MAGIC = 0x53425757      # "WWBS"
+STREAM_STATE_VERSION = 1
+STREAM_STATE_PENDING = 512
+STREAM_STATE_PIPELINE = 1            # flags bit 0: the pipeline fields hold state
+STREAM_STATE_HEADER = np.dtype([
+    ("magic", "<u4"), ("version", "<u2"), ("flags", "<u2"), ("kind", "<i4"), ("mel_length", "<i4"),
+    ("n_pending", "<i4"), ("prev_sample", "<f4"), ("post_max", "<f4"),
+    ("was_speech", "u1"), ("is_speech", "u1"), ("is_active", "u1"), ("t_is_speech", "u1"),
+    ("run_value", "<i4"), ("run_length", "<i4"), ("active_length", "<i4"), ("reserved", "<u4"),
+])
+# wwb_stream_import's reason codes (WWB_RECORD_*)
+RECORD_REASONS = {1: "bad magic", 2: "unsupported record version", 3: "unknown flag bits",
+                  4: "written by a context of another model kind", 5: "mel_length does not match this context",
+                  6: "n_pending outside [0, 511]"}
+
+
+def stream_state_dtype(L: int) -> np.dtype:
+    """numpy dtype of one whole record of a model with an L-frame window"""
+    return np.dtype([("header", STREAM_STATE_HEADER), ("pending", "<f4", (STREAM_STATE_PENDING,)),
+                     ("mel", "<f4", (int(L), 40))])
+
+
+def decode_stream_state(records, L: int) -> Dict[str, np.ndarray]:
+    """records (uint8 [n, bytes] or [bytes]; numpy or a torch tensor on any device) -> dict of per-entry arrays: every
+    header field, `pending` [n, 512] and `mel` [n, L, 40]"""
+    if not isinstance(records, np.ndarray):
+        records = records.detach().cpu().numpy()
+    dt = stream_state_dtype(L)
+    raw = np.ascontiguousarray(records).view(np.uint8).reshape(-1)
+    if raw.size % dt.itemsize:
+        raise ValueError("%d bytes are not a whole number of %d-byte records" % (raw.size, dt.itemsize))
+    rec = raw.view(dt)
+    out = {k: rec["header"][k].copy() for k in STREAM_STATE_HEADER.names}
+    out["pending"] = rec["pending"].copy()
+    out["mel"] = rec["mel"].copy()
+    return out
+
 
 _lib = None
 
@@ -598,6 +641,47 @@ class Engine:
 
     def context_reset(self) -> None:
         self._check(self.lib.wwb_context_reset(self.ctx, self._stream()))
+
+    def stream_state_bytes(self) -> int:
+        """size of one stream state record (0 without stream_alloc or on a filter-only context)"""
+        return int(self.lib.wwb_stream_state_bytes(self.ctx))
+
+    def _state_ids(self, ids) -> np.ndarray:
+        ids = np.ascontiguousarray(ids, np.int32)
+        if ids.ndim != 1:
+            raise ValueError("ids must be 1-D")
+        return ids
+
+    def stream_export(self, ids):
+        """The state of the slots in `ids` (distinct, any order) -> uint8 tensor [n_ids, stream_state_bytes()] on this
+        context's device, one record per entry (decode_stream_state reads them).  Stream-ordered after the pushes."""
+        t = self.torch
+        ids = self._state_ids(ids)
+        out = t.empty((ids.size, self.stream_state_bytes()), dtype=t.uint8, device=self.device)
+        self._check(self.lib.wwb_stream_export(self.ctx, ids.ctypes.data, ids.size, out.data_ptr() or None,
+                                               self._stream()))
+        return out
+
+    def stream_import(self, ids, records) -> None:
+        """Puts records (from stream_export of any context of the same model: uint8 [n_ids, bytes], a tensor on any
+        device or a numpy array) into the slots in `ids`, all or nothing.  Waits for the device's verdict: a bad record
+        raises ValueError("record <i>: <reason>") and no slot is touched."""
+        t = self.torch
+        ids = self._state_ids(ids)
+        if isinstance(records, np.ndarray):
+            records = t.from_numpy(np.ascontiguousarray(records).view(np.uint8))
+        if records.dtype != t.uint8:
+            raise ValueError("records must be uint8, got %s" % records.dtype)
+        nb = self.stream_state_bytes()
+        rec = records.to(self.device).contiguous()
+        if nb and rec.numel() != ids.size * nb:
+            raise ValueError("records hold %d bytes, %d entries need %d" % (rec.numel(), ids.size, ids.size * nb))
+        status = t.zeros((2,), dtype=t.int32, device=self.device)
+        self._check(self.lib.wwb_stream_import(self.ctx, ids.ctypes.data, ids.size, rec.data_ptr() or None,
+                                               status.data_ptr(), self._stream()))
+        bad, why = (int(v) for v in status.cpu())
+        if bad:
+            raise ValueError("record %d: %s" % (bad - 1, RECORD_REASONS.get(why, "reason %d" % why)))
 
     def stream_reset(self, mask=None) -> None:
         t = self.torch

@@ -15,7 +15,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libwwb200.so")
-SOURCES = ["api.cu", "filter.cu", "crnn_simt.cu", "wavenet_simt.cu", "counts.cu", "wavenet_tc.cu", "crnn_tc.cu", "host_pipeline.cu", "context.cu"]
+SOURCES = ["api.cu", "filter.cu", "crnn_simt.cu", "wavenet_simt.cu", "counts.cu", "wavenet_tc.cu", "crnn_tc.cu", "host_pipeline.cu", "context.cu",
+           "stream_state.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -483,6 +483,7 @@ int wwb_stream_alloc(wwb_ctx* ctx, int64_t max_streams, int64_t max_chunk) {
   if ((rc = dalloc(ctx, 1, &s.n_win))) return rc;
   if ((rc = dalloc(ctx, S * s.max_frames, &s.win_post))) return rc;
   if ((rc = dalloc(ctx, 2 * S + 1, &s.tables))) return rc;
+  if ((rc = dalloc(ctx, 2, &s.import_check))) return rc;
   for (int k = 0; k < 2; ++k) {
     if (!ctx->stage_host[k]) WWB_CUDA(ctx, cudaHostAlloc((void**)&ctx->stage_host[k], (2 * S + 1) * sizeof(int32_t), cudaHostAllocDefault));
     if (!ctx->stage_done[k]) WWB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->stage_done[k], cudaEventDisableTiming));
@@ -514,16 +515,16 @@ static int stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, c
                               post_max_out, st);
 }
 
-// Checks the host tables of an indexed push (nothing is touched if they are rejected), then copies the slot ids and the
-// chunk offsets to st.tables on `st` through the next page-locked staging slot.  Waiting only for that slot's previous
-// copy keeps the host from blocking behind the push before.
-static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, const int16_t* pcm,
-                        cudaStream_t st) {
+// The checks of every call that names slots by id (the indexed pushes, wwb_stream_export / wwb_stream_import); a rejected
+// call touches nothing.  n_ids in [1, max_streams], the id table and the call's device buffer `buf` present (and for a push,
+// `push` true, the length table), a ctx with a model, distinct ids in [0, max_streams) and for a push chunk lengths in
+// [1, max_chunk].
+static int check_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, bool push, const void* buf) {
   StreamState& s = ctx->st;
   if (n_ids < 1 || n_ids > s.max_streams)
     return fail(ctx, WWB_ERR_STATE, "n_ids %lld outside [1, %lld]", (long long)n_ids, (long long)s.max_streams);
-  if (!ids || !len) return fail(ctx, WWB_ERR_ARG, "NULL id or length table");
-  if (!pcm) return fail(ctx, WWB_ERR_ARG, "NULL pcm");
+  if (!ids || (push && !len)) return fail(ctx, WWB_ERR_ARG, push ? "NULL id or length table" : "NULL id table");
+  if (!buf) return fail(ctx, WWB_ERR_ARG, push ? "NULL pcm" : "NULL records");
   if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
   int64_t marked = 0;
   char why[160] = "";
@@ -534,12 +535,13 @@ static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const i
       break;
     }
     if (ctx->id_seen[id]) {
-      snprintf(why, sizeof(why), "id %d named twice (entry %lld): push again to feed a stream more samples", id, (long long)i);
+      snprintf(why, sizeof(why), push ? "id %d named twice (entry %lld): push again to feed a stream more samples"
+                                      : "id %d named twice (entry %lld)", id, (long long)i);
       break;
     }
     ctx->id_seen[id] = 1;
     ++marked;
-    if (len[i] < 1 || len[i] > s.max_chunk) {
+    if (push && (len[i] < 1 || len[i] > s.max_chunk)) {
       snprintf(why, sizeof(why), "chunk of %d samples (entry %lld) outside [1, %lld]", len[i], (long long)i,
                (long long)s.max_chunk);
       break;
@@ -547,20 +549,38 @@ static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const i
   }
   for (int64_t i = 0; i < marked; ++i) ctx->id_seen[ids[i]] = 0;
   if (why[0]) return fail(ctx, WWB_ERR_STATE, "%s", why);
+  return WWB_OK;
+}
+
+// Copies checked slot ids (and, with `len`, the chunk offsets) to st.tables on `st` through the next page-locked staging
+// slot.  Waiting only for that slot's previous copy keeps the host from blocking behind the call before.
+static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, cudaStream_t st) {
+  StreamState& s = ctx->st;
   const int k = ctx->stage_next;
   WWB_CUDA(ctx, cudaEventSynchronize(ctx->stage_done[k]));
   int32_t* h = ctx->stage_host[k];
   memcpy(h, ids, (size_t)n_ids * sizeof(int32_t));
-  int32_t at = 0;
-  for (int64_t i = 0; i < n_ids; ++i) {
-    h[n_ids + i] = at;
-    at += len[i];
+  int64_t n = n_ids;
+  if (len) {
+    int32_t at = 0;
+    for (int64_t i = 0; i < n_ids; ++i) {
+      h[n_ids + i] = at;
+      at += len[i];
+    }
+    h[2 * n_ids] = at;
+    n = 2 * n_ids + 1;
   }
-  h[2 * n_ids] = at;
-  WWB_CUDA(ctx, cudaMemcpyAsync(s.tables, h, (size_t)(2 * n_ids + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  WWB_CUDA(ctx, cudaMemcpyAsync(s.tables, h, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   WWB_CUDA(ctx, cudaEventRecord(ctx->stage_done[k], st));
   ctx->stage_next = 1 - k;
   return WWB_OK;
+}
+
+// an indexed push's tables: checked, then staged
+static int push_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, const int16_t* pcm,
+                       cudaStream_t st) {
+  int rc = check_tables(ctx, ids, n_ids, len, true, pcm);
+  return rc ? rc : stage_tables(ctx, ids, n_ids, len, st);
 }
 
 int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* is_speech,
@@ -585,7 +605,7 @@ int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids
   if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = stage_tables(ctx, ids_host, n_ids, len_host, pcm, st);
+  int rc = push_tables(ctx, ids_host, n_ids, len_host, pcm, st);
   if (rc) return rc;
   const int32_t* ids = ctx->st.tables;
   return stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, is_speech, is_active, a, threshold, post_out, n_post_out,
@@ -652,7 +672,7 @@ int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_id
   if (!ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = stage_tables(ctx, ids_host, n_ids, len_host, pcm, st);
+  int rc = push_tables(ctx, ids_host, n_ids, len_host, pcm, st);
   if (rc) return rc;
   const int32_t* ids = ctx->st.tables;
   ContextState& c = ctx->cs;
@@ -677,6 +697,43 @@ int wwb_context_reset(wwb_ctx* ctx, void* stream) {
   WWB_CUDA(ctx, cudaMemsetAsync(c.active_length, 0, S * 4, st));
   WWB_CUDA(ctx, cudaMemsetAsync(c.t_is_speech, 0, S, st));
   return wwb_stream_reset(ctx, nullptr, c.max_streams, stream);
+}
+
+int64_t wwb_stream_state_bytes(const wwb_ctx* ctx) {
+  if (!ctx || !ctx->st.max_streams || ctx->kind == WWB_MODEL_NONE) return 0;
+  return stream_state_bytes(ctx->L);
+}
+
+// the host-side checks of wwb_stream_export / wwb_stream_import
+static int check_state_call(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const void* records) {
+  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
+  if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no stream state)");
+  int rc = check_tables(ctx, ids, n_ids, nullptr, false, records);
+  if (rc) return rc;
+  if ((uintptr_t)records % 16) return fail(ctx, WWB_ERR_ARG, "records must be 16-byte aligned");
+  return WWB_OK;
+}
+
+int wwb_stream_export(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, void* records, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_state_call(ctx, ids_host, n_ids, records);
+  if (rc) return rc;
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  if ((rc = stage_tables(ctx, ids_host, n_ids, nullptr, st))) return rc;
+  return launch_stream_export(ctx, ctx->st.tables, n_ids, records, st);
+}
+
+int wwb_stream_import(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const void* records, int32_t* status,
+                      void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_state_call(ctx, ids_host, n_ids, records);
+  if (rc) return rc;
+  if (!status) return fail(ctx, WWB_ERR_ARG, "NULL status");
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  if ((rc = stage_tables(ctx, ids_host, n_ids, nullptr, st))) return rc;
+  return launch_stream_import(ctx, ctx->st.tables, n_ids, records, status, st);
 }
 
 int64_t wwb_launch_count(const wwb_ctx* ctx) { return ctx ? ctx->launches : 0; }

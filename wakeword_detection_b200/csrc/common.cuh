@@ -94,6 +94,8 @@ struct StreamState {
   // tables of an indexed push of n entries (wwb_stream_push_indexed): [0, n) slot of each entry, [n, 2n] exclusive
   // prefix sum of the chunk lengths
   int32_t* tables = nullptr;    // [2S+1]
+  // wwb_stream_import's check: [0] the lowest bad entry and its reason, [1] finished blocks (both 0 between calls)
+  unsigned long long* import_check = nullptr;
 };
 
 // per-stream state of the pipeline stages around the trigger (context.cu)
@@ -186,6 +188,11 @@ int launch_stream_finish(wwb_ctx* ctx, int64_t S, const int32_t* ids, const uint
                          float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
                          float* post_max_out, cudaStream_t st);
 int launch_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, cudaStream_t st);
+// stream state records (stream_state.cu): ids is the device id table of n entries
+int64_t stream_state_bytes(int L);
+int launch_stream_export(wwb_ctx* ctx, const int32_t* ids, int64_t n, void* records, cudaStream_t st);
+int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
+                         cudaStream_t st);
 int launch_context_vad(wwb_ctx* ctx, const int32_t* ids, const uint8_t* vad_raw, int64_t S, cudaStream_t st);
 int launch_context_timeout(wwb_ctx* ctx, const int32_t* ids, const uint8_t* trigger, int64_t S, uint8_t* is_speech_out,
                            uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out, cudaStream_t st);

@@ -42,7 +42,11 @@ class MultiStreamTrigger:
 
     push_streams(ids, chunks, is_speech, is_active) advances only the slots in `ids` (distinct, any order), each
     by its own chunk (a list of 1-D int16 arrays or tensors, any lengths up to chunk_samples): the way a server
-    receives audio.  Same dict, one row per entry of `ids`."""
+    receives audio.  Same dict, one row per entry of `ids`.
+
+    export_streams(ids) -> uint8 device tensor [n_ids, record bytes]: the state of those slots, one record each.
+    import_streams(ids, records) puts such records (from any context of the same model, any device) into the slots in
+    `ids`: to park and resume a session, move it to another slot, context or GPU, or rewind it."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, chunk_samples: int = 320,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, device: int = 0,
@@ -65,6 +69,12 @@ class MultiStreamTrigger:
                                                                    self.pre_emphasis, self.threshold)
         return {"post": post, "n_post": n_post, "trigger": trig, "post_max": pmax}
 
+    def export_streams(self, ids):
+        return self.engine.stream_export(ids)
+
+    def import_streams(self, ids, records) -> None:
+        self.engine.stream_import(ids, records)
+
     def reset(self, mask=None) -> None:
         self.engine.stream_reset(mask)
 
@@ -80,7 +90,9 @@ class MultiStreamPipeline:
 
     step(pcm[S, n] int16, vad_raw[S]) -> dict of device tensors: post, n_post, post_max, is_speech, is_active,
     activated, deactivated.  step_streams(ids, frames, vad_raw) dispatches only the slots in `ids`, each with its own
-    frame (list of 1-D int16 arrays or tensors); same dict, one row per entry of `ids`."""
+    frame (list of 1-D int16 arrays or tensors); same dict, one row per entry of `ids`.  export_streams /
+    import_streams as on MultiStreamTrigger; the records carry the VAD debounce and ActivationTimeout state too (the
+    delays are the context's own)."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, frame_width: int = 20, sample_rate: int = 16000,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, vad_rise_delay: int = 0,
@@ -101,6 +113,12 @@ class MultiStreamPipeline:
     def step_streams(self, ids, frames, vad_raw=None):
         pcm, lengths = _pack(frames)
         return self.engine.context_step_indexed(ids, pcm, lengths, vad_raw, self.pre_emphasis, self.threshold)
+
+    def export_streams(self, ids):
+        return self.engine.stream_export(ids)
+
+    def import_streams(self, ids, records) -> None:
+        self.engine.stream_import(ids, records)
 
     def reset(self) -> None:
         self.engine.context_reset()
