@@ -10,32 +10,12 @@ import pytest
 
 from conftest import get_engine, load_weights
 from oracle import restated as R
+from streaming_helpers import MEL_STATS, check_mel
 from wakeword_detection_b200 import synth
 
 pytestmark = pytest.mark.gpu
 
-MEL_RTOL = 1e-4
 POST_ATOL = 1e-3
-MEL_STATS = {"bins": 0, "at_floor": 0, "max_err": 0.0, "max_err_over_tol": 0.0}
-
-
-def check_mel(got, ref):
-    """BASELINE.md 4: |d| <= 1e-4 * max(|ref|, 1) on EVERY bin, no exemptions (the FFT is fp64 like the
-    reference's, csrc/fft64.cuh).  Bins whose reference value is exactly 0.0 (energy at or below the 1e-5 floor) are
-    counted, not exempted: they obey the same bound.  Running statistics are printed at the end of the session."""
-    got, ref = np.asarray(got, np.float64), np.asarray(ref, np.float64)
-    assert got.shape == ref.shape
-    tol = MEL_RTOL * np.maximum(np.abs(ref), 1.0)
-    err = np.abs(got - ref)
-    MEL_STATS["bins"] += int(ref.size)
-    MEL_STATS["at_floor"] += int((ref == 0.0).sum())
-    if ref.size:
-        MEL_STATS["max_err"] = max(MEL_STATS["max_err"], float(err.max()))
-        MEL_STATS["max_err_over_tol"] = max(MEL_STATS["max_err_over_tol"], float((err / tol).max()))
-        i = np.unravel_index(np.argmax(err / tol), err.shape)
-        assert np.all(err <= tol), "mel error %.3e over tolerance %.3e (ref=%.5f)" % (err[i], tol[i], ref[i])
-    return float(err.max()) if ref.size else 0.0
-
 
 @pytest.fixture(scope="module", autouse=True)
 def _mel_report():

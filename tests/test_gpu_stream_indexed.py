@@ -13,135 +13,17 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, WEIGHTS, load_weights
+from conftest import WEIGHTS, load_weights
 from oracle import restated as R
-from test_gpu_streaming import MODELS, PRECISIONS, TOL, _stream_pcm, schedule
+from streaming_helpers import (MAX_CHUNK, MAX_FRAMES, MODELS, PRECISIONS, SCRIPTS, SIZES, TOL, IndexedSchedule, IPush,
+                               assert_same_rows, engine, host, indexed_script, pipeline_script, run_indexed, schedule,
+                               script)
 from wakeword_detection_b200 import synth
 
-MAX_CHUNK = 1601
-SIZES = (1, 7, 159, 160, 161, 319, 320, 511, 512, 513, MAX_CHUNK - 1, MAX_CHUNK)
-MAX_FRAMES = (MAX_CHUNK - 1) // R.HOP + 1
+_ORACLE_CACHE = {}
 
 
-# ------------------------------------------------------------------------------------ indexed push scripts
-class IPush:
-    def __init__(self, ids, lens, speech, active, threshold, reset=None):
-        self.ids = np.asarray(ids, np.int32)
-        self.lens = np.asarray(lens, np.int32)
-        self.speech = np.asarray(speech, bool)      # per entry
-        self.active = np.asarray(active, bool)      # per entry
-        self.threshold = float(threshold)
-        self.reset = None if reset is None else np.asarray(reset, np.uint8)   # [cap] mask applied before the push
-
-
-def _frames_done(pending, n, active, fall):
-    """the samples a stream keeps pending and the frames its chunk completes (TriggerOracle's sample loop)"""
-    if active:
-        return pending, 0
-    pending += n
-    k = 0
-    while pending >= R.FFT:
-        pending -= R.HOP
-        k += 1
-    return (0 if fall else pending), k
-
-
-class IndexedSchedule:
-    """pushes + per-slot PCM; slot s consumes its own PCM in the order of the pushes that name it.  `frames[i][j]` is
-    the number of frames entry j of push i completes (counted on the host)."""
-
-    def __init__(self, name, cap, a, pushes, seed):
-        self.name, self.cap, self.a, self.pushes = name, cap, float(a), pushes
-        need = np.zeros(cap, np.int64)
-        for p in pushes:
-            need[p.ids] += p.lens
-        pcm = _stream_pcm(cap, max(int(need.max()) + 1, 40000), seed)
-        pcm[0], pcm[4] = np.roll(pcm[0], -2500), np.roll(pcm[4], -5500)   # the wake clips start at sample 500
-        cur = np.zeros(cap, np.int64)
-        pend = np.zeros(cap, np.int64)
-        speech = np.ones(cap, bool)
-        self.chunks, self.frames = [], []
-        for p in pushes:
-            if p.reset is not None:
-                pend[p.reset[:cap] != 0] = 0
-            self.chunks.append([pcm[s, cur[s]:cur[s] + n] for s, n in zip(p.ids, p.lens)])
-            fr = []
-            for s, n, sp, ac in zip(p.ids, p.lens, p.speech, p.active):
-                pend[s], k = _frames_done(pend[s], n, ac, speech[s] and not sp)
-                speech[s] = sp
-                fr.append(k)
-            self.frames.append(fr)
-            cur[p.ids] += p.lens
-
-    def packed(self, i):
-        return np.concatenate(self.chunks[i])
-
-
-def _indexed_script(name, cap, n_push, a, seed, thresholds):
-    """Random subsets of the slots in random order, each slot with its own chunk length from SIZES, plus:
-    slot `absent` sits out pushes 10..21, push 3 names only the highest slot, push 7 every slot (shuffled), push 31
-    has entries that complete max_frames frames and 0 frames, speech falls, active stretches and masked resets.
-    Slots 0 and 4 (the wake clips) are named in most pushes."""
-    r = np.random.default_rng(seed)
-    absent = cap // 2
-    speech = np.ones((n_push, cap), bool)
-    active = np.zeros((n_push, cap), bool)
-    speech[5:9, 1] = False                      # silence then speech
-    speech[14:17, 2] = False                    # a fall on slot 2 (clears its ring) ...
-    speech[14:16, 3] = False                    # ... and on its neighbour 3
-    speech[40:44, cap - 1] = False
-    active[20:27, 0] = True                     # slots 0 / 4: active for a stretch, then sampling again
-    active[36:41, 4] = True
-    resets = {12: np.arange(cap) % 3 == 0, 26: np.arange(cap) == cap - 1, 45: np.arange(cap) % 2 == 1}
-    pend = np.zeros(cap, np.int64)
-    was = np.ones(cap, bool)
-    pushes = []
-    for i in range(n_push):
-        if i == 3:
-            ids = [cap - 1]
-        elif i == 7:
-            ids = list(r.permutation(cap))
-        else:
-            pool = [s for s in range(cap) if not (10 <= i <= 21 and s == absent)]
-            ids = list(r.choice(pool, size=int(r.integers(1, len(pool) + 1)), replace=False))
-            ids += [s for s in (0, 4) if s not in ids and r.random() < 0.8]
-            r.shuffle(ids)
-        lens = [int(v) for v in r.choice(SIZES, size=len(ids))]
-        reset = resets.get(i)
-        if reset is not None:
-            pend[reset] = 0
-        if i in (30, 31):
-            rest = [s for s in ids if s not in (5, 6)]
-            ids, lens = [5, 6] + rest, [0, 0] + lens[-len(rest):] if rest else [0, 0]
-            if i == 30:       # slot 5 to exactly 511 pending samples, slot 6 to at most 510
-                lens[0] = 511 - int(pend[5]) if pend[5] < 511 else R.HOP
-                lens[1] = 1 if pend[6] <= 509 else 200
-            else:             # slot 5: 1601 samples complete max_frames frames; slot 6: 1 sample completes none
-                ids[0], ids[1] = 6, 5
-                lens[0], lens[1] = 1, MAX_CHUNK
-        ids = np.array(ids, np.int32)
-        sp, ac = speech[i, ids], active[i, ids]
-        for s, n, spk, act in zip(ids, lens, sp, ac):
-            pend[s], _ = _frames_done(pend[s], n, act, was[s] and not spk)
-            was[s] = spk
-        pushes.append(IPush(ids, lens, sp, ac, thresholds[(i // 8) % len(thresholds)],
-                            None if reset is None else reset.astype(np.uint8)))
-    return IndexedSchedule(name, cap, a, pushes, seed)
-
-
-SCRIPTS = {
-    "idx": lambda: _indexed_script("idx", 12, 56, 0.0, 21, (0.5, 0.9)),
-    "idx_pe": lambda: _indexed_script("idx_pe", 12, 56, 0.97, 22, (0.9, 0.5)),
-}
-_SCRIPT_CACHE, _ORACLE_CACHE = {}, {}
-
-
-def script(name):
-    if name not in _SCRIPT_CACHE:
-        _SCRIPT_CACHE[name] = SCRIPTS[name]()
-    return _SCRIPT_CACHE[name]
-
-
+# ------------------------------------------------------------------------------------ the oracle's run of a script
 def oracle_run(model, name):
     """per push and entry: (posteriors, trigger, post_max as the device reports it: before the reset on a fall)"""
     key = (model, name)
@@ -166,41 +48,6 @@ def oracle_run(model, name):
         out.append(res)
     _ORACLE_CACHE[key] = out
     return out
-
-
-def _engine(model, precision, cap, max_chunk=MAX_CHUNK):
-    from wakeword_detection_b200 import _cabi
-    eng = _cabi.Engine(load_weights(model), 0, precision)
-    eng.stream_alloc(cap, max_chunk)
-    return eng
-
-
-def _host(res):
-    post, npost, trig, pmax = res
-    return post.cpu().numpy(), npost.cpu().numpy(), trig.cpu().numpy().astype(bool), pmax.cpu().numpy()
-
-
-def _ipush(eng, sch, i):
-    p = sch.pushes[i]
-    return _host(eng.stream_push_indexed(p.ids, sch.packed(i), p.lens, p.speech.astype(np.uint8),
-                                         p.active.astype(np.uint8), sch.a, p.threshold))
-
-
-def run_indexed(eng, sch, between=None):
-    outs = []
-    for i, p in enumerate(sch.pushes):
-        if between is not None:
-            between(i)
-        if p.reset is not None:
-            eng.stream_reset(p.reset)
-        outs.append(_ipush(eng, sch, i))
-    return outs
-
-
-def _same(o1, o2, rows=slice(None)):
-    for i, (x, y) in enumerate(zip(o1, o2)):
-        for a, b in zip(x, y):
-            assert np.array_equal(a[rows], b[rows], equal_nan=True), i
 
 
 # ------------------------------------------------------------------------------------ the scripts (no GPU)
@@ -237,7 +84,7 @@ def test_indexed_replay_vs_oracle(model, precision, name):
     """n_post exact per entry, posteriors within tolerance, NaN tail, trigger exact outside the band, post_max"""
     sch = script(name)
     exp = oracle_run(model, name)
-    eng = _engine(model, precision, sch.cap)
+    eng = engine(model, precision, sch.cap)
     try:
         outs = run_indexed(eng, sch)
     finally:
@@ -325,7 +172,7 @@ def test_indexed_identity_equals_dense_push(model, precision):
     All four outputs of every push are identical."""
     import torch
     sch = schedule("ragged_pe")
-    ea, eb = _engine(model, precision, sch.cap, sch.max_chunk), _engine(model, precision, sch.cap, sch.max_chunk)
+    ea, eb = engine(model, precision, sch.cap, sch.max_chunk), engine(model, precision, sch.cap, sch.max_chunk)
     try:
         for i, (p, chunk) in enumerate(zip(sch.pushes, sch.chunks)):
             if p.reset is not None:
@@ -334,19 +181,12 @@ def test_indexed_identity_equals_dense_push(model, precision):
             S = p.n_streams
             sp, ac = p.speech[:S].astype(np.uint8), p.active[:S].astype(np.uint8)
             x = torch.from_numpy(chunk).to(ea.device)
-            a = _host(ea.stream_push(x, sp, ac, sch.a, p.threshold))
-            b = _host(eb.stream_push_indexed(np.arange(S), x.reshape(-1), [p.n] * S, sp, ac, sch.a, p.threshold))
-            _same([a], [b])
+            a = host(ea.stream_push(x, sp, ac, sch.a, p.threshold))
+            b = host(eb.stream_push_indexed(np.arange(S), x.reshape(-1), [p.n] * S, sp, ac, sch.a, p.threshold))
+            assert_same_rows([a], [b])
     finally:
         ea.close()
         eb.close()
-
-
-def _pipeline_script():
-    g = np.load(os.path.join(GOLDEN, "reference_pipeline.npz"))
-    cfg = dict(zip(("frame_width", "vad_rise_delay", "vad_fall_delay", "min_active", "max_active"), [int(v) for v in g["cfg"]]))
-    pcm0, raw0 = g["pipe_crnn_pcm"], g["pipe_crnn_raw"]
-    return cfg, pcm0, raw0
 
 
 @pytest.mark.gpu
@@ -357,7 +197,7 @@ def test_indexed_identity_equals_dense_context_step(model):
     windows but does not activate on it.)"""
     import torch
     from wakeword_detection_b200.wakeword import MultiStreamPipeline
-    cfg, pcm0, raw0 = _pipeline_script()
+    cfg, pcm0, raw0 = pipeline_script()
     S, nf = 5, len(raw0)
     rng = np.random.default_rng(12)
     pcm = np.stack([np.roll(pcm0, 320 * 7 * s) for s in range(S)])
@@ -407,22 +247,22 @@ def test_indexed_slots_are_isolated(model):
             speech[ids == 2] = False
         pushes.append(IPush(ids, lens, speech, np.zeros(ids.size), 0.5))
     sch = IndexedSchedule("iso", cap, 0.97, pushes, 32)
-    eng = _engine(model, "tc", cap)
+    eng = engine(model, "tc", cap)
     try:
         outs = run_indexed(eng, sch)
     finally:
         eng.close()
     for t in targets:
-        fresh = _engine(model, "tc", cap)
+        fresh = engine(model, "tc", cap)
         try:
             n_win = 0
             for i, p in enumerate(sch.pushes):
                 if t not in p.ids:
                     continue
                 j = int(np.nonzero(p.ids == t)[0][0])
-                got = _host(fresh.stream_push_indexed([t], sch.chunks[i][j], [p.lens[j]], [p.speech[j]], [p.active[j]],
+                got = host(fresh.stream_push_indexed([t], sch.chunks[i][j], [p.lens[j]], [p.speech[j]], [p.active[j]],
                                                       sch.a, p.threshold))
-                _same([tuple(x[j:j + 1] for x in outs[i])], [got])
+                assert_same_rows([tuple(x[j:j + 1] for x in outs[i])], [got])
                 n_win += int(got[1][0])
             assert n_win > 20, t
         finally:
@@ -440,7 +280,7 @@ def test_indexed_rejections_change_nothing(model):
     from wakeword_detection_b200 import _cabi
     w = load_weights(model)
     cap = 16
-    sch = _indexed_script("rej", cap, 16, 0.97, 23, (0.5,))
+    sch = indexed_script("rej", cap, 16, 0.97, 23, (0.5,))
 
     unalloc = _cabi.Engine(w, 0, "tc")
     filt = _cabi.Engine({k: w[k] for k in ("mel_w", "mel_b", "mel_floor", "mel_log_offset", "mel_scale")}, 0, "tc")
@@ -482,14 +322,14 @@ def test_indexed_rejections_change_nothing(model):
             with pytest.raises(ValueError):
                 eng._check(rc)
 
-    ea, eb = _engine(model, "tc", cap), _engine(model, "tc", cap)
+    ea, eb = engine(model, "tc", cap), engine(model, "tc", cap)
     try:
         a = run_indexed(ea, sch)
-        b = run_indexed(eb, sch, lambda i: bad_calls(eb, i))
+        b = run_indexed(eb, sch, before=lambda i: bad_calls(eb, i))
     finally:
         ea.close()
         eb.close()
-    _same(a, b)
+    assert_same_rows(a, b)
     assert sum(int(o[1].sum()) for o in a) > 50
 
 
@@ -502,7 +342,7 @@ def test_step_streams_vs_pipeline_oracle():
     from wakeword_detection_b200.wakeword import MultiStreamPipeline
     model, a = "CRNN", 0.97
     w = load_weights(model)
-    cfg, pcm0, raw0 = _pipeline_script()
+    cfg, pcm0, raw0 = pipeline_script()
     assert all(cfg[k] > 0 for k in ("vad_rise_delay", "vad_fall_delay", "min_active", "max_active"))
     cap, n_step = 8, 300
     rng = np.random.default_rng(13)

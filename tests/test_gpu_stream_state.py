@@ -6,7 +6,7 @@ state on a pipeline context (PipelineOracle).  Every check below is against the 
 the same script, bit for bit: after an import the slot's window holds the same rows as the exporting slot's, so every
 later posterior is computed from the same inputs.
 
-The scripts, oracles and helpers are those of test_gpu_stream_indexed.py / test_gpu_streaming.py.
+The scripts are the indexed ones of test_gpu_stream_indexed.py (streaming_helpers.py builds them).
 """
 import ctypes as C
 import os
@@ -18,12 +18,10 @@ import pytest
 
 from conftest import ROOT, WEIGHTS, load_weights
 from oracle import restated as R
-from test_gpu_parity import check_mel
-from test_gpu_stream_indexed import MAX_CHUNK, _pipeline_script, script
-from test_gpu_streaming import MODELS, PRECISIONS, TOL
+from streaming_helpers import (MODELS, PRECISIONS, SCRIPTS, TOL, check_mel, engine, host, pipeline_script, run_indexed,
+                               script)
 from wakeword_detection_b200 import _cabi
 
-SCRIPTS = ("idx", "idx_pe")
 # after these pushes of the indexed scripts the tests export every slot.  30: slot 5 holds exactly 511 pending samples;
 # 14 / 16: slot 2's ring was just cleared by a VAD fall; 23: slot 0 inside its active stretch (20..26); 12: after a masked
 # reset; 12 .. 21: slot 6 (cap // 2) is absent from the pushes
@@ -101,49 +99,7 @@ def test_decode_round_trips_a_hand_built_record():
 
 
 # ------------------------------------------------------------------------------------ helpers
-def _eng(model, precision="tc", cap=12, max_chunk=MAX_CHUNK, device=0):
-    eng = _cabi.Engine(load_weights(model), device, precision)
-    eng.stream_alloc(cap, max_chunk)
-    return eng
-
-
-def _out(res):
-    post, npost, trig, pmax = res
-    return post.cpu().numpy(), npost.cpu().numpy(), trig.cpu().numpy(), pmax.cpu().numpy()
-
-
-def _push(eng, sch, i, m=None):
-    """push i of the script, slot s as slot m[s]"""
-    p = sch.pushes[i]
-    ids = p.ids if m is None else m[p.ids]
-    return _out(eng.stream_push_indexed(ids, sch.packed(i), p.lens, p.speech.astype(np.uint8), p.active.astype(np.uint8),
-                                        sch.a, p.threshold))
-
-
-def _reset(eng, sch, i, m=None, cap=None):
-    p = sch.pushes[i]
-    if p.reset is None:
-        return
-    if m is None:
-        eng.stream_reset(p.reset)
-        return
-    mask = np.zeros(cap, np.uint8)
-    mask[m[np.nonzero(p.reset)[0]]] = 1
-    eng.stream_reset(mask)
-
-
-def _run(eng, sch, start=0, stop=None, m=None, cap=None, before=None):
-    """pushes start..stop-1 with their resets; before(i) runs before push i's reset"""
-    outs = []
-    for i in range(start, len(sch.pushes) if stop is None else stop):
-        if before is not None:
-            before(i)
-        _reset(eng, sch, i, m, cap)
-        outs.append(_push(eng, sch, i, m))
-    return outs
-
-
-def _same(xs, ys):
+def _same_bits(xs, ys):
     """outputs of two runs bit for bit; the second context's post rows may be longer (a larger max_chunk): NaN there"""
     assert len(xs) == len(ys)
     for i, (x, y) in enumerate(zip(xs, ys)):
@@ -199,7 +155,7 @@ def check_trigger_state(d, j, o, L, tol):
 
 # ------------------------------------------------------------------------------------ 2: the record is the reference's state
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", SCRIPTS)
+@pytest.mark.parametrize("name", list(SCRIPTS))
 @pytest.mark.parametrize("precision", PRECISIONS)
 @pytest.mark.parametrize("model", ["CRNN", "Wavenet"])
 def test_export_is_the_oracle_state(model, precision, name):
@@ -208,13 +164,13 @@ def test_export_is_the_oracle_state(model, precision, name):
     operations), a zero pending tail, the window within the mel bound, post_max within the posterior tolerance."""
     sch = script(name)
     snaps = oracle_states(model, name)
-    eng = _eng(model, precision)
+    eng = engine(model, precision, sch.cap)
     L = eng.L
     seen = {"511": False, "fall": False, "active": False}
     try:
         assert eng.stream_state_bytes() == 48 + 2048 + 160 * L
         for i in range(len(sch.pushes)):
-            _run(eng, sch, i, i + 1)
+            run_indexed(eng, sch, i, i + 1)
             if i not in CUTS:
                 continue
             rec = eng.stream_export(_slots(sch))
@@ -235,7 +191,7 @@ def test_export_is_the_oracle_state(model, precision, name):
 
 # ------------------------------------------------------------------------------------ 3: moved, the stream continues bit for bit
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", SCRIPTS)
+@pytest.mark.parametrize("name", list(SCRIPTS))
 @pytest.mark.parametrize("precision", PRECISIONS)
 @pytest.mark.parametrize("model", MODELS)
 def test_moved_streams_continue_bit_exact(model, precision, name):
@@ -246,35 +202,35 @@ def test_moved_streams_continue_bit_exact(model, precision, name):
     import torch
     sch = script(name)
     recs = {}
-    a = _eng(model, precision)
+    a = engine(model, precision, sch.cap)
 
     def export_at_cuts(i):
         if i - 1 in (23, 30):
             recs[i - 1] = a.stream_export(_slots(sch))
 
     try:
-        outs_a = _run(a, sch, before=export_at_cuts)
+        outs_a = run_indexed(a, sch, before=export_at_cuts)
     finally:
         a.close()
     r = np.random.default_rng(7)
     for cut in (23, 30):
         m = r.permutation(B_CAP)[:sch.cap].astype(np.int32)
-        b = _eng(model, precision, B_CAP, B_CHUNK)
+        b = engine(model, precision, B_CAP, B_CHUNK)
         try:
             noise = torch.randint(-3000, 3000, (B_CAP, B_CHUNK), dtype=torch.int16, device=b.device)
             for _ in range(2):
                 b.stream_push(noise, pre_emphasis=0.5)
             b.stream_import(m, recs[cut])
-            outs_b = _run(b, sch, cut + 1, m=m, cap=B_CAP)
+            outs_b = run_indexed(b, sch, cut + 1, m=m, cap=B_CAP)
         finally:
             b.close()
-        _same(outs_a[cut + 1:], outs_b)
+        _same_bits(outs_a[cut + 1:], outs_b)
     assert sum(int(o[1].sum()) for o in outs_a[24:]) > 100
 
 
 # ------------------------------------------------------------------------------------ 4: across precisions
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", SCRIPTS)
+@pytest.mark.parametrize("name", list(SCRIPTS))
 @pytest.mark.parametrize("model", MODELS)
 def test_tc_export_continues_on_f32(model, name):
     """Records exported from a tc context at cut 23 and imported into an f32 context: the window rows do not depend on
@@ -283,13 +239,13 @@ def test_tc_export_continues_on_f32(model, name):
     and the f32 run's after it."""
     sch = script(name)
     cut = 23
-    src, ref, dst = _eng(model, "tc"), _eng(model, "f32"), _eng(model, "f32")
+    src, ref, dst = engine(model, "tc", sch.cap), engine(model, "f32", sch.cap), engine(model, "f32", sch.cap)
     try:
-        _run(src, sch, 0, cut + 1)
+        run_indexed(src, sch, 0, cut + 1)
         rec = src.stream_export(_slots(sch))
-        outs_ref = _run(ref, sch)
+        outs_ref = run_indexed(ref, sch)
         dst.stream_import(_slots(sch), rec)
-        outs = _run(dst, sch, cut + 1)
+        outs = run_indexed(dst, sch, cut + 1)
     finally:
         src.close()
         ref.close()
@@ -329,9 +285,9 @@ def test_rewind_and_fresh_import(model):
     pushes of the script equal those of a fresh context."""
     sch = script("idx_pe")
     cut = 23
-    eng = _eng(model)
+    eng = engine(model, "tc", sch.cap)
     try:
-        _run(eng, sch, 0, cut + 1)
+        run_indexed(eng, sch, 0, cut + 1)
         slots = np.array([0, 4], np.int32)
         rec = eng.stream_export(slots)
         solo = [(i, j) for i in range(cut + 1, len(sch.pushes)) for j, s in enumerate(sch.pushes[i].ids) if s in slots]
@@ -340,29 +296,29 @@ def test_rewind_and_fresh_import(model):
             outs = []
             for i, j in items:
                 p = sch.pushes[i]
-                outs.append(_out(e.stream_push_indexed([slot_of(p.ids[j])], sch.chunks[i][j], [p.lens[j]], [p.speech[j]],
+                outs.append(host(e.stream_push_indexed([slot_of(p.ids[j])], sch.chunks[i][j], [p.lens[j]], [p.speech[j]],
                                                        [p.active[j]], sch.a, p.threshold)))
             return outs
 
         first = replay(eng, solo)
         eng.stream_import(slots, rec)
         again = replay(eng, solo)
-        _same(first, again)
+        _same_bits(first, again)
         assert sum(int(o[1][0]) for o in first) > 30
 
         # (b) slot 4 (used, mid-stream) gets slot 1 of a fresh context of another capacity and max_chunk
-        fresh_src = _eng(model, "tc", 3, 320)
+        fresh_src = engine(model, "tc", 3, 320)
         blank = fresh_src.stream_export([1])
         fresh_src.close()
         early = [(i, j) for i in range(len(sch.pushes)) for j, s in enumerate(sch.pushes[i].ids) if s == 4][:20]
         eng.stream_import([4], blank)
         got = replay(eng, early)
-        fresh = _eng(model)
+        fresh = engine(model, "tc", sch.cap)
         try:
             want = replay(fresh, early, lambda s: 9)
         finally:
             fresh.close()
-        _same(want, got)
+        _same_bits(want, got)
         assert sum(int(o[1][0]) for o in got) > 20
     finally:
         eng.close()
@@ -377,18 +333,18 @@ def test_export_is_pure_and_import_is_isolated(model):
     slots then export exactly the imported records, and every other slot exports the bytes it exported before."""
     import torch
     sch = script("idx_pe")
-    plain, probed = _eng(model), _eng(model)
+    plain, probed = engine(model, "tc", sch.cap), engine(model, "tc", sch.cap)
     ids = _slots(sch)
     try:
-        outs_plain = _run(plain, sch)
+        outs_plain = run_indexed(plain, sch)
 
         def probe(i):
             e1 = probed.stream_export(ids)
             e2 = probed.stream_export(ids)
             assert torch.equal(e1, e2), i
 
-        outs_probed = _run(probed, sch, before=probe)
-        _same(outs_plain, outs_probed)
+        outs_probed = run_indexed(probed, sch, before=probe)
+        _same_bits(outs_plain, outs_probed)
 
         before = probed.stream_export(ids)
         named, src = np.array([2, 7, 9], np.int32), np.array([5, 0, 11])
@@ -405,7 +361,7 @@ def test_export_is_pure_and_import_is_isolated(model):
 
 # ------------------------------------------------------------------------------------ 7: the device pipeline
 def _pipeline_run_inputs(cap, n_step, seed):
-    cfg, pcm0, raw0 = _pipeline_script()
+    cfg, pcm0, raw0 = pipeline_script()
     rng = np.random.default_rng(seed)
     lens_of = [320, 160, 319, 1, 320, 240, 7, 320]
     rows = [np.roll(pcm0, 977 * s) for s in range(cap)]
@@ -496,7 +452,7 @@ def test_pipeline_records_and_continuation():
         assert n_win > 100
 
         # a trigger-only record (no pipeline state) into slot m[s] of the pipeline context
-        trig = _eng(model, "tc", 2, 1601)
+        trig = engine(model, "tc", 2, 1601)
         try:
             pcm = np.concatenate([c for c in steps[0][1]] + [np.zeros(600, np.int16)])[:600]
             trig.stream_push_indexed([1], pcm, [600], pre_emphasis=a)
@@ -531,7 +487,8 @@ def torch_equal(x, y):
 def test_rejections_change_nothing(model):
     """Table errors raise IndexError before any device work; bad records raise ValueError naming the entry and the
     reason, and no record of the batch is applied (also when only the last one is bad).  After each, an export of every
-    slot is byte-identical to the one taken before."""
+    slot is byte-identical to the one taken before.  A dense context_step rejected for its chunk length, a NULL pcm or a
+    filter-only ctx launches no kernel: the VAD debounce and trigger state of every slot export unchanged."""
     import torch
     w = load_weights(model)
     other = "Wavenet" if model == "CRNN" else "CRNN"
@@ -545,10 +502,31 @@ def test_rejections_change_nothing(model):
                 e.stream_export([0])
             with pytest.raises(IndexError):
                 e.stream_import([0], np.zeros((1, 48), np.uint8))
+        filt.context_alloc()
+        n0 = filt.launch_count()
+        with pytest.raises(IndexError):
+            filt.context_step(np.zeros((4, 160), np.int16))
+        assert filt.launch_count() == n0
     finally:
         unalloc.close()
         filt.close()
-    src = _eng(other, "tc", 2, 320)
+    pipe = engine(model, "tc", 4, 320)
+    try:
+        pipe.context_alloc()
+        noise = torch.randint(-3000, 3000, (4, 320), dtype=torch.int16, device=pipe.device)
+        for raw in ([1, 0, 1, 0], [1, 1, 0, 0]):
+            pipe.context_step(noise, raw)
+        four = np.arange(4, dtype=np.int32)
+        p0, n0 = pipe.stream_export(four), pipe.launch_count()
+        with pytest.raises(IndexError):
+            pipe.context_step(np.zeros((4, 321), np.int16))
+        assert pipe.lib.wwb_context_step(pipe.ctx, None, 4, 320, None, C.c_float(0), C.c_float(0.5), *([None] * 7),
+                                         pipe._stream()) == -1
+        assert pipe.launch_count() == n0
+        assert torch.equal(pipe.stream_export(four), p0)
+    finally:
+        pipe.close()
+    src = engine(other, "tc", 2, 320)
     try:
         foreign = src.stream_export([0, 1])
     finally:
@@ -556,10 +534,10 @@ def test_rejections_change_nothing(model):
 
     sch = script("idx_pe")
     cap = sch.cap
-    eng = _eng(model)
+    eng = engine(model, "tc", sch.cap)
     nb = eng.stream_state_bytes()
     try:
-        _run(eng, sch, 0, 31)
+        run_indexed(eng, sch, 0, 31)
         ids = _slots(sch)
         e0 = eng.stream_export(ids)
 
@@ -639,20 +617,20 @@ def test_move_to_another_gpu(model):
         pytest.skip("needs two GPUs")
     sch = script("idx_pe")
     cut = 23
-    a = _eng(model)
+    a = engine(model, "tc", sch.cap)
     try:
-        _run(a, sch, 0, cut + 1)
+        run_indexed(a, sch, 0, cut + 1)
         rec = a.stream_export(_slots(sch))
-        outs_a = _run(a, sch, cut + 1)
+        outs_a = run_indexed(a, sch, cut + 1)
     finally:
         a.close()
     m = np.random.default_rng(9).permutation(B_CAP)[:sch.cap].astype(np.int32)
-    b = _eng(model, "tc", B_CAP, B_CHUNK, device=1)
+    b = engine(model, "tc", B_CAP, B_CHUNK, device=1)
     try:
         moved = rec.to("cuda:1")
         b.stream_import(m, moved)
         with torch.cuda.device(1):
-            outs_b = _run(b, sch, cut + 1, m=m, cap=B_CAP)
+            outs_b = run_indexed(b, sch, cut + 1, m=m, cap=B_CAP)
     finally:
         b.close()
-    _same(outs_a, outs_b)
+    _same_bits(outs_a, outs_b)

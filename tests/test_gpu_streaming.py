@@ -13,18 +13,12 @@ import pytest
 
 from conftest import GOLDEN, WEIGHTS, load_weights
 from oracle import restated as R
+from streaming_helpers import (CHUNKS, MODELS, PRECISIONS, SCHEDULES, TOL, Push, Schedule, assert_same_rows,
+                               engine, host, schedule, wake_clip)
 from wakeword_detection_b200 import synth
 
-MODELS = ("CRNN", "CRNN_arik_original", "Wavenet")
-PRECISIONS = ("f32", "tc", "tc_fast")
-TOL = {"f32": 1e-3, "tc": 1e-3, "tc_fast": 2e-2}
-CHUNKS = (1, 7, 159, 160, 161, 319, 320, 511, 512, 513, 1599, 1600, 1601)
 STATS = {}
-
-
-def _wake(name):
-    import os
-    return np.load(os.path.join(GOLDEN, "wake_%s_pcm.npy" % name))
+_ORACLE_CACHE = {}
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -34,110 +28,7 @@ def _report():
         print("\n[stream replay] %s %s: %d windows checked against the oracle, max |err| %.3e" % (model, prec, n, err))
 
 
-# ------------------------------------------------------------------------------------ push scripts
-class Push:
-    def __init__(self, n, n_streams, speech, active, threshold, reset=None):
-        self.n, self.n_streams, self.threshold = int(n), int(n_streams), float(threshold)
-        self.speech = np.asarray(speech, bool)
-        self.active = np.asarray(active, bool)
-        self.reset = None if reset is None else np.asarray(reset, np.uint8)
-
-
-class Schedule:
-    """pushes + per-stream PCM; stream s consumes its own PCM only in the pushes that cover it."""
-
-    def __init__(self, name, cap, max_chunk, a, pcm, pushes):
-        self.name, self.cap, self.max_chunk, self.a = name, cap, max_chunk, float(a)
-        self.pushes = pushes
-        cur = np.zeros(cap, np.int64)
-        self.chunks = []
-        for p in pushes:
-            S = p.n_streams
-            assert 1 <= S <= cap and 1 <= p.n <= max_chunk
-            c = np.stack([pcm[s, cur[s]:cur[s] + p.n] for s in range(S)])
-            assert c.shape == (S, p.n), "stream PCM too short for the script"
-            self.chunks.append(c)
-            cur[:S] += p.n
-        self.max_frames = (max_chunk - 1) // R.HOP + 1
-
-
-def _clip_runs(n, seed):
-    """noise with runs at both int16 rails: -32768 / 32767 become -1.0000305 / 1.0 before the clip to [-1, 1]"""
-    x = synth.stream_int16(n, 0, seed, 3)
-    r = np.random.default_rng(seed)
-    for at in r.integers(0, n - 400, size=max(1, n // 3000)):
-        x[at:at + r.integers(40, 400)] = -32768 if r.random() < 0.5 else 32767
-    return x
-
-
-def _stream_pcm(cap, n, seed):
-    pcm = np.stack([synth.stream_int16(n, (s % 5) + (s % 5 > 2), seed, s) for s in range(cap)])
-    pcm[0, 3000:3000 + 35200] = _wake("crnn")[:n - 3000]
-    if cap > 4:
-        pcm[4, 6000:6000 + 35200] = _wake("wavenet")[:n - 6000]
-    if cap > 3:
-        pcm[3] = _clip_runs(n, seed)
-    return pcm
-
-
-def _ragged(name, cap, n_push, a, seed, thresholds):
-    """max_chunk = 1601 on one allocation: every chunk size of CHUNKS, a push that completes exactly max_frames frames,
-    pushes that complete none, pushes over prefixes of the streams, masked resets (one mask shorter than cap) and the
-    speech / activation scripts below."""
-    r = np.random.default_rng(seed)
-    ns = list(CHUNKS)                                   # 1 + 7 + 159 + 160 + 161 = 488 < 512 samples after five pushes
-    total = sum(ns)
-    fix = (R.FFT + 159 - total) % R.HOP or R.HOP        # leaves 511 samples pending: the next 1601 completes 11 frames
-    ns += [fix, 1601]
-    ns += [int(v) for v in r.choice(CHUNKS, size=n_push - len(ns))]
-    speech = np.ones((n_push, cap), bool)
-    active = np.zeros((n_push, cap), bool)
-    speech[:10, 1] = False                              # stream 1: silence, then speech (no fall)
-    speech[25:30, 2] = False                            # stream 2: speech, a fall at push 25 (reset), speech again
-    if cap > 5:
-        speech[45:47, 5] = False
-    active[40:48, 0] = True                             # streams 0 / 4: active for a stretch, then sampling again
-    if cap > 4:
-        active[50:56, 4] = True
-    n_streams = np.full(n_push, cap)
-    n_streams[12:17] = cap - 1                          # the last stream sits out five pushes
-    n_streams[20:22] = 1
-    n_streams[33:36] = cap // 2
-    resets = {28: [0, 1, 0, 1, 0, 1][:cap - 1]}         # shorter than cap: the streams past its end keep their state
-    if n_push > 52:
-        m = np.zeros(cap, np.uint8)
-        m[[0, cap - 1]] = 1
-        resets[52] = m
-    pushes = [Push(ns[i], n_streams[i], speech[i], active[i], thresholds[(i // 8) % len(thresholds)], resets.get(i))
-              for i in range(n_push)]
-    pcm = _stream_pcm(cap, sum(ns) + 1, seed)
-    return Schedule(name, cap, 1601, a, pcm, pushes)
-
-
-def _long(name, a):
-    """max_chunk = 16000: 97 then 100 (= max_frames) frames per push"""
-    cap, n_push = 2, 4
-    pcm = np.stack([synth.stream_int16(16000 * n_push, 2, 5, s) for s in range(cap)])
-    pcm[0, 8000:8000 + 35200] = _wake("crnn")
-    pcm[1, 20000:20000 + 35200] = _wake("wavenet")
-    pushes = [Push(16000, cap, np.ones(cap), np.zeros(cap), 0.9) for _ in range(n_push)]
-    return Schedule(name, cap, 16000, a, pcm, pushes)
-
-
-SCHEDULES = {
-    "ragged_pe": lambda: _ragged("ragged_pe", 10, 64, 0.97, 1, (0.5, 0.9)),
-    "ragged": lambda: _ragged("ragged", 7, 40, 0.0, 2, (0.5,)),
-    "long_pe": lambda: _long("long_pe", 0.97),
-}
-_SCHED_CACHE, _ORACLE_CACHE = {}, {}
-
-
-def schedule(name):
-    if name not in _SCHED_CACHE:
-        _SCHED_CACHE[name] = SCHEDULES[name]()
-    return _SCHED_CACHE[name]
-
-
+# ------------------------------------------------------------------------------------ the oracle's run of a schedule
 def oracle_run(model, sname):
     """Per push and covered stream: (posteriors, trigger, post_max as the device reports it).  On a VAD fall the
     device reports the maximum before its reset (stream_finish_kernel writes it, then clears the state)."""
@@ -166,21 +57,12 @@ def oracle_run(model, sname):
     return out
 
 
-def _engine(model, precision, cap, max_chunk):
-    from wakeword_detection_b200 import _cabi
-    eng = _cabi.Engine(load_weights(model), 0, precision)
-    eng.stream_alloc(cap, max_chunk)
-    return eng
-
-
-def _push(eng, sch, i, chunk=None):
+def _push(eng, sch, i):
     import torch
     p = sch.pushes[i]
     S = p.n_streams
-    c = torch.from_numpy(sch.chunks[i] if chunk is None else chunk).to(eng.device)
-    post, npost, trig, pmax = eng.stream_push(c, p.speech[:S].astype(np.uint8), p.active[:S].astype(np.uint8),
-                                              sch.a, p.threshold)
-    return post.cpu().numpy(), npost.cpu().numpy(), trig.cpu().numpy().astype(bool), pmax.cpu().numpy()
+    c = torch.from_numpy(sch.chunks[i]).to(eng.device)
+    return host(eng.stream_push(c, p.speech[:S].astype(np.uint8), p.active[:S].astype(np.uint8), sch.a, p.threshold))
 
 
 def run_device(eng, sch, between=None):
@@ -284,7 +166,7 @@ def test_trigger_oracle_is_the_padded_window_formula(a):
 def test_stream_replay_vs_oracle(model, precision, sname):
     sch = schedule(sname)
     exp = oracle_run(model, sname)
-    eng = _engine(model, precision, sch.cap, sch.max_chunk)
+    eng = engine(model, precision, sch.cap, sch.max_chunk)
     try:
         assert eng.stream_max_frames() == sch.max_frames
         outs = run_device(eng, sch)
@@ -351,14 +233,8 @@ def _small_schedule(cap, n_push, a, seed, n_streams=None, resets=None, speech=Tr
     pushes = [Push(ns[i], n_streams.get(i, cap), np.full(cap, speech), np.zeros(cap), 0.5, resets.get(i))
               for i in range(n_push)]
     pcm = np.stack([synth.stream_int16(sum(ns) + 1, 2 + (s % 2) * 3, seed, s) for s in range(cap)])
-    pcm[0, 600:600 + 35200] = _wake("crnn")[:sum(ns) + 1 - 600]
+    pcm[0, 600:600 + 35200] = wake_clip("crnn")[:sum(ns) + 1 - 600]
     return Schedule("small", cap, 1601, a, pcm, pushes)
-
-
-def _assert_same(o1, o2, streams=slice(None)):
-    for i, (x, y) in enumerate(zip(o1, o2)):
-        for a, b in zip(x, y):
-            assert np.array_equal(a[streams], b[streams], equal_nan=True), i
 
 
 @pytest.mark.gpu
@@ -369,8 +245,8 @@ def test_skipped_stream_keeps_its_state(model):
     cap, skip = 4, range(4, 9)
     sch = _small_schedule(cap, 16, 0.97, 5, n_streams={i: cap - 1 for i in skip})
     w = load_weights(model)
-    eng = _engine(model, "tc", cap, 1601)
-    fresh = _engine(model, "tc", cap, 1601)
+    eng = engine(model, "tc", cap, 1601)
+    fresh = engine(model, "tc", cap, 1601)
     try:
         a = run_device(eng, sch)
         keep = [i for i in range(len(sch.pushes)) if i not in skip]
@@ -379,7 +255,7 @@ def test_skipped_stream_keeps_its_state(model):
         eng.close()
         fresh.close()
     s = cap - 1
-    _assert_same([a[i] for i in keep], b, streams=s)
+    assert_same_rows([a[i] for i in keep], b, rows=s)
     o = R.TriggerOracle(w, 0.5, sch.a)
     n_win = 0
     for j, i in enumerate(keep):
@@ -403,7 +279,7 @@ def test_masked_reset(model):
     with_reset = _small_schedule(cap, 14, 0.97, 6, resets={at: mask})
     without = _small_schedule(cap, 14, 0.97, 6)
     w = load_weights(model)
-    e1, e2 = _engine(model, "tc", cap, 1601), _engine(model, "tc", cap, 1601)
+    e1, e2 = engine(model, "tc", cap, 1601), engine(model, "tc", cap, 1601)
     try:
         a = run_device(e1, with_reset)
         b = run_device(e2, without)
@@ -411,8 +287,8 @@ def test_masked_reset(model):
         e1.close()
         e2.close()
     untouched = np.array([1, 3, 4, 5, 6, 7])
-    _assert_same(a, b, streams=untouched)
-    _assert_same(a[:at], b[:at])
+    assert_same_rows(a, b, rows=untouched)
+    assert_same_rows(a[:at], b[:at])
     for s in (0, 2):
         o = R.TriggerOracle(w, 0.5, with_reset.a)
         for i, chunk in enumerate(with_reset.chunks):
@@ -460,13 +336,13 @@ def test_rejected_pushes_and_batch_calls_leave_the_state_alone(model, precision)
             eng.pipeline(big, hop=2, pre_emphasis=0.97)
 
     for name, between in (("base", None), ("again", None), ("rejected", rejected), ("batch", batch_calls)):
-        eng = _engine(model, precision, cap, 1601)
+        eng = engine(model, precision, cap, 1601)
         try:
             runs[name] = run_device(eng, sch, None if between is None else (lambda i, e=eng, f=between: f(e, i)))
         finally:
             eng.close()
     for name in ("again", "rejected", "batch"):
-        _assert_same(runs["base"], runs[name])
+        assert_same_rows(runs["base"], runs[name])
     assert sum(int(o[1].sum()) for o in runs["base"]) > 100
 
 

@@ -180,6 +180,14 @@ def _f32(a) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(a), dtype=np.float32)
 
 
+def _pcm_dtype(dtype) -> int:
+    """WWB_PCM_* of a numpy or torch PCM dtype"""
+    code = {"int16": WWB_PCM_I16, "float32": WWB_PCM_F32}.get(str(dtype).replace("torch.", ""))
+    if code is None:
+        raise ValueError("PCM must be int16 or float32, got %s" % dtype)
+    return code
+
+
 def make_weights_struct(w: Optional[Dict[str, np.ndarray]], filt: Dict[str, np.ndarray]):
     """Packs host arrays into the C struct; returns (struct, keepalive list)."""
     keep = []
@@ -304,12 +312,7 @@ class Engine:
         t = self.torch
         if isinstance(pcm, np.ndarray):
             pcm = t.from_numpy(np.ascontiguousarray(pcm))
-        if pcm.dtype == t.int16:
-            dt = WWB_PCM_I16
-        elif pcm.dtype == t.float32:
-            dt = WWB_PCM_F32
-        else:
-            raise ValueError("PCM must be int16 or float32, got %s" % pcm.dtype)
+        dt = _pcm_dtype(pcm.dtype)
         if pcm.dim() == 1:
             pcm = pcm[None]
         if pcm.dim() != 2:
@@ -395,12 +398,7 @@ class Engine:
         pcm = np.ascontiguousarray(pcm)
         if pcm.ndim == 1:
             pcm = pcm[None]
-        if pcm.dtype == np.int16:
-            dt = WWB_PCM_I16
-        elif pcm.dtype == np.float32:
-            dt = WWB_PCM_F32
-        else:
-            raise ValueError("PCM must be int16 or float32")
+        dt = _pcm_dtype(pcm.dtype)
         S, N = pcm.shape
         nw = self.num_windows(self.num_frames(N), hop)
         post = out if out is not None else np.empty((S, nw), np.float32)
@@ -416,12 +414,7 @@ class Engine:
         `sweep_wait()` returns.  Returns the result record (dict of numpy arrays) that the wait fills."""
         if pcm.ndim != 2 or not pcm.flags.c_contiguous:
             raise ValueError("PCM must be a C-contiguous [n_streams, n_samples] array")
-        if pcm.dtype == np.int16:
-            dt = WWB_PCM_I16
-        elif pcm.dtype == np.float32:
-            dt = WWB_PCM_F32
-        else:
-            raise ValueError("PCM must be int16 or float32")
+        dt = _pcm_dtype(pcm.dtype)
         engines = [self] + list(others)
         S, N = pcm.shape
         F = self.num_frames(N)
@@ -530,25 +523,11 @@ class Engine:
                     threshold: float = 0.5):
         """pcm [S, n] int16 -> (post [S, max_frames] (NaN = none), n_post [S] int32,
         trigger [S] uint8, post_max [S] float32) device tensors."""
-        t = self.torch
-        x = self._dev(pcm, t.int16)
-        if x.dim() == 1:
-            x = x[None]
+        x = self._dense(pcm)
         S, n = x.shape
-        mf = self.stream_max_frames()
-        sp = self._dev(np.asarray(is_speech), t.uint8) if is_speech is not None and not isinstance(is_speech, t.Tensor) \
-            else (is_speech.to(self.device, t.uint8) if is_speech is not None else None)
-        ac = self._dev(np.asarray(is_active), t.uint8) if is_active is not None and not isinstance(is_active, t.Tensor) \
-            else (is_active.to(self.device, t.uint8) if is_active is not None else None)
-        post = t.empty((S, mf), dtype=t.float32, device=self.device)
-        npost = t.empty((S,), dtype=t.int32, device=self.device)
-        trig = t.empty((S,), dtype=t.uint8, device=self.device)
-        pmax = t.empty((S,), dtype=t.float32, device=self.device)
-        self._check(self.lib.wwb_stream_push(
-            self.ctx, x.data_ptr(), S, n, sp.data_ptr() if sp is not None else None,
-            ac.data_ptr() if ac is not None else None, float(pre_emphasis), float(threshold),
-            post.data_ptr(), npost.data_ptr(), trig.data_ptr(), pmax.data_ptr(), self._stream()))
-        return post, npost, trig, pmax
+        out = self._trigger_out(S)
+        self._call(self.lib.wwb_stream_push, (x.data_ptr(), S, n), (is_speech, is_active), pre_emphasis, threshold, out)
+        return out
 
     def _flags(self, a):
         """optional per-stream uint8 flags -> device tensor (or None)"""
@@ -556,6 +535,11 @@ class Engine:
         if a is None:
             return None
         return a.to(self.device, t.uint8) if isinstance(a, t.Tensor) else self._dev(np.asarray(a), t.uint8)
+
+    def _dense(self, pcm):
+        """the int16 PCM of a dense push or step on the device, [S, n]"""
+        x = self._dev(pcm, self.torch.int16)
+        return x[None] if x.dim() == 1 else x
 
     def _indexed(self, ids, pcm_packed, lengths):
         """host int32 id / length tables and the packed int16 PCM on the device, checked for shape (the library checks
@@ -570,24 +554,40 @@ class Engine:
                              % (int(lengths.astype(np.int64).sum()), list(x.shape)))
         return ids, lengths, x
 
+    def _trigger_out(self, S: int):
+        """the outputs of a push over S entries: post [S, max_frames], n_post, trigger, post_max"""
+        t = self.torch
+        return (t.empty((S, self.stream_max_frames()), dtype=t.float32, device=self.device),
+                t.empty((S,), dtype=t.int32, device=self.device), t.empty((S,), dtype=t.uint8, device=self.device),
+                t.empty((S,), dtype=t.float32, device=self.device))
+
+    def _pipeline_out(self, S: int):
+        """the outputs of a step over S entries, by name in the C ABI's order"""
+        t = self.torch
+        out = {"post": t.empty((S, self.stream_max_frames()), dtype=t.float32, device=self.device),
+               "n_post": t.empty((S,), dtype=t.int32, device=self.device),
+               "post_max": t.empty((S,), dtype=t.float32, device=self.device)}
+        for k in ("is_speech", "is_active", "activated", "deactivated"):
+            out[k] = t.empty((S,), dtype=t.uint8, device=self.device)
+        return out
+
+    def _call(self, fn, streams, flags, pre_emphasis, threshold, outputs) -> None:
+        """fn(ctx, *streams, *flags, pre_emphasis, threshold, *outputs, stream): the C call of every push and step;
+        `streams` name the streams and their PCM, `flags` are the optional per-entry uint8 inputs"""
+        flags = [self._flags(f) for f in flags]
+        self._check(fn(self.ctx, *streams, *[None if f is None else f.data_ptr() for f in flags], float(pre_emphasis),
+                       float(threshold), *[o.data_ptr() for o in outputs], self._stream()))
+
     def stream_push_indexed(self, ids, pcm_packed, lengths, is_speech=None, is_active=None, pre_emphasis: float = 0.0,
                             threshold: float = 0.5):
         """One chunk for each slot in `ids` (distinct, any order), chunk i of lengths[i] samples, packed back to back in
         `pcm_packed` (1-D int16) -> (post [n_ids, max_frames] (NaN = none), n_post [n_ids] int32, trigger [n_ids] uint8,
         post_max [n_ids] float32) device tensors, one row per entry of `ids`.  is_speech / is_active per entry."""
-        t = self.torch
         ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
-        K = ids.size
-        sp, ac = self._flags(is_speech), self._flags(is_active)
-        post = t.empty((K, self.stream_max_frames()), dtype=t.float32, device=self.device)
-        npost = t.empty((K,), dtype=t.int32, device=self.device)
-        trig = t.empty((K,), dtype=t.uint8, device=self.device)
-        pmax = t.empty((K,), dtype=t.float32, device=self.device)
-        self._check(self.lib.wwb_stream_push_indexed(
-            self.ctx, ids.ctypes.data, K, lengths.ctypes.data, x.data_ptr(), sp.data_ptr() if sp is not None else None,
-            ac.data_ptr() if ac is not None else None, float(pre_emphasis), float(threshold),
-            post.data_ptr(), npost.data_ptr(), trig.data_ptr(), pmax.data_ptr(), self._stream()))
-        return post, npost, trig, pmax
+        out = self._trigger_out(ids.size)
+        self._call(self.lib.wwb_stream_push_indexed, (ids.ctypes.data, ids.size, lengths.ctypes.data, x.data_ptr()),
+                   (is_speech, is_active), pre_emphasis, threshold, out)
+        return out
 
     def context_alloc(self, frame_width: int = 20, vad_rise_delay: int = 0, vad_fall_delay: int = 0, min_active: int = 500,
                       max_active: int = 5000) -> None:
@@ -599,44 +599,20 @@ class Engine:
         """One SpeechPipeline dispatch for every stream: vad debounce -> wake-word trigger -> activation timeout.
         pcm [S, n] int16, vad_raw [S] (None = speech) -> dict of device tensors: post [S, max_frames] (NaN = none),
         n_post, post_max, is_speech, is_active, activated, deactivated."""
-        t = self.torch
-        x = self._dev(pcm, t.int16)
-        if x.dim() == 1:
-            x = x[None]
+        x = self._dense(pcm)
         S, n = x.shape
-        mf = self.stream_max_frames()
-        raw = None
-        if vad_raw is not None:
-            raw = vad_raw.to(self.device, t.uint8) if isinstance(vad_raw, t.Tensor) else self._dev(np.asarray(vad_raw), t.uint8)
-        out = {"post": t.empty((S, mf), dtype=t.float32, device=self.device),
-               "n_post": t.empty((S,), dtype=t.int32, device=self.device),
-               "post_max": t.empty((S,), dtype=t.float32, device=self.device)}
-        for k in ("is_speech", "is_active", "activated", "deactivated"):
-            out[k] = t.empty((S,), dtype=t.uint8, device=self.device)
-        self._check(self.lib.wwb_context_step(
-            self.ctx, x.data_ptr(), S, n, raw.data_ptr() if raw is not None else None, float(pre_emphasis), float(threshold),
-            out["post"].data_ptr(), out["n_post"].data_ptr(), out["post_max"].data_ptr(), out["is_speech"].data_ptr(),
-            out["is_active"].data_ptr(), out["activated"].data_ptr(), out["deactivated"].data_ptr(), self._stream()))
+        out = self._pipeline_out(S)
+        self._call(self.lib.wwb_context_step, (x.data_ptr(), S, n), (vad_raw,), pre_emphasis, threshold, out.values())
         return out
 
     def context_step_indexed(self, ids, pcm_packed, lengths, vad_raw=None, pre_emphasis: float = 0.0,
                              threshold: float = 0.5):
         """context_step for the slots in `ids` only, tables and packing as in stream_push_indexed; vad_raw per entry ->
         the dict of context_step with one row per entry of `ids`."""
-        t = self.torch
         ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
-        K = ids.size
-        raw = self._flags(vad_raw)
-        out = {"post": t.empty((K, self.stream_max_frames()), dtype=t.float32, device=self.device),
-               "n_post": t.empty((K,), dtype=t.int32, device=self.device),
-               "post_max": t.empty((K,), dtype=t.float32, device=self.device)}
-        for k in ("is_speech", "is_active", "activated", "deactivated"):
-            out[k] = t.empty((K,), dtype=t.uint8, device=self.device)
-        self._check(self.lib.wwb_context_step_indexed(
-            self.ctx, ids.ctypes.data, K, lengths.ctypes.data, x.data_ptr(), raw.data_ptr() if raw is not None else None,
-            float(pre_emphasis), float(threshold), out["post"].data_ptr(), out["n_post"].data_ptr(),
-            out["post_max"].data_ptr(), out["is_speech"].data_ptr(), out["is_active"].data_ptr(),
-            out["activated"].data_ptr(), out["deactivated"].data_ptr(), self._stream()))
+        out = self._pipeline_out(ids.size)
+        self._call(self.lib.wwb_context_step_indexed, (ids.ctypes.data, ids.size, lengths.ctypes.data, x.data_ptr()),
+                   (vad_raw,), pre_emphasis, threshold, out.values())
         return out
 
     def context_reset(self) -> None:

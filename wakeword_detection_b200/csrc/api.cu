@@ -515,23 +515,57 @@ static int stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, c
                               post_max_out, st);
 }
 
-// The checks of every call that names slots by id (the indexed pushes, wwb_stream_export / wwb_stream_import); a rejected
-// call touches nothing.  n_ids in [1, max_streams], the id table and the call's device buffer `buf` present (and for a push,
-// `push` true, the length table), a ctx with a model, distinct ids in [0, max_streams) and for a push chunk lengths in
-// [1, max_chunk].
-static int check_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, bool push, const void* buf) {
+// vad debounce -> stream_push -> activation timeout over S entries (ids / off as in stream_push)
+static int context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids, const int32_t* off,
+                        const uint8_t* vad_raw, float a, float threshold, float* post_out, int32_t* n_post_out,
+                        float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out, uint8_t* activated_out,
+                        uint8_t* deactivated_out, cudaStream_t st) {
+  ContextState& c = ctx->cs;
+  int rc = launch_context_vad(ctx, ids, vad_raw, S, st);
+  if (rc) return rc;
+  if ((rc = stream_push(ctx, pcm, S, n, ids, off, c.e_is_speech, c.e_is_active, a, threshold, post_out, n_post_out,
+                        c.trigger, post_max_out, st))) return rc;
+  return launch_context_timeout(ctx, ids, c.trigger, S, is_speech_out, is_active_out, activated_out, deactivated_out, st);
+}
+
+// The state a streaming call needs: wwb_stream_alloc, with `pipeline` wwb_context_alloc too, and with `model` encoder
+// weights (not a filter-only ctx).
+static int check_state(wwb_ctx* ctx, bool pipeline, bool model) {
+  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
+  if (pipeline && !ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
+  if (model && ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
+  return WWB_OK;
+}
+
+// The checks of a dense push (`pipeline`: a dense step): the state allocated, S in [1, max_streams], n in [1, max_chunk],
+// pcm present, then a model (a NULL pcm is reported before a filter-only ctx).
+static int check_dense(wwb_ctx* ctx, bool pipeline, int64_t S, int64_t n, const int16_t* pcm) {
+  const int64_t cap = pipeline ? ctx->cs.max_streams : ctx->st.max_streams;
+  if (!cap) return check_state(ctx, pipeline, true);
+  if (S < 1 || S > cap) return fail(ctx, WWB_ERR_STATE, "n_streams %lld outside [1, %lld]", (long long)S, (long long)cap);
+  if (n < 1 || n > ctx->st.max_chunk)
+    return fail(ctx, WWB_ERR_STATE, "chunk of %lld samples outside [1, %lld]", (long long)n, (long long)ctx->st.max_chunk);
+  if (!pcm) return fail(ctx, WWB_ERR_ARG, "NULL pcm");
+  return check_state(ctx, pipeline, true);
+}
+
+// The table checks of every call that names slots by id (the indexed pushes and steps, wwb_stream_export /
+// wwb_stream_import; a rejected call touches nothing): n_ids in [1, cap] (cap: max_streams of allocated state), the id
+// table and the call's device buffer `buf` present (and for a push, `push` true, the length table), distinct ids in
+// [0, cap) and for a push chunk lengths in [1, max_chunk].
+static int check_tables(wwb_ctx* ctx, int64_t cap, const int32_t* ids, int64_t n_ids, const int32_t* len, bool push,
+                        const void* buf) {
   StreamState& s = ctx->st;
-  if (n_ids < 1 || n_ids > s.max_streams)
-    return fail(ctx, WWB_ERR_STATE, "n_ids %lld outside [1, %lld]", (long long)n_ids, (long long)s.max_streams);
+  if (n_ids < 1 || n_ids > cap)
+    return fail(ctx, WWB_ERR_STATE, "n_ids %lld outside [1, %lld]", (long long)n_ids, (long long)cap);
   if (!ids || (push && !len)) return fail(ctx, WWB_ERR_ARG, push ? "NULL id or length table" : "NULL id table");
   if (!buf) return fail(ctx, WWB_ERR_ARG, push ? "NULL pcm" : "NULL records");
-  if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
   int64_t marked = 0;
   char why[160] = "";
   for (int64_t i = 0; i < n_ids; ++i) {
     const int32_t id = ids[i];
-    if (id < 0 || id >= s.max_streams) {
-      snprintf(why, sizeof(why), "id %d of entry %lld outside [0, %lld)", id, (long long)i, (long long)s.max_streams);
+    if (id < 0 || id >= cap) {
+      snprintf(why, sizeof(why), "id %d of entry %lld outside [0, %lld)", id, (long long)i, (long long)cap);
       break;
     }
     if (ctx->id_seen[id]) {
@@ -576,23 +610,24 @@ static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const i
   return WWB_OK;
 }
 
-// an indexed push's tables: checked, then staged
-static int push_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, const int16_t* pcm,
-                       cudaStream_t st) {
-  int rc = check_tables(ctx, ids, n_ids, len, true, pcm);
-  return rc ? rc : stage_tables(ctx, ids, n_ids, len, st);
+// an indexed push's (`pipeline`: step's) tables: checked in the order of check_dense, then staged
+static int push_tables(wwb_ctx* ctx, bool pipeline, const int32_t* ids, int64_t n_ids, const int32_t* len,
+                       const int16_t* pcm, cudaStream_t st) {
+  const int64_t cap = pipeline ? ctx->cs.max_streams : ctx->st.max_streams;
+  if (!cap) return check_state(ctx, pipeline, true);
+  int rc = check_tables(ctx, cap, ids, n_ids, len, true, pcm);
+  if (rc || (rc = check_state(ctx, pipeline, true))) return rc;
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  return stage_tables(ctx, ids, n_ids, len, st);
 }
 
 int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* is_speech,
                     const uint8_t* is_active, float a, float threshold, float* post_out, int32_t* n_post_out,
                     uint8_t* trigger_out, float* post_max_out, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
-  if (S < 1 || S > ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "n_streams %lld exceeds capacity %lld", (long long)S, (long long)ctx->st.max_streams);
-  if (n < 1 || n > ctx->st.max_chunk) return fail(ctx, WWB_ERR_STATE, "chunk of %lld samples exceeds capacity %lld", (long long)n, (long long)ctx->st.max_chunk);
-  if (!pcm) return fail(ctx, WWB_ERR_ARG, "NULL pcm");
+  int rc = check_dense(ctx, false, S, n, pcm);
+  if (rc) return rc;
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no encode/detect weights)");
   return stream_push(ctx, pcm, S, n, nullptr, nullptr, is_speech, is_active, a, threshold, post_out, n_post_out,
                      trigger_out, post_max_out, (cudaStream_t)stream);
 }
@@ -602,10 +637,8 @@ int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids
                             float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
                             float* post_max_out, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = push_tables(ctx, ids_host, n_ids, len_host, pcm, st);
+  int rc = push_tables(ctx, false, ids_host, n_ids, len_host, pcm, st);
   if (rc) return rc;
   const int32_t* ids = ctx->st.tables;
   return stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, is_speech, is_active, a, threshold, post_out, n_post_out,
@@ -614,7 +647,8 @@ int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids
 
 int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
+  int rc = check_state(ctx, false, false);
+  if (rc) return rc;
   if (S < 1 || S > ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "n_streams out of range");
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   return launch_stream_reset(ctx, mask, S, (cudaStream_t)stream);
@@ -623,7 +657,8 @@ int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, void* stream)
 int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, int vad_fall_delay_ms, int min_active_ms,
                       int max_active_ms) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
+  int rc = check_state(ctx, false, false);
+  if (rc) return rc;
   if (ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "context state already allocated");
   if (frame_width_ms < 1 || vad_rise_delay_ms < 0 || vad_fall_delay_ms < 0 || min_active_ms < 0 || max_active_ms < 0)
     return fail(ctx, WWB_ERR_ARG, "bad pipeline timing");
@@ -634,7 +669,6 @@ int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, i
   c.fall_length = vad_fall_delay_ms / frame_width_ms;
   c.min_active = (float)min_active_ms / (float)frame_width_ms; // activation_timeout.py:20-21 (true division)
   c.max_active = (float)max_active_ms / (float)frame_width_ms;
-  int rc;
   if ((rc = dalloc(ctx, S, &c.run_value))) return rc;
   if ((rc = dalloc(ctx, S, &c.run_length))) return rc;
   if ((rc = dalloc(ctx, S, &c.is_speech))) return rc;
@@ -652,16 +686,11 @@ int wwb_context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, con
                      float* post_out, int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
                      uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
-  if (S < 1 || S > ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "n_streams %lld exceeds capacity %lld", (long long)S, (long long)ctx->cs.max_streams);
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = launch_context_vad(ctx, nullptr, vad_raw, S, st);
+  int rc = check_dense(ctx, true, S, n, pcm);
   if (rc) return rc;
-  if ((rc = wwb_stream_push(ctx, pcm, S, n, ctx->cs.e_is_speech, ctx->cs.e_is_active, a, threshold, post_out, n_post_out,
-                            ctx->cs.trigger, post_max_out, stream))) return rc;
-  return launch_context_timeout(ctx, nullptr, ctx->cs.trigger, S, is_speech_out, is_active_out, activated_out,
-                                deactivated_out, st);
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  return context_step(ctx, pcm, S, n, nullptr, nullptr, vad_raw, a, threshold, post_out, n_post_out, post_max_out,
+                      is_speech_out, is_active_out, activated_out, deactivated_out, (cudaStream_t)stream);
 }
 
 int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
@@ -669,23 +698,18 @@ int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_id
                              int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
                              uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = push_tables(ctx, ids_host, n_ids, len_host, pcm, st);
+  int rc = push_tables(ctx, true, ids_host, n_ids, len_host, pcm, st);
   if (rc) return rc;
   const int32_t* ids = ctx->st.tables;
-  ContextState& c = ctx->cs;
-  if ((rc = launch_context_vad(ctx, ids, vad_raw, n_ids, st))) return rc;
-  if ((rc = stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, c.e_is_speech, c.e_is_active, a, threshold, post_out,
-                        n_post_out, c.trigger, post_max_out, st))) return rc;
-  return launch_context_timeout(ctx, ids, c.trigger, n_ids, is_speech_out, is_active_out, activated_out, deactivated_out,
-                                st);
+  return context_step(ctx, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out, post_max_out,
+                      is_speech_out, is_active_out, activated_out, deactivated_out, st);
 }
 
 int wwb_context_reset(wwb_ctx* ctx, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  if (!ctx->cs.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_context_alloc has not been called");
+  int rc = check_state(ctx, true, false);
+  if (rc) return rc;
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
   ContextState& c = ctx->cs;
@@ -696,7 +720,7 @@ int wwb_context_reset(wwb_ctx* ctx, void* stream) {
   WWB_CUDA(ctx, cudaMemsetAsync(c.is_active, 0, S, st));
   WWB_CUDA(ctx, cudaMemsetAsync(c.active_length, 0, S * 4, st));
   WWB_CUDA(ctx, cudaMemsetAsync(c.t_is_speech, 0, S, st));
-  return wwb_stream_reset(ctx, nullptr, c.max_streams, stream);
+  return launch_stream_reset(ctx, nullptr, c.max_streams, st);
 }
 
 int64_t wwb_stream_state_bytes(const wwb_ctx* ctx) {
@@ -706,10 +730,8 @@ int64_t wwb_stream_state_bytes(const wwb_ctx* ctx) {
 
 // the host-side checks of wwb_stream_export / wwb_stream_import
 static int check_state_call(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const void* records) {
-  if (!ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "wwb_stream_alloc has not been called");
-  if (ctx->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx holds a filter only (no stream state)");
-  int rc = check_tables(ctx, ids, n_ids, nullptr, false, records);
-  if (rc) return rc;
+  int rc = check_state(ctx, false, true);
+  if (rc || (rc = check_tables(ctx, ctx->st.max_streams, ids, n_ids, nullptr, false, records))) return rc;
   if ((uintptr_t)records % 16) return fail(ctx, WWB_ERR_ARG, "records must be 16-byte aligned");
   return WWB_OK;
 }
