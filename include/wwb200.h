@@ -59,8 +59,8 @@ enum { WWB_COUNT_FRR_MAX = 0, WWB_COUNT_FAR_EDGES = 1 };
  * (FC weights [out,in]; see wakeword_detection_b200/weights.py).  Unused family = NULL. */
 typedef struct {
   int32_t kind;       /* WWB_MODEL_*                                              */
-  int32_t mel_length; /* encoder window length in mel frames: 151 (CRNN) / 182     */
-  int32_t n_out;      /* detect outputs: 1 (sigmoid) or 2 (softmax)                */
+  int32_t mel_length; /* encoder window length in mel frames: 151 (CRNN) / 17..182 (WaveNet; shipped 182) */
+  int32_t n_out;      /* detect outputs: CRNN 1 (sigmoid) or 2 (softmax); WaveNet 2 (softmax) */
   int32_t n_mel;      /* 40 */
   int32_t n_bins;     /* 257 */
   /* filter.tflite: FC -> max(floor) -> log -> -offset -> *scale */
@@ -105,6 +105,9 @@ const char* wwb_last_error(const wwb_ctx* ctx);
  * utils/evaluate_models.py:30-36): uploads the weights, builds twiddle/mel tables. */
 int wwb_create(int device, const wwb_weights* w, int precision, wwb_ctx** out);
 int wwb_destroy(wwb_ctx* ctx);
+/* WWB_PREC_TC / TC_FAST are refused (WWB_ERR_ARG, the ctx keeps its precision) for a model whose weights cannot be
+ * packed for the tensor cores: a WaveNet with a BatchNorm scale of 0 or an operand outside the fp16 range (DESIGN.md §4).
+ * wwb_create refuses such a model at those precisions; it loads at WWB_PREC_F32. */
 int wwb_set_precision(wwb_ctx* ctx, int precision);
 int wwb_sync(wwb_ctx* ctx, void* stream);
 

@@ -51,13 +51,17 @@ def stft_magnitude(frames: np.ndarray) -> np.ndarray:
     return np.abs(spec).astype(F32)
 
 
-def mel_from_magnitude(mag: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
-    """filter.tflite (SURVEY.md A1): FC -> max(.,1e-5) -> log -> -(-11.5129) -> *0.5."""
-    y = mag.astype(F32) @ w["mel_w"].T.astype(F32) + w["mel_b"].astype(F32)
-    y = np.maximum(y.astype(F32), F32(w["mel_floor"]))
-    y = np.log(y).astype(F32)
-    y = (y - F32(w["mel_log_offset"])).astype(F32)
-    return (y * F32(w["mel_scale"])).astype(F32)
+def mel_from_magnitude(mag: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
+    """filter.tflite (SURVEY.md A1): FC -> max(.,1e-5) -> log -> -(-11.5129) -> *0.5.
+
+    `dtype` is the arithmetic of this and every model function below: float32 follows the reference, float64 is the
+    high-precision reference the kernels' error is measured against."""
+    F = np.dtype(dtype).type
+    y = mag.astype(F) @ w["mel_w"].T.astype(F) + w["mel_b"].astype(F)
+    y = np.maximum(y.astype(F), F(w["mel_floor"]))
+    y = np.log(y).astype(F)
+    y = (y - F(w["mel_log_offset"])).astype(F)
+    return (y * F(w["mel_scale"])).astype(F)
 
 
 def num_frames(n_samples: int) -> int:
@@ -84,123 +88,129 @@ def mel_stream(x: np.ndarray, w: Dict[str, np.ndarray], a: float = 0.0) -> np.nd
 
 # ----------------------------------------------------------------------------
 # CRNN  (SURVEY.md Appendix A2; architecture cross-check wwdetect/CRNN/model.py:21-56)
-def _sigmoid(x):
+def _sigmoid(x, dtype=F32):
+    F = np.dtype(dtype).type
     with np.errstate(over="ignore"):
-        return (F32(1) / (F32(1) + np.exp(-x.astype(F32)))).astype(F32)
+        return (F(1) / (F(1) + np.exp(-x.astype(F)))).astype(F)
 
 
-def crnn_conv(mel: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
+def crnn_conv(mel: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
     """mel [B, L=151, 40] (time, freq) -> [B, 19, 640] with feature = f*32 + c.
     CONV_2D 32@(5 freq x 20 time), stride (2 freq, 8 time), SAME (freq pad 1/2,
     time pad 6/7), fused ReLU, then TRANSPOSE/RESHAPE to [time, freq*chan]."""
+    F = np.dtype(dtype).type
     B, L, M = mel.shape
     kf, kt = w["conv_w"].shape[1], w["conv_w"].shape[2]
     of, ot = -(-M // 2), -(-L // 8)
     pf = max((of - 1) * 2 + kf - M, 0)
     pt = max((ot - 1) * 8 + kt - L, 0)
-    x = np.pad(mel.astype(F32), ((0, 0), (pt // 2, pt - pt // 2), (pf // 2, pf - pf // 2)))
+    x = np.pad(mel.astype(F), ((0, 0), (pt // 2, pt - pt // 2), (pf // 2, pf - pf // 2)))
     fi = (np.arange(of) * 2)[:, None] + np.arange(kf)[None, :]          # [of, kf]
     ti = (np.arange(ot) * 8)[:, None] + np.arange(kt)[None, :]          # [ot, kt]
     # patches[b, t, f, kf, kt]
     patches = x[:, ti[:, None, None, :], fi[None, :, :, None]]
-    cw = w["conv_w"].reshape(w["conv_w"].shape[0], kf * kt).astype(F32)
-    y = patches.reshape(B, ot, of, kf * kt) @ cw.T + w["conv_b"].astype(F32)
-    y = np.maximum(y.astype(F32), F32(0))
+    cw = w["conv_w"].reshape(w["conv_w"].shape[0], kf * kt).astype(F)
+    y = patches.reshape(B, ot, of, kf * kt) @ cw.T + w["conv_b"].astype(F)
+    y = np.maximum(y.astype(F), F(0))
     return y.reshape(B, ot, of * cw.shape[0])
 
 
-def _gru(seq: np.ndarray, W, U, bi, br, reverse: bool) -> np.ndarray:
+def _gru(seq: np.ndarray, W, U, bi, br, reverse: bool, dtype=F32) -> np.ndarray:
     """Keras GRU v2 (reset_after=True), gate order z|r|h, h0 = 0; returns the
     output sequence in *original* time order (CRNN/encode.tflite WHILE bodies)."""
+    F = np.dtype(dtype).type
     B, T, _ = seq.shape
     H = U.shape[1]
-    xw = (seq.astype(F32) @ W.T.astype(F32) + bi.astype(F32)).astype(F32)     # [B,T,3H]
-    h = np.zeros((B, H), F32)
-    out = np.zeros((B, T, H), F32)
+    xw = (seq.astype(F) @ W.T.astype(F) + bi.astype(F)).astype(F)     # [B,T,3H]
+    h = np.zeros((B, H), F)
+    out = np.zeros((B, T, H), F)
     order = range(T - 1, -1, -1) if reverse else range(T)
     for t in order:
-        hu = (h @ U.T.astype(F32) + br.astype(F32)).astype(F32)
-        z = _sigmoid(xw[:, t, :H] + hu[:, :H])
-        r = _sigmoid(xw[:, t, H:2 * H] + hu[:, H:2 * H])
-        c = np.tanh(xw[:, t, 2 * H:] + r * hu[:, 2 * H:]).astype(F32)
-        h = (z * h + (F32(1) - z) * c).astype(F32)
+        hu = (h @ U.T.astype(F) + br.astype(F)).astype(F)
+        z = _sigmoid(xw[:, t, :H] + hu[:, :H], F)
+        r = _sigmoid(xw[:, t, H:2 * H] + hu[:, H:2 * H], F)
+        c = np.tanh(xw[:, t, 2 * H:] + r * hu[:, 2 * H:]).astype(F)
+        h = (z * h + (F(1) - z) * c).astype(F)
         out[:, t] = h
     return out
 
 
-def crnn_encode(mel: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
+def crnn_encode(mel: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
     """mel windows [B, 151, 40] -> encoder output [B, 64] = [fwd_last, bwd_last]."""
-    x = crnn_conv(mel, w)
-    f1 = _gru(x, w["gru1_f_w"], w["gru1_f_u"], w["gru1_f_bi"], w["gru1_f_br"], False)
-    b1 = _gru(x, w["gru1_b_w"], w["gru1_b_u"], w["gru1_b_bi"], w["gru1_b_br"], True)
+    x = crnn_conv(mel, w, dtype)
+    f1 = _gru(x, w["gru1_f_w"], w["gru1_f_u"], w["gru1_f_bi"], w["gru1_f_br"], False, dtype)
+    b1 = _gru(x, w["gru1_b_w"], w["gru1_b_u"], w["gru1_b_bi"], w["gru1_b_br"], True, dtype)
     s1 = np.concatenate([f1, b1], axis=2)
-    f2 = _gru(s1, w["gru2_f_w"], w["gru2_f_u"], w["gru2_f_bi"], w["gru2_f_br"], False)
-    b2 = _gru(s1, w["gru2_b_w"], w["gru2_b_u"], w["gru2_b_bi"], w["gru2_b_br"], True)
+    f2 = _gru(s1, w["gru2_f_w"], w["gru2_f_u"], w["gru2_f_bi"], w["gru2_f_br"], False, dtype)
+    b2 = _gru(s1, w["gru2_b_w"], w["gru2_b_u"], w["gru2_b_bi"], w["gru2_b_br"], True, dtype)
     return np.concatenate([f2[:, -1], b2[:, 0]], axis=1)
 
 
-def crnn_detect(enc: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
+def crnn_detect(enc: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
     """[B, 64] -> detect output [B, n] (n=1 sigmoid head | n=2 softmax head)."""
-    h = np.maximum(enc.astype(F32) @ w["det1_w"].T + w["det1_b"], F32(0)).astype(F32)
-    z = (h @ w["det2_w"].T + w["det2_b"]).astype(F32)
+    F = np.dtype(dtype).type
+    h = np.maximum(enc.astype(F) @ w["det1_w"].T + w["det1_b"], F(0)).astype(F)
+    z = (h @ w["det2_w"].T + w["det2_b"]).astype(F)
     if z.shape[1] == 1:
-        return _sigmoid(z)
+        return _sigmoid(z, F)
     z = z - z.max(axis=1, keepdims=True)
-    e = np.exp(z).astype(F32)
-    return (e / e.sum(axis=1, keepdims=True)).astype(F32)
+    e = np.exp(z).astype(F)
+    return (e / e.sum(axis=1, keepdims=True)).astype(F)
 
 
 # ----------------------------------------------------------------------------
 # WaveNet  (SURVEY.md Appendix A3; cross-check wwdetect/wavenet/wavenet_model.py:11-128)
-def wavenet_encode(mel: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
-    """mel windows [B, 182, 40] -> [B, 182, 32] (sum of the 24 skip branches)."""
+def wavenet_encode(mel: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
+    """mel windows [B, L, 40] -> [B, L, 32] (sum of the 24 skip branches)."""
+    F = np.dtype(dtype).type
     B, T, _ = mel.shape
-    x = np.maximum(mel.astype(F32) @ w["in_w"].T + w["in_b"], F32(0)).astype(F32)
+    x = np.maximum(mel.astype(F) @ w["in_w"].T + w["in_b"], F(0)).astype(F)
     nb = w["sig_w"].shape[0]
     out = None
     for k in range(nb):
         d = int(w["dilation"][k])
-        u = (x * w["bn_mul"][k] + w["bn_add"][k]).astype(F32)
+        u = (x * w["bn_mul"][k] + w["bn_add"][k]).astype(F)
         up = np.pad(u, ((0, 0), (2 * d, 0), (0, 0)))            # zeros *after* the BN affine
         taps = np.concatenate([up[:, j * d:j * d + T] for j in range(3)], axis=2)   # [B,T,48]
         a_s = taps @ w["sig_w"][k].reshape(16, 48).T + w["sig_b"][k]
         a_t = taps @ w["tanh_w"][k].reshape(16, 48).T + w["tanh_b"][k]
-        g = (np.tanh(a_t.astype(F32)).astype(F32) * _sigmoid(a_s)).astype(F32)
-        s = np.maximum(g @ w["skip_w"][k].T + w["skip_b"][k], F32(0)).astype(F32)
-        out = s if out is None else (out + s).astype(F32)
+        g = (np.tanh(a_t.astype(F)).astype(F) * _sigmoid(a_s, F)).astype(F)
+        s = np.maximum(g @ w["skip_w"][k].T + w["skip_b"][k], F(0)).astype(F)
+        out = s if out is None else (out + s).astype(F)
         if k < nb - 1:
-            x = (np.maximum(g @ w["res_w"][k].T + w["res_b"][k], F32(0)) + x).astype(F32)
+            x = (np.maximum(g @ w["res_w"][k].T + w["res_b"][k], F(0)) + x).astype(F)
     return out
 
 
-def wavenet_detect(enc: np.ndarray, w: Dict[str, np.ndarray]) -> np.ndarray:
-    """[B, 182, 32] -> softmax [B, 2]: ReLU -> 1x1 32->32 ReLU -> 1x1 32->2 -> max over
+def wavenet_detect(enc: np.ndarray, w: Dict[str, np.ndarray], dtype=F32) -> np.ndarray:
+    """[B, L, 32] -> softmax [B, 2]: ReLU -> 1x1 32->32 ReLU -> 1x1 32->2 -> max over
     time -> softmax (Wavenet/detect.tflite)."""
-    h = np.maximum(enc.astype(F32), F32(0))
-    h = np.maximum(h @ w["det1_w"].T + w["det1_b"], F32(0)).astype(F32)
-    z = (h @ w["det2_w"].T + w["det2_b"]).astype(F32).max(axis=1)
+    F = np.dtype(dtype).type
+    h = np.maximum(enc.astype(F), F(0))
+    h = np.maximum(h @ w["det1_w"].T + w["det1_b"], F(0)).astype(F)
+    z = (h @ w["det2_w"].T + w["det2_b"]).astype(F).max(axis=1)
     z = z - z.max(axis=1, keepdims=True)
-    e = np.exp(z).astype(F32)
-    return (e / e.sum(axis=1, keepdims=True)).astype(F32)
+    e = np.exp(z).astype(F)
+    return (e / e.sum(axis=1, keepdims=True)).astype(F)
 
 
 def is_crnn(w) -> bool:
     return "conv_w" in w
 
 
-def encode(mel: np.ndarray, w) -> np.ndarray:
-    return crnn_encode(mel, w) if is_crnn(w) else wavenet_encode(mel, w)
+def encode(mel: np.ndarray, w, dtype=F32) -> np.ndarray:
+    return crnn_encode(mel, w, dtype) if is_crnn(w) else wavenet_encode(mel, w, dtype)
 
 
-def detect(enc: np.ndarray, w) -> np.ndarray:
-    return crnn_detect(enc, w) if is_crnn(w) else wavenet_detect(enc, w)
+def detect(enc: np.ndarray, w, dtype=F32) -> np.ndarray:
+    return crnn_detect(enc, w, dtype) if is_crnn(w) else wavenet_detect(enc, w, dtype)
 
 
-def posterior(mel: np.ndarray, w) -> np.ndarray:
+def posterior(mel: np.ndarray, w, dtype=F32) -> np.ndarray:
     """Wake-class probability per window: out[..., -1] covers both CRNN heads and the
     WaveNet head (SURVEY.md §8 note N1; wakeword/tflite.py:228-231,
     evaluate_models.py:80,86)."""
-    return detect(encode(mel, w), w)[:, -1]
+    return detect(encode(mel, w, dtype), w, dtype)[:, -1]
 
 
 # ----------------------------------------------------------------------------

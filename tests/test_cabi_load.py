@@ -59,6 +59,15 @@ def test_bad_arguments_rejected_before_any_device_work():
     st.n_bins = 129
     assert lib.wwb_create(0, C.byref(st), 0, C.byref(ctx)) == -1
     assert b"geometry" in lib.wwb_last_error(None)
+    # WaveNet: the head is a 2-way softmax (a [1, 32] det2_w would be read as [2, 32]), and both WaveNet paths hold
+    # windows of up to 182 frames (the fp32 path's shared buffer has 182 + 18 rows)
+    w = load_weights("Wavenet")
+    for field, value, msg in (("n_out", 1, b"n_out"), ("mel_length", 183, b"window"), ("mel_length", 192, b"window")):
+        for precision in (0, 1):
+            st, keep = _cabi.make_weights_struct(w, w)
+            setattr(st, field, value)
+            assert lib.wwb_create(0, C.byref(st), precision, C.byref(ctx)) == -1 and not ctx.value
+            assert msg in lib.wwb_last_error(None)
 
 
 def test_weights_struct_packing():

@@ -115,6 +115,9 @@ static int build_filter_tables(wwb_ctx* ctx, const wwb_weights* w) {
     }
   }
   band_seg0[kMel] = (int)seg_band.size();
+  if (seg_band.size() > (size_t)kMaxSeg)
+    return fail(ctx, WWB_ERR_ARG, "mel matrix has %d segments (runs of up to %d consecutive non-zero bins); at most %d supported",
+                (int)seg_band.size(), kSegTaps, kMaxSeg);
   MelTables& mt = ctx->mel;
   mt.n_seg = (int)seg_band.size();
   mt.n_tap = (int)tap_bin.size();
@@ -128,22 +131,61 @@ static int build_filter_tables(wwb_ctx* ctx, const wwb_weights* w) {
   return WWB_OK;
 }
 
+// floor(log2 x) for a finite x > 0
+static int floor_log2(double x) {
+  int e;
+  frexp(x, &e);
+  return e - 1;
+}
+
+static float max_abs(const float* p, size_t n) {
+  float m = 0.f;
+  for (size_t i = 0; i < n; ++i)
+    if (std::isfinite(p[i])) m = std::max(m, fabsf(p[i]));
+  return m;
+}
+
+static void scale(std::vector<float>& v, float s) {
+  for (float& x : v) x *= s;
+}
+
 static int build_crnn(wwb_ctx* ctx, const wwb_weights* w) {
   CrnnWeights& C = ctx->crnn;
   int rc;
   if (!w->conv_w || !w->conv_b || !w->det1_w || !w->det2_w) return fail(ctx, WWB_ERR_ARG, "CRNN weights missing");
   for (int i = 0; i < 4; ++i)
     if (!w->gru_w[i] || !w->gru_u[i] || !w->gru_bi[i] || !w->gru_br[i]) return fail(ctx, WWB_ERR_ARG, "GRU weights missing");
+  // Power-of-two rescale (DESIGN.md §4): conv weights and bias times sigma, layer-1 input weights over sigma.  Exact in
+  // fp32 (ReLU is positively homogeneous), so both paths compute the same function.  sigma = 2^floor(log2(g / c) / 2)
+  // balances the largest layer-1 weight g against the largest conv weight c, so that the conv activations and the
+  // layer-1 weights, fp16 hi/lo operands on the tensor cores, stay in fp16's normal range for models trained at any
+  // feature scale.  Every power-of-two member of the family (conv * s, layer-1 / s) gets the same weights here.
+  std::vector<float> conv_w(w->conv_w, w->conv_w + 32 * 100), conv_b(w->conv_b, w->conv_b + 32);
+  std::vector<float> w1[2] = {std::vector<float>(w->gru_w[0], w->gru_w[0] + 96 * 640),
+                              std::vector<float>(w->gru_w[1], w->gru_w[1] + 96 * 640)};
+  {
+    const float c = max_abs(conv_w.data(), conv_w.size());
+    const float g = std::max(max_abs(w1[0].data(), w1[0].size()), max_abs(w1[1].data(), w1[1].size()));
+    if (c > 0.f && g > 0.f) {
+      const int e = floor_log2((double)g / (double)c);
+      const float sigma = ldexpf(1.f, e >= 0 ? e / 2 : -((1 - e) / 2));
+      scale(conv_w, sigma);
+      scale(conv_b, sigma);
+      scale(w1[0], 1.f / sigma);
+      scale(w1[1], 1.f / sigma);
+    }
+  }
+  const float* gru_w[4] = {w1[0].data(), w1[1].data(), w->gru_w[2], w->gru_w[3]};
   // conv [32][100] -> [100][32]
-  if ((rc = upload(ctx, transposed(w->conv_w, 32, 100), &C.conv_w))) return rc;
-  if ((rc = upload(ctx, std::vector<float>(w->conv_b, w->conv_b + 32), &C.conv_b))) return rc;
-  if ((rc = upload(ctx, crnn_pack_conv(w->conv_w), &C.tc_conv))) return rc;
+  if ((rc = upload(ctx, transposed(conv_w.data(), 32, 100), &C.conv_w))) return rc;
+  if ((rc = upload(ctx, conv_b, &C.conv_b))) return rc;
+  if ((rc = upload(ctx, crnn_pack_conv(conv_w.data()), &C.tc_conv))) return rc;
   for (int layer = 0; layer < 2; ++layer) {
     const int in = layer == 0 ? 640 : 64;
     // both directions side by side: Wt [in][192], bias [192]
     std::vector<float> wt((size_t)in * 192), bi(192);
     for (int dir = 0; dir < 2; ++dir) {
-      const float* src = w->gru_w[layer * 2 + dir];   // [96][in]
+      const float* src = gru_w[layer * 2 + dir];   // [96][in]
       for (int n = 0; n < 96; ++n) {
         bi[dir * 96 + n] = w->gru_bi[layer * 2 + dir][n];
         for (int k = 0; k < in; ++k) wt[(size_t)k * 192 + dir * 96 + n] = src[(size_t)n * in + k];
@@ -154,7 +196,7 @@ static int build_crnn(wwb_ctx* ctx, const wwb_weights* w) {
     {  // tensor-core path: [192][in] (fwd units then bwd units), split into fp16 hi/lo stages
       std::vector<float> w_nk((size_t)192 * in);
       for (int dir = 0; dir < 2; ++dir)
-        memcpy(&w_nk[(size_t)dir * 96 * in], w->gru_w[layer * 2 + dir], sizeof(float) * 96 * in);
+        memcpy(&w_nk[(size_t)dir * 96 * in], gru_w[layer * 2 + dir], sizeof(float) * 96 * in);
       if (layer == 0 && (rc = upload(ctx, crnn_pack_w1(w_nk.data()), &C.tc_w1))) return rc;
       if (layer == 1 && (rc = upload(ctx, crnn_pack_w2(w_nk.data()), &C.tc_w2))) return rc;
     }
@@ -189,9 +231,25 @@ static int build_wavenet(wwb_ctx* ctx, const wwb_weights* w) {
   int rc;
   if (!w->in_w || !w->bn_mul || !w->sig_w || !w->tanh_w || !w->res_w || !w->skip_w || !w->dilation || !w->det1_w)
     return fail(ctx, WWB_ERR_ARG, "WaveNet weights missing");
-  if ((rc = upload(ctx, transposed(w->in_w, 16, 40), &N.in_w))) return rc;
-  if ((rc = upload(ctx, std::vector<float>(w->in_b, w->in_b + 16), &N.in_b))) return rc;
-  if ((rc = upload(ctx, std::vector<float>(w->bn_mul, w->bn_mul + 24 * 16), &N.bn_mul))) return rc;
+  // Power-of-two rescale of the residual stream x (DESIGN.md §4): in_w, in_b, res_w and res_b times sigma, bn_mul over
+  // sigma.  Exact in fp32, so both paths compute the same function.  The tensor-core path folds bn_mul into the gate
+  // weights and feeds x itself as the fp16 hi/lo operand, so the split error depends on where the model sits in this
+  // family.  sigma brings the largest |bn_mul| into [64, 128), the octave of the shipped model (sigma = 1 there), and
+  // maps every power-of-two member of the family onto the same weights.
+  std::vector<float> in_w(w->in_w, w->in_w + 16 * 40), in_b(w->in_b, w->in_b + 16), bn_mul(w->bn_mul, w->bn_mul + 24 * 16),
+      res_w(w->res_w, w->res_w + 23 * 16 * 16), res_b(w->res_b, w->res_b + 23 * 16);
+  const float bn_max = max_abs(bn_mul.data(), bn_mul.size());
+  if (bn_max > 0.f) {
+    const float sigma = ldexpf(1.f, floor_log2(bn_max) - 6);
+    scale(in_w, sigma);
+    scale(in_b, sigma);
+    scale(res_w, sigma);
+    scale(res_b, sigma);
+    scale(bn_mul, 1.f / sigma);
+  }
+  if ((rc = upload(ctx, transposed(in_w.data(), 16, 40), &N.in_w))) return rc;
+  if ((rc = upload(ctx, in_b, &N.in_b))) return rc;
+  if ((rc = upload(ctx, bn_mul, &N.bn_mul))) return rc;
   if ((rc = upload(ctx, std::vector<float>(w->bn_add, w->bn_add + 24 * 16), &N.bn_add))) return rc;
   std::vector<float> gw(24 * 48 * 32), gb(24 * 32), rw(24 * 16 * 48, 0.f), rb(24 * 48, 0.f);
   for (int b = 0; b < 24; ++b) {
@@ -209,21 +267,26 @@ static int build_wavenet(wwb_ctx* ctx, const wwb_weights* w) {
     }
     for (int i = 0; i < 16; ++i) {
       if (b < 23)
-        for (int o = 0; o < 16; ++o) rw[((size_t)b * 16 + i) * 48 + o] = w->res_w[((size_t)b * 16 + o) * 16 + i];
+        for (int o = 0; o < 16; ++o) rw[((size_t)b * 16 + i) * 48 + o] = res_w[((size_t)b * 16 + o) * 16 + i];
       for (int o = 0; o < 32; ++o) rw[((size_t)b * 16 + i) * 48 + 16 + o] = w->skip_w[((size_t)b * 32 + o) * 16 + i];
     }
     if (b < 23)
-      for (int o = 0; o < 16; ++o) rb[b * 48 + o] = w->res_b[b * 16 + o];
+      for (int o = 0; o < 16; ++o) rb[b * 48 + o] = res_b[b * 16 + o];
     for (int o = 0; o < 32; ++o) rb[b * 48 + 16 + o] = w->skip_b[b * 32 + o];
   }
-  {
-    std::vector<unsigned char> blocks = wavenet_pack_blocks(gw.data(), gb.data(), rw.data(), rb.data(), w->bn_mul,
+  {  // tensor-core blobs only when they can be packed; otherwise wwb_set_precision refuses tc / tc_fast
+    std::vector<unsigned char> blocks = wavenet_pack_blocks(gw.data(), gb.data(), rw.data(), rb.data(), bn_mul.data(),
                                                             w->bn_add, N.dilation);
-    if (blocks.empty()) return fail(ctx, WWB_ERR_ARG, "WaveNet: a BatchNorm scale of 0 cannot be folded into the tensor-core path (use precision f32)");
-    if ((rc = upload(ctx, blocks, &N.tc_blocks))) return rc;
-    std::vector<unsigned char> head = wavenet_pack_head(w->bn_mul, w->bn_add, w->det1_w, w->det1_b, w->det2_w, w->det2_b);
-    if (head.empty()) return fail(ctx, WWB_ERR_ARG, "WaveNet: a BatchNorm scale of 0 cannot be folded into the tensor-core path (use precision f32)");
-    if ((rc = upload(ctx, head, &N.tc_head))) return rc;
+    std::vector<unsigned char> head = wavenet_pack_head(bn_mul.data(), w->bn_add, w->det1_w, w->det1_b, w->det2_w, w->det2_b);
+    if (blocks.empty() || head.empty()) {
+      const bool zero = std::find(bn_mul.begin(), bn_mul.end(), 0.f) != bn_mul.end();
+      ctx->tc_refused = zero ? "WaveNet: a BatchNorm scale of 0 cannot be folded into the tensor-core weights; use precision f32"
+                             : "WaveNet: a tensor-core operand (folded gate weight or bias, padding row -bn_add/bn_mul after "
+                               "the rescale, or head weight) is outside the fp16 range; use precision f32";
+    } else {
+      if ((rc = upload(ctx, blocks, &N.tc_blocks))) return rc;
+      if ((rc = upload(ctx, head, &N.tc_head))) return rc;
+    }
   }
   if ((rc = upload(ctx, gw, &N.gate_w))) return rc;
   if ((rc = upload(ctx, gb, &N.gate_b))) return rc;
@@ -267,10 +330,12 @@ int wwb_create(int device, const wwb_weights* w, int precision, wwb_ctx** out) {
     return fail(nullptr, WWB_ERR_ARG, "bad model kind");
   if (w->kind == WWB_MODEL_CRNN && w->mel_length != 151)
     return fail(nullptr, WWB_ERR_ARG, "CRNN window of %d frames unsupported (expected 151)", w->mel_length);
-  if (w->kind == WWB_MODEL_WAVENET && (w->mel_length < 17 || w->mel_length > 192))
-    return fail(nullptr, WWB_ERR_ARG, "WaveNet window of %d frames unsupported", w->mel_length);
-  if (w->kind != WWB_MODEL_NONE && w->n_out != 1 && w->n_out != 2)
-    return fail(nullptr, WWB_ERR_ARG, "n_out must be 1 or 2");
+  if (w->kind == WWB_MODEL_WAVENET && (w->mel_length < 17 || w->mel_length > 182))
+    return fail(nullptr, WWB_ERR_ARG, "WaveNet window of %d frames unsupported (expected 17..182)", w->mel_length);
+  if (w->kind == WWB_MODEL_CRNN && w->n_out != 1 && w->n_out != 2)
+    return fail(nullptr, WWB_ERR_ARG, "CRNN n_out %d unsupported (expected 1 or 2)", w->n_out);
+  if (w->kind == WWB_MODEL_WAVENET && w->n_out != 2)
+    return fail(nullptr, WWB_ERR_ARG, "WaveNet n_out %d unsupported (expected 2: the head is a 2-way softmax)", w->n_out);
   int n_dev = 0;
   cudaError_t e = cudaGetDeviceCount(&n_dev);
   if (e != cudaSuccess || n_dev == 0) {
@@ -328,6 +393,7 @@ int wwb_set_precision(wwb_ctx* ctx, int precision) {
   if (!ctx) return WWB_ERR_ARG;
   if (precision != WWB_PREC_F32 && precision != WWB_PREC_TC && precision != WWB_PREC_TC_FAST)
     return fail(ctx, WWB_ERR_ARG, "unknown precision %d", precision);
+  if (precision != WWB_PREC_F32 && !ctx->tc_refused.empty()) return fail(ctx, WWB_ERR_ARG, "%s", ctx->tc_refused.c_str());
   ctx->precision = precision;
   return WWB_OK;
 }

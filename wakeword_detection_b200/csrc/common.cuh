@@ -20,6 +20,7 @@ constexpr int kMel = 40;
 // A "segment" is up to kSegTaps consecutive non-zeros of one mel band; a band owns a
 // contiguous range of segments so partial sums are combined in a fixed order.
 constexpr int kSegTaps = 8;
+constexpr int kMaxSeg = 128;   // segments the filter kernels hold in shared memory (wwb_create refuses more)
 struct MelTables {
   int n_seg = 0;          // total segments
   int* seg_band = nullptr;   // [n_seg]
@@ -122,6 +123,7 @@ struct wwb_ctx {
   int L = 0;          // mel_length
   int n_out = 1;
   int precision = WWB_PREC_F32;
+  std::string tc_refused;   // why the model has no tensor-core weights (empty: it has them)
   int sm_count = 148;
   float mel_floor = 1e-5f, mel_log_offset = 0.f, mel_scale = 0.5f;
   wwb::MelTables mel;
@@ -240,6 +242,7 @@ int wavenet_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, floa
                             float* post, cudaStream_t st);
 int wavenet_tc_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* det_out,
                           float* post, cudaStream_t st);
+// the tensor-core operand blobs; empty if a BatchNorm scale is 0 or a packed operand is outside the fp16 range
 std::vector<unsigned char> wavenet_pack_blocks(const float* gate_w, const float* gate_b, const float* rs_w,
                                                const float* rs_b, const float* bn_mul, const float* bn_add,
                                                const int* dilation);

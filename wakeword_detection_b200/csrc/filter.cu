@@ -23,7 +23,6 @@ constexpr int F_WARPS = 12;                // independent warp pipelines per CTA
 constexpr int F_THREADS = F_WARPS * 32;    // 384 (x 168 registers = one CTA per SM)
 constexpr int F_RING = 1024;               // floats per warp ring (>= 672 live samples + 320 staged ahead)
 constexpr int MAGP = 272;                  // magnitude entries per warp (257 bins + zeroed padding read by padded taps)
-constexpr int MAX_SEG = 128;
 
 struct MelParams {
   MelTables mt;
@@ -49,7 +48,7 @@ struct __align__(16) FilterWarpSmem {
   float ring[F_RING];
   double2 xch[2][16 * f64::XP];
   float2 mag[MAGP];          // [bin] = (frame of half 0, frame of half 1): one 8-byte load serves both frames
-  float2 partial[MAX_SEG];
+  float2 partial[kMaxSeg];
 };
 
 struct __align__(16) FilterSmem {
@@ -59,8 +58,8 @@ struct __align__(16) FilterSmem {
   double2 twj[256];          // W256^(j k2) at [16 j + k2]
   // mel tables: a segment = up to 8 CONSECUTIVE bins of one band (the non-zeros of a mel band are contiguous), padded to 8
   // taps with weight 0 (fma(0, x, acc) == acc: the padded taps read the following bins / the zeroed padding); band -> segments
-  float seg_w[MAX_SEG][8];
-  int seg_bin0[MAX_SEG];
+  float seg_w[kMaxSeg][8];
+  int seg_bin0[kMaxSeg];
   int band_seg0[kMel + 1];
   float band_bias[kMel];
 };
@@ -291,7 +290,6 @@ int launch_filter(wwb_ctx* ctx, const void* pcm, int dtype, int64_t S, int64_t N
   if (S < 0 || N < 0 || pitch < N) return fail(ctx, WWB_ERR_ARG, "bad filter geometry");
   int64_t F = wwb_num_frames(N);
   if (S == 0 || F == 0) return WWB_OK;
-  if (ctx->mel.n_seg > MAX_SEG) return fail(ctx, WWB_ERR_ARG, "mel matrix has too many segments");
   FilterParams P;
   P.pcm = pcm; P.n_streams = S; P.n_samples = N; P.pitch = pitch;
   P.n_frames = F;

@@ -228,7 +228,8 @@ __global__ void __launch_bounds__(W_THREADS) wavenet_detect_kernel(const float* 
 int wavenet_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* det_out, float* post,
                             cudaStream_t st) {
   if (wm.n_win == 0) return WWB_OK;
-  if (ctx->L > W_THREADS) return fail(ctx, WWB_ERR_ARG, "WaveNet window longer than %d frames", W_THREADS);
+  // `us` holds W_T + W_PAD + 2 rows: a longer window would write past it (wwb_create refuses one)
+  if (ctx->L > W_T) return fail(ctx, WWB_ERR_ARG, "WaveNet window longer than %d frames", W_T);
   WnParams P;
   P.wm = wm; P.w = ctx->wn; P.L = ctx->L; P.enc_out = enc_out; P.det_out = det_out; P.post = post;
   wavenet_simt_kernel<<<(unsigned)wm.n_win, W_THREADS, 0, st>>>(P);

@@ -695,69 +695,73 @@ static double gate_scale(int n) { return n < 16 ? -2.8853900817779268 : -1.44269
 // so that epilogue 1 consumes the accumulator in two self-contained halves
 static int gate_col(int n) { const int c = n & 15; return (c >> 3) * 16 + (n >> 4) * 8 + (c & 7); }
 
-static void put_split(std::vector<unsigned char>& buf, size_t hi_off, size_t lo_off, float x, bool split) {
+// false if x is outside the fp16 range (hi rounds to infinity) or not finite
+static bool put_split(std::vector<unsigned char>& buf, size_t hi_off, size_t lo_off, float x, bool split) {
   __half h = __float2half_rn(x);
   __half l = split ? __float2half_rn(x - __half2float(h)) : __float2half_rn(0.f);
   memcpy(&buf[hi_off], &h, 2);
   memcpy(&buf[lo_off], &l, 2);
+  return isfinite(__half2float(h));
 }
 
 // gate_w [24][48][32] (k = tap*16+ch ; n), rs_w [24][16][48], biases, bn, dilation (fp32 device-layout copies
 // made by api.cu on the host before upload)
 // padding rows for a block whose BatchNorm is (mul, add): x_pad = -add / mul (=> u_pad = 0), as the 64-byte
-// (hi chunk 0, hi chunk 1, lo chunk 0, lo chunk 1) image of one U row.  false if a scale is 0 (cannot be folded).
+// (hi chunk 0, hi chunk 1, lo chunk 0, lo chunk 1) image of one U row.  false if a scale is 0 (cannot be folded) or
+// -add / mul is outside the fp16 range.
 static bool put_pad_rows(std::vector<unsigned char>& out, size_t off, const float* mul, const float* add) {
+  bool ok = true;
   for (int c = 0; c < 16; ++c) {
     if (mul[c] == 0.f) return false;
     const size_t o = off + (size_t)(c / 8) * 16 + (c % 8) * 2;
-    put_split(out, o, o + 32, (float)(-(double)add[c] / (double)mul[c]), true);
+    ok &= put_split(out, o, o + 32, (float)(-(double)add[c] / (double)mul[c]), true);
   }
-  return true;
+  return ok;
 }
 
 std::vector<unsigned char> wavenet_pack_blocks(const float* gate_w, const float* gate_b, const float* rs_w,
                                                const float* rs_b, const float* bn_mul, const float* bn_add,
                                                const int* dilation) {
   std::vector<unsigned char> out((size_t)24 * WN_WBLK, 0);
+  bool ok = true;
   for (int b = 0; b < 24; ++b) {
     const size_t base = (size_t)b * WN_WBLK;
     for (int k = 0; k < 48; ++k)
       for (int n = 0; n < 32; ++n) {
         const int c = k / 8, e = k % 8;
         const size_t off = base + ((size_t)c * 32 + gate_col(n)) * 16 + e * 2;
-        put_split(out, off, off + 3072, (float)((double)gate_w[((size_t)b * 48 + k) * 32 + n] * (double)bn_mul[b * 16 + k % 16] * gate_scale(n)), true);
+        ok &= put_split(out, off, off + 3072, (float)((double)gate_w[((size_t)b * 48 + k) * 32 + n] * (double)bn_mul[b * 16 + k % 16] * gate_scale(n)), true);
       }
     for (int k = 0; k < 16; ++k)
       for (int n = 0; n < 48; ++n) {
         const int c = k / 8, e = k % 8;
         const size_t off = base + WN_GATE_B + ((size_t)c * 48 + n) * 16 + e * 2;
-        put_split(out, off, off + 1536, rs_w[((size_t)b * 16 + k) * 48 + n], true);
+        ok &= put_split(out, off, off + 1536, rs_w[((size_t)b * 16 + k) * 48 + n], true);
       }
     float f[113] = {0};
     f[112] = (float)dilation[b];
     memcpy(&out[base + WN_OFF_F32], f, sizeof(f));
-    if (b < 23 && !put_pad_rows(out, base + WN_OFF_F32 + 320, bn_mul + (b + 1) * 16, bn_add + (b + 1) * 16)) return {};
+    if (b < 23) ok &= put_pad_rows(out, base + WN_OFF_F32 + 320, bn_mul + (b + 1) * 16, bn_add + (b + 1) * 16);
     // bias operands of the 'ones' GEMM: row n = (hi, lo, 0, ...); the second k-chunk stays zero
     for (int n = 0; n < 32; ++n) {
       const size_t off = base + WN_OFF_GBIAS + (size_t)gate_col(n) * 16;
       double bsum = gate_b[b * 32 + n];   // + W * bn_add (the folded BatchNorm shift)
       for (int k = 0; k < 48; ++k) bsum += (double)gate_w[((size_t)b * 48 + k) * 32 + n] * (double)bn_add[b * 16 + k % 16];
-      put_split(out, off, off + 2, (float)(bsum * gate_scale(n)), true);
+      ok &= put_split(out, off, off + 2, (float)(bsum * gate_scale(n)), true);
     }
     for (int n = 0; n < 48; ++n) {
       const size_t off = base + WN_OFF_RBIAS + (size_t)n * 16;
-      put_split(out, off, off + 2, rs_b[b * 48 + n], true);
+      ok &= put_split(out, off, off + 2, rs_b[b * 48 + n], true);
     }
   }
-  return out;
+  return ok ? out : std::vector<unsigned char>();
 }
 
 std::vector<unsigned char> wavenet_pack_head(const float* bn_mul0, const float* bn_add0, const float* det1_w_nk,
                                              const float* det1_b, const float* det2_w, const float* det2_b) {
   std::vector<unsigned char> out(sizeof(WnHead), 0);
   WnHead* h = reinterpret_cast<WnHead*>(out.data());
-  if (!put_pad_rows(out, offsetof(WnHead, pad0), bn_mul0, bn_add0)) return {};
-  h = reinterpret_cast<WnHead*>(out.data());
+  bool ok = put_pad_rows(out, offsetof(WnHead, pad0), bn_mul0, bn_add0);
   memcpy(h->det1_b, det1_b, sizeof(h->det1_b));
   memcpy(h->det2_w, det2_w, sizeof(h->det2_w));
   memcpy(h->det2_b, det2_b, sizeof(h->det2_b));
@@ -766,9 +770,9 @@ std::vector<unsigned char> wavenet_pack_head(const float* bn_mul0, const float* 
     for (int k = 0; k < 32; ++k) {
       const int c = k / 8, e = k % 8;
       const size_t off = boff + ((size_t)c * 32 + n) * 16 + e * 2;
-      put_split(out, off, off + 2048, det1_w_nk[n * 32 + k], true);
+      ok &= put_split(out, off, off + 2048, det1_w_nk[n * 32 + k], true);
     }
-  return out;
+  return ok ? out : std::vector<unsigned char>();
 }
 
 // Input layer (Wavenet/encode.tflite op 0: 1x1 conv 40 -> 16 + ReLU, SURVEY.md Appendix A3) once per mel row, fp32:
