@@ -265,6 +265,39 @@ int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_id
 /* all stages of all streams back to their initial state */
 int wwb_context_reset(wwb_ctx* ctx, void* stream);
 
+/* ---- several wake words on the same streams: [vad debounce -> trigger 0 -> ... -> trigger K-1 -> ActivationTimeout],
+ * the reference's SpeechPipeline with one WakewordTrigger stage per model (spokestack/pipeline.py:25-28 calls the
+ * stages in order with one shared SpeechContext).  Stage k is the trigger of ctxs[k]: its own model, pre_emphasis_host[k],
+ * threshold_host[k] and its own per-stream state (sample ring, previous sample, mel window, posterior max, VAD latch).
+ * ctxs[0] also holds the pipeline state (wwb_context_alloc).  Per pipeline frame and stream: the VAD debounce, then
+ * stage k = 0 .. K-1 in order with is_active = the stream's is_active at the start of the step OR the triggers of stages
+ * 0 .. k-1 in this step (a stage that sees is_active consumes nothing, as wakeword/tflite.py:139, but still records its
+ * VAD edge and resets on a fall), then the activation timeout on the merged activation.  With K = 1 this is
+ * wwb_context_step bit for bit.
+ * Stage list (checked before any device work; a rejected call changes no state of any stage): 1 <= K <= WWB_MAX_STAGES,
+ * distinct non-NULL ctxs on one device, none filter-only, ctxs[0] with wwb_context_alloc, every stage with
+ * wwb_stream_alloc of ctxs[0]'s max_streams, n (or every chunk length) within each stage's max_chunk, pre_emphasis_host
+ * and threshold_host present (WWB_ERR_ARG: K, NULL, repeated ctx, device; WWB_ERR_STATE: state, capacity, chunk).
+ * Outputs (device): post_out_dev[k] [n_streams, max_frames of stage k], n_post_out_dev[k], post_max_out_dev[k] per stage
+ * as in wwb_context_step (each array may be NULL, and so may any entry); is_speech .. deactivated per stream as in
+ * wwb_context_step (activated: some stage triggered while the stream was inactive); activated_by_out_dev int8 [n_streams]
+ * the stage that triggered, -1 if none.  Errors are reported on ctxs[0]. */
+#define WWB_MAX_STAGES 8
+int wwb_context_step_chain(wwb_ctx* const* ctxs, int n_stages, const int16_t* pcm_dev, int64_t n_streams, int64_t n,
+                           const uint8_t* vad_raw_dev, const float* pre_emphasis_host, const float* threshold_host,
+                           float* const* post_out_dev, int32_t* const* n_post_out_dev, float* const* post_max_out_dev,
+                           uint8_t* is_speech_out_dev, uint8_t* is_active_out_dev, uint8_t* activated_out_dev,
+                           uint8_t* deactivated_out_dev, int8_t* activated_by_out_dev, void* stream);
+/* wwb_context_step_chain for the slots named in ids_host, with the tables, checks and per-entry outputs of
+ * wwb_context_step_indexed; the tables are checked and staged once (ctxs[0]'s staging) for every stage. */
+int wwb_context_step_chain_indexed(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
+                                   const int32_t* len_host, const int16_t* pcm_dev, const uint8_t* vad_raw_dev,
+                                   const float* pre_emphasis_host, const float* threshold_host,
+                                   float* const* post_out_dev, int32_t* const* n_post_out_dev,
+                                   float* const* post_max_out_dev, uint8_t* is_speech_out_dev,
+                                   uint8_t* is_active_out_dev, uint8_t* activated_out_dev, uint8_t* deactivated_out_dev,
+                                   int8_t* activated_by_out_dev, void* stream);
+
 /* ---- stream state records: a stream's state out of its slot and back, to park an idle session, move it to another
  * slot, context or GPU, or rewind it.  One record per stream, of wwb_stream_state_bytes(ctx) bytes; its layout does not
  * depend on the capacity, max_chunk, precision or device of the ctx that wrote it:
@@ -322,6 +355,13 @@ int wwb_stream_export(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, void
  * none.  The pipeline's delays are per ctx and not carried.  Host-side checks as wwb_stream_export. */
 int wwb_stream_import(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const void* records_dev, int32_t* status_dev,
                       void* stream);
+/* wwb_stream_import into every stage of a trigger chain (the stage list of wwb_context_step_chain), all or nothing
+ * across the stages: records_dev[k] holds stage k's n_ids records (wwb_stream_export of a stage-k ctx; stage 0's carry
+ * the pipeline fields).  Every record of every stage is checked on the device before any is applied; status_dev int32[3]
+ * receives {0, 0, 0}, else {1 + the lowest bad entry, WWB_RECORD_*, stage} of the first stage with a bad record and no
+ * slot of any stage is touched. */
+int wwb_stream_import_chain(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
+                            const void* const* records_dev, int32_t* status_dev, void* stream);
 
 /* number of kernels this library has launched on ctx since creation (bench accounting) */
 int64_t wwb_launch_count(const wwb_ctx* ctx);

@@ -18,6 +18,7 @@ WWB_MODEL_NONE, WWB_MODEL_CRNN, WWB_MODEL_WAVENET = -1, 0, 1
 WWB_PCM_I16, WWB_PCM_F32 = 0, 1
 WWB_PREC_F32, WWB_PREC_TC, WWB_PREC_TC_FAST = 0, 1, 2
 WWB_COUNT_FRR_MAX, WWB_COUNT_FAR_EDGES = 0, 1
+WWB_MAX_STAGES = 8   # trigger stages of one chain (wwb_context_step_chain)
 PRECISIONS = {"f32": WWB_PREC_F32, "tc": WWB_PREC_TC, "tc_fast": WWB_PREC_TC_FAST}
 
 _fp = C.POINTER(C.c_float)
@@ -75,9 +76,15 @@ PROTOTYPES = {
     "wwb_context_step_indexed": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp,
                                            _vp, _vp, _vp]),
     "wwb_context_reset": (C.c_int, [_vp, _vp]),
+    "wwb_context_step_chain": (C.c_int, [C.POINTER(_vp), C.c_int, _vp, _i64, _i64, _vp, _vp, _vp, C.POINTER(_vp),
+                                         C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _vp, _vp, _vp, _vp]),
+    "wwb_context_step_chain_indexed": (C.c_int, [C.POINTER(_vp), C.c_int, _vp, _i64, _vp, _vp, _vp, _vp, _vp,
+                                                 C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _vp, _vp,
+                                                 _vp, _vp]),
     "wwb_stream_state_bytes": (_i64, [_vp]),
     "wwb_stream_export": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "wwb_stream_import": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),
+    "wwb_stream_import_chain": (C.c_int, [C.POINTER(_vp), C.c_int, _vp, _i64, C.POINTER(_vp), _vp, _vp]),
     "wwb_launch_count": (_i64, [_vp]),
     "wwb_debug_buffer": (C.c_int, [_vp, _vp]),
 }
@@ -617,6 +624,92 @@ class Engine:
 
     def context_reset(self) -> None:
         self._check(self.lib.wwb_context_reset(self.ctx, self._stream()))
+
+    # -- trigger chains: this engine's trigger and pipeline state, then one trigger stage per engine in `others` ---------
+    def _chain(self, others):
+        """(engines, ctx array) of the chain [self] + others"""
+        engines = [self] + list(others)
+        return engines, (_vp * len(engines))(*[e.ctx for e in engines])
+
+    @staticmethod
+    def _per_stage(v, K: int) -> np.ndarray:
+        """a scalar or K values -> float32 [K] host array"""
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(v, np.float32), (K,)))
+
+    def _chain_out(self, engines, S: int):
+        """the outputs of a chain step over S entries, by name in the C ABI's order: the keys of _pipeline_out with
+        post [K, S, max_frames], n_post [K, S] and post_max [K, S] per stage, then activated_by [S] int8"""
+        t = self.torch
+        K = len(engines)
+        mf = {e.stream_max_frames() for e in engines}
+        if len(mf) != 1:
+            raise ValueError("the stages take chunks of different max_frames %s; allocate them alike" % sorted(mf))
+        out = {"post": t.empty((K, S, mf.pop()), dtype=t.float32, device=self.device),
+               "n_post": t.empty((K, S), dtype=t.int32, device=self.device),
+               "post_max": t.empty((K, S), dtype=t.float32, device=self.device)}
+        for k in ("is_speech", "is_active", "activated", "deactivated"):
+            out[k] = t.empty((S,), dtype=t.uint8, device=self.device)
+        out["activated_by"] = t.empty((S,), dtype=t.int8, device=self.device)
+        return out
+
+    def _call_chain(self, fn, others, streams, vad_raw, pre_emphasis, thresholds, S: int):
+        engines, ctxs = self._chain(others)
+        K = len(engines)
+        a, thr = self._per_stage(pre_emphasis, K), self._per_stage(thresholds, K)
+        out = self._chain_out(engines, S)
+        rows = lambda x: (_vp * K)(*[x[k].data_ptr() for k in range(K)])
+        vad = self._flags(vad_raw)
+        self._check(fn(ctxs, K, *streams, None if vad is None else vad.data_ptr(), a.ctypes.data, thr.ctypes.data,
+                       rows(out["post"]), rows(out["n_post"]), rows(out["post_max"]),
+                       *[o.data_ptr() for o in list(out.values())[3:]], self._stream()))
+        return out
+
+    def context_step_chain(self, others: Sequence["Engine"], pcm, vad_raw=None, pre_emphasis=0.0, thresholds=0.5):
+        """One SpeechPipeline dispatch with one wake-word stage per engine: vad debounce -> trigger of this engine ->
+        trigger of each engine in `others` -> activation timeout (wwb_context_step_chain).  This engine holds the
+        pipeline state (context_alloc); every engine has stream state of the same capacity on the same device.
+        pre_emphasis / thresholds: one value per stage or one for all.  -> the dict of context_step with post
+        [K, S, max_frames], n_post [K, S] and post_max [K, S] per stage, plus activated_by [S] int8 (-1: none)."""
+        x = self._dense(pcm)
+        S, n = x.shape
+        return self._call_chain(self.lib.wwb_context_step_chain, others, (x.data_ptr(), S, n), vad_raw, pre_emphasis,
+                                thresholds, S)
+
+    def context_step_chain_indexed(self, others: Sequence["Engine"], ids, pcm_packed, lengths, vad_raw=None,
+                                   pre_emphasis=0.0, thresholds=0.5):
+        """context_step_chain for the slots in `ids` only, tables and packing as in stream_push_indexed."""
+        ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
+        return self._call_chain(self.lib.wwb_context_step_chain_indexed, others,
+                                (ids.ctypes.data, ids.size, lengths.ctypes.data, x.data_ptr()), vad_raw, pre_emphasis,
+                                thresholds, ids.size)
+
+    def stream_import_chain(self, others: Sequence["Engine"], ids, records) -> None:
+        """stream_import into every stage of the chain [self] + others, all or nothing across the stages: records[k]
+        (uint8 [n_ids, bytes of stage k]) from stream_export of a stage-k engine.  A bad record raises
+        ValueError("stage <k> record <i>: <reason>") and no slot of any stage is touched."""
+        t = self.torch
+        engines, ctxs = self._chain(others)
+        ids = self._state_ids(ids)
+        if len(records) != len(engines):
+            raise ValueError("%d record sets for %d stages" % (len(records), len(engines)))
+        recs = []
+        for k, (e, r) in enumerate(zip(engines, records)):
+            if isinstance(r, np.ndarray):
+                r = t.from_numpy(np.ascontiguousarray(r).view(np.uint8))
+            if r.dtype != t.uint8:
+                raise ValueError("stage %d: records must be uint8, got %s" % (k, r.dtype))
+            r = r.to(self.device).contiguous()
+            nb = e.stream_state_bytes()
+            if nb and r.numel() != ids.size * nb:
+                raise ValueError("stage %d: records hold %d bytes, %d entries need %d" % (k, r.numel(), ids.size, ids.size * nb))
+            recs.append(r)
+        status = t.zeros((3,), dtype=t.int32, device=self.device)
+        ptrs = (_vp * len(recs))(*[r.data_ptr() or None for r in recs])
+        self._check(self.lib.wwb_stream_import_chain(ctxs, len(engines), ids.ctypes.data, ids.size, ptrs,
+                                                     status.data_ptr(), self._stream()))
+        bad, why, stage = (int(v) for v in status.cpu())
+        if bad:
+            raise ValueError("stage %d record %d: %s" % (stage, bad - 1, RECORD_REASONS.get(why, "reason %d" % why)))
 
     def stream_state_bytes(self) -> int:
         """size of one stream state record (0 without stream_alloc or on a filter-only context)"""

@@ -744,6 +744,7 @@ int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, i
   if ((rc = dalloc(ctx, S, &c.trigger))) return rc;
   if ((rc = dalloc(ctx, S, &c.e_is_speech))) return rc;
   if ((rc = dalloc(ctx, S, &c.e_is_active))) return rc;
+  if ((rc = dalloc(ctx, S, &c.activated_by))) return rc;
   c.max_streams = (int64_t)S;
   return WWB_OK;
 }
@@ -770,6 +771,104 @@ int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_id
   const int32_t* ids = ctx->st.tables;
   return context_step(ctx, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out, post_max_out,
                       is_speech_out, is_active_out, activated_out, deactivated_out, st);
+}
+
+// vad debounce -> trigger stages 0 .. K-1 -> activation timeout over S entries (ids / off as in stream_push), the
+// pipeline state on ctxs[0].  Every stage reads is_speech / is_active from ctxs[0]'s per-entry scratch and writes its
+// trigger to ctxs[0]'s cs.trigger, which context_chain_kernel folds into the is_active of the next stage.
+static int context_step_chain(wwb_ctx* const* ctxs, int K, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids,
+                              const int32_t* off, const uint8_t* vad_raw, const float* a, const float* threshold,
+                              float* const* post_out, int32_t* const* n_post_out, float* const* post_max_out,
+                              uint8_t* is_speech_out, uint8_t* is_active_out, uint8_t* activated_out,
+                              uint8_t* deactivated_out, int8_t* activated_by_out, cudaStream_t st) {
+  wwb_ctx* c0 = ctxs[0];
+  ContextState& c = c0->cs;
+  int rc = launch_context_vad(c0, ids, vad_raw, S, st);
+  if (rc) return rc;
+  for (int k = 0; k < K; ++k) {
+    if ((rc = stream_push(ctxs[k], pcm, S, n, ids, off, c.e_is_speech, c.e_is_active, a[k], threshold[k],
+                          post_out ? post_out[k] : nullptr, n_post_out ? n_post_out[k] : nullptr, c.trigger,
+                          post_max_out ? post_max_out[k] : nullptr, st)))
+      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
+    if ((rc = launch_context_chain(c0, S, k, k == K - 1, activated_by_out, st))) return rc;
+  }
+  return launch_context_timeout(c0, ids, c.trigger, S, is_speech_out, is_active_out, activated_out, deactivated_out, st);
+}
+
+// The stage list of a trigger chain, reported on ctxs[0] (non-NULL): 1 <= K <= WWB_MAX_STAGES, distinct non-NULL ctxs on
+// ctxs[0]'s device, each with a model and stream state of ctxs[0]'s max_streams, ctxs[0] with pipeline state.
+static int check_chain(wwb_ctx* const* ctxs, int K) {
+  wwb_ctx* c0 = ctxs[0];
+  if (K < 1 || K > WWB_MAX_STAGES) return fail(c0, WWB_ERR_ARG, "%d stages outside [1, %d]", K, WWB_MAX_STAGES);
+  for (int k = 0; k < K; ++k) {
+    wwb_ctx* ck = ctxs[k];
+    if (!ck) return fail(c0, WWB_ERR_ARG, "stage %d: NULL ctx", k);
+    for (int j = 0; j < k; ++j)
+      if (ctxs[j] == ck) return fail(c0, WWB_ERR_ARG, "stage %d: the ctx of stage %d again (each stage needs its own)", k, j);
+    if (ck->device != c0->device)
+      return fail(c0, WWB_ERR_ARG, "stage %d: ctx on device %d, stage 0 on device %d", k, ck->device, c0->device);
+    int rc = check_state(ck, k == 0, true);
+    if (rc) return fail(c0, rc, "stage %d: %s", k, ck->err.c_str());
+    if (ck->st.max_streams != c0->st.max_streams)
+      return fail(c0, WWB_ERR_STATE, "stage %d: stream state for %lld streams, stage 0 for %lld", k,
+                  (long long)ck->st.max_streams, (long long)c0->st.max_streams);
+  }
+  return WWB_OK;
+}
+
+// chunks of n samples (len == NULL) or of len[0 .. n_ids) samples within the max_chunk of every stage after the first
+// (stage 0's is checked with its tables)
+static int check_chain_chunks(wwb_ctx* const* ctxs, int K, int64_t n, const int32_t* len, int64_t n_ids) {
+  for (int k = 1; k < K; ++k) {
+    const int64_t cap = ctxs[k]->st.max_chunk;
+    for (int64_t i = 0; i < (len ? n_ids : 1); ++i) {
+      const int64_t m = len ? len[i] : n;
+      if (m > cap)
+        return fail(ctxs[0], WWB_ERR_STATE, "stage %d: chunk of %lld samples (entry %lld) outside [1, %lld]", k,
+                    (long long)m, (long long)i, (long long)cap);
+    }
+  }
+  return WWB_OK;
+}
+
+int wwb_context_step_chain(wwb_ctx* const* ctxs, int n_stages, const int16_t* pcm, int64_t S, int64_t n,
+                           const uint8_t* vad_raw, const float* a, const float* threshold, float* const* post_out,
+                           int32_t* const* n_post_out, float* const* post_max_out, uint8_t* is_speech_out,
+                           uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out,
+                           int8_t* activated_by_out, void* stream) {
+  if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
+  wwb_ctx* c0 = ctxs[0];
+  int rc = check_chain(ctxs, n_stages);
+  if (rc) return rc;
+  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
+  if ((rc = check_dense(c0, true, S, n, pcm)) || (rc = check_chain_chunks(ctxs, n_stages, n, nullptr, 0))) return rc;
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  return context_step_chain(ctxs, n_stages, pcm, S, n, nullptr, nullptr, vad_raw, a, threshold, post_out, n_post_out,
+                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out,
+                            (cudaStream_t)stream);
+}
+
+int wwb_context_step_chain_indexed(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
+                                   const int32_t* len_host, const int16_t* pcm, const uint8_t* vad_raw, const float* a,
+                                   const float* threshold, float* const* post_out, int32_t* const* n_post_out,
+                                   float* const* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
+                                   uint8_t* activated_out, uint8_t* deactivated_out, int8_t* activated_by_out,
+                                   void* stream) {
+  if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
+  wwb_ctx* c0 = ctxs[0];
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_chain(ctxs, n_stages);
+  if (rc) return rc;
+  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
+  if ((rc = check_tables(c0, c0->cs.max_streams, ids_host, n_ids, len_host, true, pcm)) ||
+      (rc = check_chain_chunks(ctxs, n_stages, 0, len_host, n_ids)))
+    return rc;
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  if ((rc = stage_tables(c0, ids_host, n_ids, len_host, st))) return rc;
+  const int32_t* ids = c0->st.tables;
+  return context_step_chain(ctxs, n_stages, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out,
+                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out,
+                            st);
 }
 
 int wwb_context_reset(wwb_ctx* ctx, void* stream) {
@@ -822,6 +921,31 @@ int wwb_stream_import(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, cons
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   if ((rc = stage_tables(ctx, ids_host, n_ids, nullptr, st))) return rc;
   return launch_stream_import(ctx, ctx->st.tables, n_ids, records, status, st);
+}
+
+int wwb_stream_import_chain(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
+                            const void* const* records, int32_t* status, void* stream) {
+  if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
+  wwb_ctx* c0 = ctxs[0];
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_chain(ctxs, n_stages);
+  if (rc) return rc;
+  if (!records) return fail(c0, WWB_ERR_ARG, "NULL records array");
+  if ((rc = check_state_call(c0, ids_host, n_ids, records[0]))) return rc;
+  for (int k = 1; k < n_stages; ++k)
+    if (!records[k] || (uintptr_t)records[k] % 16)
+      return fail(c0, WWB_ERR_ARG, "stage %d: records NULL or not 16-byte aligned", k);
+  if (!status) return fail(c0, WWB_ERR_ARG, "NULL status");
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  if ((rc = stage_tables(c0, ids_host, n_ids, nullptr, st))) return rc;
+  // every stage's check before any scatter: a bad record of any stage leaves status[0] != 0 and every scatter idle
+  for (int k = 0; k < n_stages; ++k)
+    if ((rc = launch_stream_check_stage(ctxs[k], n_ids, records[k], status, k, st)))
+      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
+  for (int k = 0; k < n_stages; ++k)
+    if ((rc = launch_stream_scatter(ctxs[k], c0->st.tables, n_ids, records[k], status, st)))
+      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
+  return WWB_OK;
 }
 
 int64_t wwb_launch_count(const wwb_ctx* ctx) { return ctx ? ctx->launches : 0; }

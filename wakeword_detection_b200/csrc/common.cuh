@@ -113,6 +113,7 @@ struct ContextState {
   uint8_t* trigger = nullptr;        // [S] scratch: the push's trigger output
   uint8_t* e_is_speech = nullptr;    // [S] scratch: is_speech / is_active per entry of the push (context_vad_kernel)
   uint8_t* e_is_active = nullptr;
+  int8_t* activated_by = nullptr;    // [S] scratch of a trigger chain: the stage that triggered so far, -1 if none
 };
 
 }  // namespace wwb
@@ -195,7 +196,14 @@ int64_t stream_state_bytes(int L);
 int launch_stream_export(wwb_ctx* ctx, const int32_t* ids, int64_t n, void* records, cudaStream_t st);
 int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
                          cudaStream_t st);
+// the two halves of launch_stream_import for a trigger chain: the check of stage `stage`'s records into status int32[3]
+// (kept if an earlier stage's check failed), and the scatter, which does nothing unless status[0] is 0
+int launch_stream_check_stage(wwb_ctx* ctx, int64_t n, const void* records, int32_t* status, int stage, cudaStream_t st);
+int launch_stream_scatter(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, const int32_t* status,
+                          cudaStream_t st);
 int launch_context_vad(wwb_ctx* ctx, const int32_t* ids, const uint8_t* vad_raw, int64_t S, cudaStream_t st);
+// after trigger stage k of a chain (its trigger in cs.trigger): see context_chain_kernel
+int launch_context_chain(wwb_ctx* ctx, int64_t S, int k, bool last, int8_t* activated_by_out, cudaStream_t st);
 int launch_context_timeout(wwb_ctx* ctx, const int32_t* ids, const uint8_t* trigger, int64_t S, uint8_t* is_speech_out,
                            uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out, cudaStream_t st);
 

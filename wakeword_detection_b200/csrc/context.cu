@@ -9,7 +9,8 @@
 //                                                       max_active deactivates
 // One wwb_context_step = one SpeechPipeline._dispatch (spokestack/pipeline.py:25-28) for every stream: two one-thread-
 // per-stream kernels around the streaming push.  Both run over the entries i of the push, with the state of slot ids[i]
-// (ids NULL = i) and every per-entry input and output at i.
+// (ids NULL = i) and every per-entry input and output at i.  A trigger chain (wwb_context_step_chain) runs one push per
+// stage, each on its own ctx, with context_chain_kernel after each; the pipeline state and this scratch are stage 0's.
 #include "common.cuh"
 
 namespace wwb {
@@ -66,6 +67,33 @@ __global__ void context_timeout_kernel(ContextState C, const int32_t* __restrict
   if (is_active_out) is_active_out[i] = (uint8_t)act;
   if (activated_out) activated_out[i] = (uint8_t)activated;
   if (deactivated_out) deactivated_out[i] = (uint8_t)deactivated;
+}
+
+// Between the trigger stages of wwb_context_step_chain, after stage k's push wrote its trigger into C.trigger: a trigger
+// activates the stream for the stages after k (e_is_active is their is_active input) and names k as the stage that
+// activated it.  A stage triggers only while its is_active input is 0, so at most one stage per step does.  After the last
+// stage C.trigger holds the merged trigger that context_timeout_kernel reads.
+__global__ void context_chain_kernel(ContextState C, int64_t S, int k, bool last, int8_t* __restrict__ activated_by_out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= S) return;
+  const bool trig = C.trigger[i] != 0;
+  int by = k == 0 ? -1 : C.activated_by[i];
+  if (trig) {
+    by = k;
+    C.e_is_active[i] = 1;
+  }
+  if (last) {
+    C.trigger[i] = by >= 0 ? 1 : 0;
+    if (activated_by_out) activated_by_out[i] = (int8_t)by;
+  } else {
+    C.activated_by[i] = (int8_t)by;
+  }
+}
+
+int launch_context_chain(wwb_ctx* ctx, int64_t S, int k, bool last, int8_t* activated_by_out, cudaStream_t st) {
+  context_chain_kernel<<<(unsigned)((S + 127) / 128), 128, 0, st>>>(ctx->cs, S, k, last, activated_by_out);
+  WWB_CHECK_LAUNCH(ctx);
+  return WWB_OK;
 }
 
 int launch_context_vad(wwb_ctx* ctx, const int32_t* ids, const uint8_t* vad_raw, int64_t S, cudaStream_t st) {

@@ -122,9 +122,12 @@ __global__ void __launch_bounds__(kStateThreads) stream_export_kernel(const Stat
 
 // One thread per record: the first failing check of the lowest bad entry lands in import_check[0] as
 // (~entry << 32 | reason) through atomicMax; the last block to finish writes the status and clears the scratch.
+// stage < 0: status int32[2] of wwb_stream_import.  stage >= 0 (wwb_stream_import_chain, stages checked in order):
+// status int32[3] with the stage, left as it is when an earlier stage's check failed.
 __global__ void __launch_bounds__(kStateThreads) stream_check_kernel(const float4* __restrict__ records, int64_t n,
                                                                       int64_t rec4, int kind, int L,
-                                                                      unsigned long long* check, int32_t* status) {
+                                                                      unsigned long long* check, int32_t* status,
+                                                                      int stage) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
     RecordHeader r;
@@ -151,8 +154,11 @@ __global__ void __launch_bounds__(kStateThreads) stream_check_kernel(const float
   if (last && threadIdx.x == 0) {
     const unsigned long long key = atomicExch(&check[0], 0ull);
     check[1] = 0;
-    status[0] = key ? (int32_t)(0xffffffffull - (key >> 32)) + 1 : 0;
-    status[1] = (int32_t)(key & 0xffffffffull);
+    if (stage <= 0 || status[0] == 0) {
+      status[0] = key ? (int32_t)(0xffffffffull - (key >> 32)) + 1 : 0;
+      status[1] = (int32_t)(key & 0xffffffffull);
+      if (stage >= 0) status[2] = key ? stage : 0;
+    }
   }
 }
 
@@ -227,15 +233,25 @@ int launch_stream_export(wwb_ctx* ctx, const int32_t* ids, int64_t n, void* reco
   return WWB_OK;
 }
 
-int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
-                         cudaStream_t st) {
-  const StateParams P = state_params(ctx, ids, n);
+int launch_stream_check_stage(wwb_ctx* ctx, int64_t n, const void* records, int32_t* status, int stage, cudaStream_t st) {
   stream_check_kernel<<<(unsigned)((n + kStateThreads - 1) / kStateThreads), kStateThreads, 0, st>>>(
-      (const float4*)records, n, P.rec4, ctx->kind, ctx->L, ctx->st.import_check, status);
+      (const float4*)records, n, stream_state_bytes(ctx->L) / 16, ctx->kind, ctx->L, ctx->st.import_check, status, stage);
   WWB_CHECK_LAUNCH(ctx);
+  return WWB_OK;
+}
+
+int launch_stream_scatter(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, const int32_t* status,
+                          cudaStream_t st) {
+  const StateParams P = state_params(ctx, ids, n);
   stream_import_kernel<<<(unsigned)n, kStateThreads, 0, st>>>(P, (const float4*)records, status);
   WWB_CHECK_LAUNCH(ctx);
   return WWB_OK;
+}
+
+int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
+                         cudaStream_t st) {
+  int rc = launch_stream_check_stage(ctx, n, records, status, -1, st);
+  return rc ? rc : launch_stream_scatter(ctx, ids, n, records, status, st);
 }
 
 }  // namespace wwb

@@ -127,6 +127,65 @@ class MultiStreamPipeline:
         self.engine.close()
 
 
+class MultiWakewordPipeline:
+    """S speech pipelines listening for several wake words, [vad debounce -> WakewordTrigger(model 0) -> ... ->
+    WakewordTrigger(model K-1) -> ActivationTimeout], the reference's SpeechPipeline with one trigger stage per model
+    (spokestack/pipeline.py:25-28), advanced by one call with all state on the device.  Stage k sees the is_active that
+    the stages before it set in the same frame: once one stage triggers, the later ones skip that frame's chunk.
+
+    models: list of (model_dir, model_type) or dicts with model_dir, model_type and optionally posterior_threshold (0.5)
+    and pre_emphasis (0.0); each stage keeps its own filter and window state.
+    step(pcm[S, n] int16, vad_raw[S]) / step_streams(ids, frames, vad_raw) -> the dict of MultiStreamPipeline with post
+    [K, S, max_frames], n_post [K, S] and post_max [K, S] per stage, plus activated_by [S] (int8: the stage that
+    triggered, -1 if none).  export_streams(ids) -> one record tensor per stage (stage 0's carries the pipeline state);
+    import_streams(ids, records) puts them back, all or nothing across the stages."""
+
+    def __init__(self, models, n_streams: int, frame_width: int = 20, sample_rate: int = 16000, vad_rise_delay: int = 0,
+                 vad_fall_delay: int = 0, min_active: int = 500, max_active: int = 5000, device: int = 0,
+                 precision: str = "tc") -> None:
+        from . import weights as W
+        stages = [dict(m) if isinstance(m, dict) else {"model_dir": m[0], "model_type": m[1]} for m in models]
+        if not 1 <= len(stages) <= _cabi.WWB_MAX_STAGES:
+            raise ValueError("%d stages outside [1, %d]" % (len(stages), _cabi.WWB_MAX_STAGES))
+        self.n_streams = int(n_streams)
+        self.frame_samples = int(frame_width * sample_rate / 1000)
+        self.pre_emphasis = [float(m.get("pre_emphasis", 0.0)) for m in stages]
+        self.thresholds = [float(m.get("posterior_threshold", 0.5)) for m in stages]
+        self.engines = []
+        try:
+            for m in stages:
+                e = _cabi.Engine(W.load_model_dir(m["model_dir"], m["model_type"]), device, precision)
+                self.engines.append(e)
+                e.stream_alloc(self.n_streams, self.frame_samples)
+            self.engines[0].context_alloc(frame_width, vad_rise_delay, vad_fall_delay, min_active, max_active)
+        except BaseException:
+            self.close()
+            raise
+
+    def step(self, pcm, vad_raw=None):
+        return self.engines[0].context_step_chain(self.engines[1:], pcm, vad_raw, self.pre_emphasis, self.thresholds)
+
+    def step_streams(self, ids, frames, vad_raw=None):
+        pcm, lengths = _pack(frames)
+        return self.engines[0].context_step_chain_indexed(self.engines[1:], ids, pcm, lengths, vad_raw,
+                                                          self.pre_emphasis, self.thresholds)
+
+    def export_streams(self, ids):
+        return [e.stream_export(ids) for e in self.engines]
+
+    def import_streams(self, ids, records) -> None:
+        self.engines[0].stream_import_chain(self.engines[1:], ids, records)
+
+    def reset(self) -> None:
+        self.engines[0].context_reset()
+        for e in self.engines[1:]:
+            e.stream_reset()
+
+    def close(self) -> None:
+        for e in self.engines:
+            e.close()
+
+
 class WakewordTrigger:
     """Detects the presence of a wakeword in the audio input (single stream)."""
 
