@@ -136,26 +136,33 @@ def _k1_inputs(cap, n_step, seed):
 def test_one_stage_equals_context_step():
     """K = 1, CRNN tc, pre-emphasis 0.97, the golden pipeline script with rise and fall delays on 6 streams: every output
     of the dense chain step equals wwb_context_step's and every output of the indexed chain step (random subsets, ragged
-    frames, permuted ids) equals wwb_context_step_indexed's, bit for bit; activated_by is 0 exactly where a trigger fired."""
+    frames, permuted ids) equals wwb_context_step_indexed's, bit for bit; activated_by is 0 exactly where a trigger fired.
+    Launches per call: a step launches two kernels (vad, timeout) more than a push of the same shape on a ctx of the same
+    model, dense and indexed, and a one-stage chain step, which asks for activated_by, one more than the step."""
     model, a, thr, cap = "CRNN", 0.97, 0.5, 6
     cfg, rows, raws = _k1_inputs(cap, 0, 5)
     nf = min(len(r) for r in raws)
     engines = []
     try:
-        for _ in range(4):
+        for j in range(5):
             e = _cabi.Engine(load_weights(model), 0, "tc")
             e.stream_alloc(cap, FRAME)
-            e.context_alloc(**cfg)
+            if j < 4:
+                e.context_alloc(**cfg)
             engines.append(e)
-        ref, chain, iref, ichain = engines
+        ref, chain, iref, ichain, push = engines
         rng = np.random.default_rng(9)
         cur, k = np.zeros(cap, np.int64), np.zeros(cap, np.int64)
         trig = 0
         for i in range(nf):
             pcm = np.stack([r[i * FRAME:(i + 1) * FRAME] for r in rows])
             vad = np.array([r[i] for r in raws], np.uint8)
+            n0 = [e.launch_count() for e in (push, ref, chain)]
+            push.stream_push(pcm, pre_emphasis=a, threshold=thr)
             want = host(ref.context_step(pcm, vad, a, thr))
             got = host(chain.context_step_chain([], pcm, vad, a, thr))
+            d = [e.launch_count() - n for e, n in zip((push, ref, chain), n0)]
+            assert d[1:] == [d[0] + 2, d[0] + 3], (i, d)
             for key in want:
                 w, g = want[key], got[key]
                 if key in ("post", "n_post", "post_max"):
@@ -171,8 +178,12 @@ def test_one_stage_equals_context_step():
             ivad = np.array([raws[s][k[s] % nf] for s in ids], np.uint8)
             cur[ids] += lens
             k[ids] += 1
+            n0 = [e.launch_count() for e in (push, iref, ichain)]
+            push.stream_push_indexed(ids, packed, lens, pre_emphasis=a, threshold=thr)
             want = host(iref.context_step_indexed(ids, packed, lens, ivad, a, thr))
             got = host(ichain.context_step_chain_indexed([], ids, packed, lens, ivad, a, thr))
+            d = [e.launch_count() - n for e, n in zip((push, iref, ichain), n0)]
+            assert d[1:] == [d[0] + 2, d[0] + 3], (i, d)
             for key in want:
                 g = got[key][0] if key in ("post", "n_post", "post_max") else got[key]
                 assert np.array_equal(want[key], g, equal_nan=True), (i, key)

@@ -568,14 +568,22 @@ class Engine:
                 t.empty((S,), dtype=t.int32, device=self.device), t.empty((S,), dtype=t.uint8, device=self.device),
                 t.empty((S,), dtype=t.float32, device=self.device))
 
-    def _pipeline_out(self, S: int):
-        """the outputs of a step over S entries, by name in the C ABI's order"""
+    def _step_out(self, S: int, engines=None):
+        """the outputs of a step over S entries, by name in the C ABI's order: post [S, max_frames], n_post, post_max,
+        is_speech, is_active, activated, deactivated; for the chain of `engines` post [K, S, max_frames], n_post [K, S]
+        and post_max [K, S] per stage, then activated_by [S] int8"""
         t = self.torch
-        out = {"post": t.empty((S, self.stream_max_frames()), dtype=t.float32, device=self.device),
-               "n_post": t.empty((S,), dtype=t.int32, device=self.device),
-               "post_max": t.empty((S,), dtype=t.float32, device=self.device)}
+        K = () if engines is None else (len(engines),)
+        mf = {e.stream_max_frames() for e in engines or [self]}
+        if len(mf) != 1:
+            raise ValueError("the stages take chunks of different max_frames %s; allocate them alike" % sorted(mf))
+        out = {"post": t.empty(K + (S, mf.pop()), dtype=t.float32, device=self.device),
+               "n_post": t.empty(K + (S,), dtype=t.int32, device=self.device),
+               "post_max": t.empty(K + (S,), dtype=t.float32, device=self.device)}
         for k in ("is_speech", "is_active", "activated", "deactivated"):
             out[k] = t.empty((S,), dtype=t.uint8, device=self.device)
+        if engines is not None:
+            out["activated_by"] = t.empty((S,), dtype=t.int8, device=self.device)
         return out
 
     def _call(self, fn, streams, flags, pre_emphasis, threshold, outputs) -> None:
@@ -608,7 +616,7 @@ class Engine:
         n_post, post_max, is_speech, is_active, activated, deactivated."""
         x = self._dense(pcm)
         S, n = x.shape
-        out = self._pipeline_out(S)
+        out = self._step_out(S)
         self._call(self.lib.wwb_context_step, (x.data_ptr(), S, n), (vad_raw,), pre_emphasis, threshold, out.values())
         return out
 
@@ -617,7 +625,7 @@ class Engine:
         """context_step for the slots in `ids` only, tables and packing as in stream_push_indexed; vad_raw per entry ->
         the dict of context_step with one row per entry of `ids`."""
         ids, lengths, x = self._indexed(ids, pcm_packed, lengths)
-        out = self._pipeline_out(ids.size)
+        out = self._step_out(ids.size)
         self._call(self.lib.wwb_context_step_indexed, (ids.ctypes.data, ids.size, lengths.ctypes.data, x.data_ptr()),
                    (vad_raw,), pre_emphasis, threshold, out.values())
         return out
@@ -636,27 +644,11 @@ class Engine:
         """a scalar or K values -> float32 [K] host array"""
         return np.ascontiguousarray(np.broadcast_to(np.asarray(v, np.float32), (K,)))
 
-    def _chain_out(self, engines, S: int):
-        """the outputs of a chain step over S entries, by name in the C ABI's order: the keys of _pipeline_out with
-        post [K, S, max_frames], n_post [K, S] and post_max [K, S] per stage, then activated_by [S] int8"""
-        t = self.torch
-        K = len(engines)
-        mf = {e.stream_max_frames() for e in engines}
-        if len(mf) != 1:
-            raise ValueError("the stages take chunks of different max_frames %s; allocate them alike" % sorted(mf))
-        out = {"post": t.empty((K, S, mf.pop()), dtype=t.float32, device=self.device),
-               "n_post": t.empty((K, S), dtype=t.int32, device=self.device),
-               "post_max": t.empty((K, S), dtype=t.float32, device=self.device)}
-        for k in ("is_speech", "is_active", "activated", "deactivated"):
-            out[k] = t.empty((S,), dtype=t.uint8, device=self.device)
-        out["activated_by"] = t.empty((S,), dtype=t.int8, device=self.device)
-        return out
-
     def _call_chain(self, fn, others, streams, vad_raw, pre_emphasis, thresholds, S: int):
         engines, ctxs = self._chain(others)
         K = len(engines)
         a, thr = self._per_stage(pre_emphasis, K), self._per_stage(thresholds, K)
-        out = self._chain_out(engines, S)
+        out = self._step_out(S, engines)
         rows = lambda x: (_vp * K)(*[x[k].data_ptr() for k in range(K)])
         vad = self._flags(vad_raw)
         self._check(fn(ctxs, K, *streams, None if vad is None else vad.data_ptr(), a.ctypes.data, thr.ctypes.data,
@@ -692,17 +684,8 @@ class Engine:
         ids = self._state_ids(ids)
         if len(records) != len(engines):
             raise ValueError("%d record sets for %d stages" % (len(records), len(engines)))
-        recs = []
-        for k, (e, r) in enumerate(zip(engines, records)):
-            if isinstance(r, np.ndarray):
-                r = t.from_numpy(np.ascontiguousarray(r).view(np.uint8))
-            if r.dtype != t.uint8:
-                raise ValueError("stage %d: records must be uint8, got %s" % (k, r.dtype))
-            r = r.to(self.device).contiguous()
-            nb = e.stream_state_bytes()
-            if nb and r.numel() != ids.size * nb:
-                raise ValueError("stage %d: records hold %d bytes, %d entries need %d" % (k, r.numel(), ids.size, ids.size * nb))
-            recs.append(r)
+        recs = [self._records(r, ids.size, e.stream_state_bytes(), "stage %d: " % k)
+                for k, (e, r) in enumerate(zip(engines, records))]
         status = t.zeros((3,), dtype=t.int32, device=self.device)
         ptrs = (_vp * len(recs))(*[r.data_ptr() or None for r in recs])
         self._check(self.lib.wwb_stream_import_chain(ctxs, len(engines), ids.ctypes.data, ids.size, ptrs,
@@ -714,6 +697,19 @@ class Engine:
     def stream_state_bytes(self) -> int:
         """size of one stream state record (0 without stream_alloc or on a filter-only context)"""
         return int(self.lib.wwb_stream_state_bytes(self.ctx))
+
+    def _records(self, records, n_ids: int, nb: int, prefix: str = ""):
+        """records of one stage (uint8 [n_ids, nb], a tensor on any device or a numpy array) -> a contiguous uint8
+        tensor on this context's device; a wrong dtype or size raises ValueError starting with `prefix`"""
+        t = self.torch
+        if isinstance(records, np.ndarray):
+            records = t.from_numpy(np.ascontiguousarray(records).view(np.uint8))
+        if records.dtype != t.uint8:
+            raise ValueError("%srecords must be uint8, got %s" % (prefix, records.dtype))
+        rec = records.to(self.device).contiguous()
+        if nb and rec.numel() != n_ids * nb:
+            raise ValueError("%srecords hold %d bytes, %d entries need %d" % (prefix, rec.numel(), n_ids, n_ids * nb))
+        return rec
 
     def _state_ids(self, ids) -> np.ndarray:
         ids = np.ascontiguousarray(ids, np.int32)
@@ -737,14 +733,7 @@ class Engine:
         raises ValueError("record <i>: <reason>") and no slot is touched."""
         t = self.torch
         ids = self._state_ids(ids)
-        if isinstance(records, np.ndarray):
-            records = t.from_numpy(np.ascontiguousarray(records).view(np.uint8))
-        if records.dtype != t.uint8:
-            raise ValueError("records must be uint8, got %s" % records.dtype)
-        nb = self.stream_state_bytes()
-        rec = records.to(self.device).contiguous()
-        if nb and rec.numel() != ids.size * nb:
-            raise ValueError("records hold %d bytes, %d entries need %d" % (rec.numel(), ids.size, ids.size * nb))
+        rec = self._records(records, ids.size, self.stream_state_bytes())
         status = t.zeros((2,), dtype=t.int32, device=self.device)
         self._check(self.lib.wwb_stream_import(self.ctx, ids.ctypes.data, ids.size, rec.data_ptr() or None,
                                                status.data_ptr(), self._stream()))

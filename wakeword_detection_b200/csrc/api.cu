@@ -581,19 +581,6 @@ static int stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, c
                               post_max_out, st);
 }
 
-// vad debounce -> stream_push -> activation timeout over S entries (ids / off as in stream_push)
-static int context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids, const int32_t* off,
-                        const uint8_t* vad_raw, float a, float threshold, float* post_out, int32_t* n_post_out,
-                        float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out, uint8_t* activated_out,
-                        uint8_t* deactivated_out, cudaStream_t st) {
-  ContextState& c = ctx->cs;
-  int rc = launch_context_vad(ctx, ids, vad_raw, S, st);
-  if (rc) return rc;
-  if ((rc = stream_push(ctx, pcm, S, n, ids, off, c.e_is_speech, c.e_is_active, a, threshold, post_out, n_post_out,
-                        c.trigger, post_max_out, st))) return rc;
-  return launch_context_timeout(ctx, ids, c.trigger, S, is_speech_out, is_active_out, activated_out, deactivated_out, st);
-}
-
 // The state a streaming call needs: wwb_stream_alloc, with `pipeline` wwb_context_alloc too, and with `model` encoder
 // weights (not a filter-only ctx).
 static int check_state(wwb_ctx* ctx, bool pipeline, bool model) {
@@ -676,15 +663,13 @@ static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const i
   return WWB_OK;
 }
 
-// an indexed push's (`pipeline`: step's) tables: checked in the order of check_dense, then staged
-static int push_tables(wwb_ctx* ctx, bool pipeline, const int32_t* ids, int64_t n_ids, const int32_t* len,
-                       const int16_t* pcm, cudaStream_t st) {
+// the checks of an indexed push (`pipeline`: step) in the order of check_dense
+static int check_indexed(wwb_ctx* ctx, bool pipeline, const int32_t* ids, int64_t n_ids, const int32_t* len,
+                         const int16_t* pcm) {
   const int64_t cap = pipeline ? ctx->cs.max_streams : ctx->st.max_streams;
   if (!cap) return check_state(ctx, pipeline, true);
   int rc = check_tables(ctx, cap, ids, n_ids, len, true, pcm);
-  if (rc || (rc = check_state(ctx, pipeline, true))) return rc;
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  return stage_tables(ctx, ids, n_ids, len, st);
+  return rc ? rc : check_state(ctx, pipeline, true);
 }
 
 int wwb_stream_push(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* is_speech,
@@ -704,8 +689,10 @@ int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids
                             float* post_max_out, void* stream) {
   if (!ctx) return WWB_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = push_tables(ctx, false, ids_host, n_ids, len_host, pcm, st);
+  int rc = check_indexed(ctx, false, ids_host, n_ids, len_host, pcm);
   if (rc) return rc;
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  if ((rc = stage_tables(ctx, ids_host, n_ids, len_host, st))) return rc;
   const int32_t* ids = ctx->st.tables;
   return stream_push(ctx, pcm, n_ids, 0, ids, ids + n_ids, is_speech, is_active, a, threshold, post_out, n_post_out,
                      trigger_out, post_max_out, st);
@@ -749,33 +736,15 @@ int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, i
   return WWB_OK;
 }
 
-int wwb_context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* vad_raw, float a, float threshold,
-                     float* post_out, int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
-                     uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
-  if (!ctx) return WWB_ERR_ARG;
-  int rc = check_dense(ctx, true, S, n, pcm);
-  if (rc) return rc;
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  return context_step(ctx, pcm, S, n, nullptr, nullptr, vad_raw, a, threshold, post_out, n_post_out, post_max_out,
-                      is_speech_out, is_active_out, activated_out, deactivated_out, (cudaStream_t)stream);
-}
-
-int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
-                             const int16_t* pcm, const uint8_t* vad_raw, float a, float threshold, float* post_out,
-                             int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
-                             uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
-  if (!ctx) return WWB_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = push_tables(ctx, true, ids_host, n_ids, len_host, pcm, st);
-  if (rc) return rc;
-  const int32_t* ids = ctx->st.tables;
-  return context_step(ctx, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out, post_max_out,
-                      is_speech_out, is_active_out, activated_out, deactivated_out, st);
+// stage k's failure rc, reported on ctxs[0]: stage 0's as it stands, a later stage's under its number
+static int stage_fail(wwb_ctx* const* ctxs, int k, int rc) {
+  return k == 0 ? rc : fail(ctxs[0], rc, "stage %d: %s", k, ctxs[k]->err.c_str());
 }
 
 // vad debounce -> trigger stages 0 .. K-1 -> activation timeout over S entries (ids / off as in stream_push), the
 // pipeline state on ctxs[0].  Every stage reads is_speech / is_active from ctxs[0]'s per-entry scratch and writes its
-// trigger to ctxs[0]'s cs.trigger, which context_chain_kernel folds into the is_active of the next stage.
+// trigger to ctxs[0]'s cs.trigger, which context_chain_kernel folds into the is_active of the next stage.  With K = 1 and
+// no activated_by_out that kernel would change no state (cs.trigger keeps its 0 / 1), so it is not launched.
 static int context_step_chain(wwb_ctx* const* ctxs, int K, const int16_t* pcm, int64_t S, int64_t n, const int32_t* ids,
                               const int32_t* off, const uint8_t* vad_raw, const float* a, const float* threshold,
                               float* const* post_out, int32_t* const* n_post_out, float* const* post_max_out,
@@ -789,26 +758,31 @@ static int context_step_chain(wwb_ctx* const* ctxs, int K, const int16_t* pcm, i
     if ((rc = stream_push(ctxs[k], pcm, S, n, ids, off, c.e_is_speech, c.e_is_active, a[k], threshold[k],
                           post_out ? post_out[k] : nullptr, n_post_out ? n_post_out[k] : nullptr, c.trigger,
                           post_max_out ? post_max_out[k] : nullptr, st)))
-      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
-    if ((rc = launch_context_chain(c0, S, k, k == K - 1, activated_by_out, st))) return rc;
+      return stage_fail(ctxs, k, rc);
+    if ((K > 1 || activated_by_out) && (rc = launch_context_chain(c0, S, k, k == K - 1, activated_by_out, st))) return rc;
   }
   return launch_context_timeout(c0, ids, c.trigger, S, is_speech_out, is_active_out, activated_out, deactivated_out, st);
 }
 
-// The stage list of a trigger chain, reported on ctxs[0] (non-NULL): 1 <= K <= WWB_MAX_STAGES, distinct non-NULL ctxs on
-// ctxs[0]'s device, each with a model and stream state of ctxs[0]'s max_streams, ctxs[0] with pipeline state.
+// 1 <= K <= WWB_MAX_STAGES, reported on c0
+static int check_count(wwb_ctx* c0, int K) {
+  if (K < 1 || K > WWB_MAX_STAGES) return fail(c0, WWB_ERR_ARG, "%d stages outside [1, %d]", K, WWB_MAX_STAGES);
+  return WWB_OK;
+}
+
+// Stages 1 .. K-1 of a trigger chain, reported on ctxs[0] (stage 0 is checked as a single-model call): distinct non-NULL
+// ctxs on ctxs[0]'s device, each with a model and stream state of ctxs[0]'s max_streams.
 static int check_chain(wwb_ctx* const* ctxs, int K) {
   wwb_ctx* c0 = ctxs[0];
-  if (K < 1 || K > WWB_MAX_STAGES) return fail(c0, WWB_ERR_ARG, "%d stages outside [1, %d]", K, WWB_MAX_STAGES);
-  for (int k = 0; k < K; ++k) {
+  for (int k = 1; k < K; ++k) {
     wwb_ctx* ck = ctxs[k];
     if (!ck) return fail(c0, WWB_ERR_ARG, "stage %d: NULL ctx", k);
     for (int j = 0; j < k; ++j)
       if (ctxs[j] == ck) return fail(c0, WWB_ERR_ARG, "stage %d: the ctx of stage %d again (each stage needs its own)", k, j);
     if (ck->device != c0->device)
       return fail(c0, WWB_ERR_ARG, "stage %d: ctx on device %d, stage 0 on device %d", k, ck->device, c0->device);
-    int rc = check_state(ck, k == 0, true);
-    if (rc) return fail(c0, rc, "stage %d: %s", k, ck->err.c_str());
+    int rc = check_state(ck, false, true);
+    if (rc) return stage_fail(ctxs, k, rc);
     if (ck->st.max_streams != c0->st.max_streams)
       return fail(c0, WWB_ERR_STATE, "stage %d: stream state for %lld streams, stage 0 for %lld", k,
                   (long long)ck->st.max_streams, (long long)c0->st.max_streams);
@@ -831,21 +805,70 @@ static int check_chain_chunks(wwb_ctx* const* ctxs, int K, int64_t n, const int3
   return WWB_OK;
 }
 
+// The dense and the indexed step over the stages ctxs[0 .. K) (K = 1: wwb_context_step / _indexed).  Every check runs
+// before any device work, in this order: K, the per-stage arrays, stage 0 as a single-model step, the later stages, their
+// chunk lengths.  The id tables of an indexed step are staged once, on ctxs[0], and every stage reads that device copy.
+static int step_dense(wwb_ctx* const* ctxs, int K, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* vad_raw,
+                      const float* a, const float* threshold, float* const* post_out, int32_t* const* n_post_out,
+                      float* const* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out, uint8_t* activated_out,
+                      uint8_t* deactivated_out, int8_t* activated_by_out, cudaStream_t st) {
+  wwb_ctx* c0 = ctxs[0];
+  int rc = check_count(c0, K);
+  if (rc) return rc;
+  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
+  if ((rc = check_dense(c0, true, S, n, pcm)) || (rc = check_chain(ctxs, K)) ||
+      (rc = check_chain_chunks(ctxs, K, n, nullptr, 0)))
+    return rc;
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  return context_step_chain(ctxs, K, pcm, S, n, nullptr, nullptr, vad_raw, a, threshold, post_out, n_post_out,
+                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out, st);
+}
+
+static int step_indexed(wwb_ctx* const* ctxs, int K, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                        const int16_t* pcm, const uint8_t* vad_raw, const float* a, const float* threshold,
+                        float* const* post_out, int32_t* const* n_post_out, float* const* post_max_out,
+                        uint8_t* is_speech_out, uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out,
+                        int8_t* activated_by_out, cudaStream_t st) {
+  wwb_ctx* c0 = ctxs[0];
+  int rc = check_count(c0, K);
+  if (rc) return rc;
+  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
+  if ((rc = check_indexed(c0, true, ids_host, n_ids, len_host, pcm)) || (rc = check_chain(ctxs, K)) ||
+      (rc = check_chain_chunks(ctxs, K, 0, len_host, n_ids)))
+    return rc;
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  if ((rc = stage_tables(c0, ids_host, n_ids, len_host, st))) return rc;
+  const int32_t* ids = c0->st.tables;
+  return context_step_chain(ctxs, K, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out,
+                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out, st);
+}
+
+int wwb_context_step(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n, const uint8_t* vad_raw, float a, float threshold,
+                     float* post_out, int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
+                     uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  return step_dense(&ctx, 1, pcm, S, n, vad_raw, &a, &threshold, &post_out, &n_post_out, &post_max_out, is_speech_out,
+                    is_active_out, activated_out, deactivated_out, nullptr, (cudaStream_t)stream);
+}
+
+int wwb_context_step_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const int32_t* len_host,
+                             const int16_t* pcm, const uint8_t* vad_raw, float a, float threshold, float* post_out,
+                             int32_t* n_post_out, float* post_max_out, uint8_t* is_speech_out, uint8_t* is_active_out,
+                             uint8_t* activated_out, uint8_t* deactivated_out, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  return step_indexed(&ctx, 1, ids_host, n_ids, len_host, pcm, vad_raw, &a, &threshold, &post_out, &n_post_out,
+                      &post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, nullptr,
+                      (cudaStream_t)stream);
+}
+
 int wwb_context_step_chain(wwb_ctx* const* ctxs, int n_stages, const int16_t* pcm, int64_t S, int64_t n,
                            const uint8_t* vad_raw, const float* a, const float* threshold, float* const* post_out,
                            int32_t* const* n_post_out, float* const* post_max_out, uint8_t* is_speech_out,
                            uint8_t* is_active_out, uint8_t* activated_out, uint8_t* deactivated_out,
                            int8_t* activated_by_out, void* stream) {
   if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
-  wwb_ctx* c0 = ctxs[0];
-  int rc = check_chain(ctxs, n_stages);
-  if (rc) return rc;
-  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
-  if ((rc = check_dense(c0, true, S, n, pcm)) || (rc = check_chain_chunks(ctxs, n_stages, n, nullptr, 0))) return rc;
-  WWB_CUDA(c0, cudaSetDevice(c0->device));
-  return context_step_chain(ctxs, n_stages, pcm, S, n, nullptr, nullptr, vad_raw, a, threshold, post_out, n_post_out,
-                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out,
-                            (cudaStream_t)stream);
+  return step_dense(ctxs, n_stages, pcm, S, n, vad_raw, a, threshold, post_out, n_post_out, post_max_out, is_speech_out,
+                    is_active_out, activated_out, deactivated_out, activated_by_out, (cudaStream_t)stream);
 }
 
 int wwb_context_step_chain_indexed(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
@@ -855,20 +878,9 @@ int wwb_context_step_chain_indexed(wwb_ctx* const* ctxs, int n_stages, const int
                                    uint8_t* activated_out, uint8_t* deactivated_out, int8_t* activated_by_out,
                                    void* stream) {
   if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
-  wwb_ctx* c0 = ctxs[0];
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = check_chain(ctxs, n_stages);
-  if (rc) return rc;
-  if (!a || !threshold) return fail(c0, WWB_ERR_ARG, "NULL pre-emphasis or threshold array");
-  if ((rc = check_tables(c0, c0->cs.max_streams, ids_host, n_ids, len_host, true, pcm)) ||
-      (rc = check_chain_chunks(ctxs, n_stages, 0, len_host, n_ids)))
-    return rc;
-  WWB_CUDA(c0, cudaSetDevice(c0->device));
-  if ((rc = stage_tables(c0, ids_host, n_ids, len_host, st))) return rc;
-  const int32_t* ids = c0->st.tables;
-  return context_step_chain(ctxs, n_stages, pcm, n_ids, 0, ids, ids + n_ids, vad_raw, a, threshold, post_out, n_post_out,
-                            post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out,
-                            st);
+  return step_indexed(ctxs, n_stages, ids_host, n_ids, len_host, pcm, vad_raw, a, threshold, post_out, n_post_out,
+                      post_max_out, is_speech_out, is_active_out, activated_out, deactivated_out, activated_by_out,
+                      (cudaStream_t)stream);
 }
 
 int wwb_context_reset(wwb_ctx* ctx, void* stream) {
@@ -911,41 +923,45 @@ int wwb_stream_export(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, void
   return launch_stream_export(ctx, ctx->st.tables, n_ids, records, st);
 }
 
+// records[k] (n_ids each) into the slots ids_host names of stage k's ctx, all or nothing: the ids staged once on
+// ctxs[0], then every stage's check before any scatter, so that a bad record of any stage leaves status[0] != 0 and every
+// scatter idle.  `chain`: status int32[3] with the stage (wwb_stream_import_chain), else int32[2] (wwb_stream_import).
+static int import_records(wwb_ctx* const* ctxs, int K, bool chain, const int32_t* ids_host, int64_t n_ids,
+                          const void* const* records, int32_t* status, cudaStream_t st) {
+  wwb_ctx* c0 = ctxs[0];
+  WWB_CUDA(c0, cudaSetDevice(c0->device));
+  int rc = stage_tables(c0, ids_host, n_ids, nullptr, st);
+  if (rc) return rc;
+  for (int k = 0; k < K; ++k)
+    if ((rc = launch_stream_check_stage(ctxs[k], n_ids, records[k], status, chain ? k : -1, st)))
+      return stage_fail(ctxs, k, rc);
+  for (int k = 0; k < K; ++k)
+    if ((rc = launch_stream_scatter(ctxs[k], c0->st.tables, n_ids, records[k], status, st))) return stage_fail(ctxs, k, rc);
+  return WWB_OK;
+}
+
 int wwb_stream_import(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const void* records, int32_t* status,
                       void* stream) {
   if (!ctx) return WWB_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
   int rc = check_state_call(ctx, ids_host, n_ids, records);
   if (rc) return rc;
   if (!status) return fail(ctx, WWB_ERR_ARG, "NULL status");
-  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
-  if ((rc = stage_tables(ctx, ids_host, n_ids, nullptr, st))) return rc;
-  return launch_stream_import(ctx, ctx->st.tables, n_ids, records, status, st);
+  return import_records(&ctx, 1, false, ids_host, n_ids, &records, status, (cudaStream_t)stream);
 }
 
 int wwb_stream_import_chain(wwb_ctx* const* ctxs, int n_stages, const int32_t* ids_host, int64_t n_ids,
                             const void* const* records, int32_t* status, void* stream) {
   if (!ctxs || !ctxs[0]) return WWB_ERR_ARG;
   wwb_ctx* c0 = ctxs[0];
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = check_chain(ctxs, n_stages);
-  if (rc) return rc;
+  int rc = check_count(c0, n_stages);
+  if (rc || (rc = check_state(c0, true, true)) || (rc = check_chain(ctxs, n_stages))) return rc;
   if (!records) return fail(c0, WWB_ERR_ARG, "NULL records array");
   if ((rc = check_state_call(c0, ids_host, n_ids, records[0]))) return rc;
   for (int k = 1; k < n_stages; ++k)
     if (!records[k] || (uintptr_t)records[k] % 16)
       return fail(c0, WWB_ERR_ARG, "stage %d: records NULL or not 16-byte aligned", k);
   if (!status) return fail(c0, WWB_ERR_ARG, "NULL status");
-  WWB_CUDA(c0, cudaSetDevice(c0->device));
-  if ((rc = stage_tables(c0, ids_host, n_ids, nullptr, st))) return rc;
-  // every stage's check before any scatter: a bad record of any stage leaves status[0] != 0 and every scatter idle
-  for (int k = 0; k < n_stages; ++k)
-    if ((rc = launch_stream_check_stage(ctxs[k], n_ids, records[k], status, k, st)))
-      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
-  for (int k = 0; k < n_stages; ++k)
-    if ((rc = launch_stream_scatter(ctxs[k], c0->st.tables, n_ids, records[k], status, st)))
-      return k == 0 ? rc : fail(c0, rc, "stage %d: %s", k, ctxs[k]->err.c_str());
-  return WWB_OK;
+  return import_records(ctxs, n_stages, true, ids_host, n_ids, records, status, (cudaStream_t)stream);
 }
 
 int64_t wwb_launch_count(const wwb_ctx* ctx) { return ctx ? ctx->launches : 0; }

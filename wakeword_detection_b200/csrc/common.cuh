@@ -194,10 +194,8 @@ int launch_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, cudaStream
 // stream state records (stream_state.cu): ids is the device id table of n entries
 int64_t stream_state_bytes(int L);
 int launch_stream_export(wwb_ctx* ctx, const int32_t* ids, int64_t n, void* records, cudaStream_t st);
-int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
-                         cudaStream_t st);
-// the two halves of launch_stream_import for a trigger chain: the check of stage `stage`'s records into status int32[3]
-// (kept if an earlier stage's check failed), and the scatter, which does nothing unless status[0] is 0
+// an import: the check of one ctx's records into status int32[2] (stage < 0), or for stage `stage` of a chain into
+// status int32[3] (kept if an earlier stage's check failed), then the scatter, which does nothing unless status[0] is 0
 int launch_stream_check_stage(wwb_ctx* ctx, int64_t n, const void* records, int32_t* status, int stage, cudaStream_t st);
 int launch_stream_scatter(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, const int32_t* status,
                           cudaStream_t st);

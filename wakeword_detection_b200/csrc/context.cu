@@ -7,10 +7,11 @@
 //                                                       state; a trigger sets context.is_active
 //   activation timeout spokestack/activation_timeout.py:25-38  counts active frames; after min_active a VAD fall or
 //                                                       max_active deactivates
-// One wwb_context_step = one SpeechPipeline._dispatch (spokestack/pipeline.py:25-28) for every stream: two one-thread-
-// per-stream kernels around the streaming push.  Both run over the entries i of the push, with the state of slot ids[i]
-// (ids NULL = i) and every per-entry input and output at i.  A trigger chain (wwb_context_step_chain) runs one push per
-// stage, each on its own ctx, with context_chain_kernel after each; the pipeline state and this scratch are stage 0's.
+// One step = one SpeechPipeline._dispatch (spokestack/pipeline.py:25-28) for every stream: two one-thread-per-stream
+// kernels around the trigger stages.  Both run over the entries i of the push, with the state of slot ids[i] (ids NULL =
+// i) and every per-entry input and output at i.  A step runs one streaming push per trigger stage, each on its own ctx,
+// with context_chain_kernel after each; the pipeline state and this scratch are stage 0's.  wwb_context_step is a chain
+// of one stage without activated_by, where context_chain_kernel would change no state and is not launched.
 #include "common.cuh"
 
 namespace wwb {

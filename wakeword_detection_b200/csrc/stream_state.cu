@@ -248,10 +248,4 @@ int launch_stream_scatter(wwb_ctx* ctx, const int32_t* ids, int64_t n, const voi
   return WWB_OK;
 }
 
-int launch_stream_import(wwb_ctx* ctx, const int32_t* ids, int64_t n, const void* records, int32_t* status,
-                         cudaStream_t st) {
-  int rc = launch_stream_check_stage(ctx, n, records, status, -1, st);
-  return rc ? rc : launch_stream_scatter(ctx, ids, n, records, status, st);
-}
-
 }  // namespace wwb
