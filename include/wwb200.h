@@ -59,7 +59,7 @@ enum { WWB_COUNT_FRR_MAX = 0, WWB_COUNT_FAR_EDGES = 1 };
  * (FC weights [out,in]; see wakeword_detection_b200/weights.py).  Unused family = NULL. */
 typedef struct {
   int32_t kind;       /* WWB_MODEL_*                                              */
-  int32_t mel_length; /* encoder window length in mel frames: 151 (CRNN) / 17..182 (WaveNet; shipped 182) */
+  int32_t mel_length; /* encoder window length in mel frames: 17..256 (CRNN; shipped 151) / 17..182 (WaveNet; shipped 182) */
   int32_t n_out;      /* detect outputs: CRNN 1 (sigmoid) or 2 (softmax); WaveNet 2 (softmax) */
   int32_t n_mel;      /* 40 */
   int32_t n_bins;     /* 257 */
@@ -339,7 +339,8 @@ enum {
   WWB_RECORD_BAD_LENGTH = 5,  /* mel_length differs from this ctx's */
   WWB_RECORD_BAD_PENDING = 6  /* n_pending outside [0, 511] */
 };
-/* record size in bytes; 0 without wwb_stream_alloc or on a filter-only ctx */
+/* record size in bytes, 48 + 2048 + 160 * mel_length (shipped CRNN, L = 151: 26 256; shipped WaveNet, L = 182: 31 216);
+ * 0 without wwb_stream_alloc or on a filter-only ctx */
 int64_t wwb_stream_state_bytes(const wwb_ctx* ctx);
 /* Gathers the state of the slots named in ids_host (host table, the rules of wwb_stream_push_indexed: distinct, in
  * [0, max_streams), 1 <= n_ids <= max_streams) into records_dev (16-byte aligned): entry i's record at

@@ -179,7 +179,7 @@ static int build_crnn(wwb_ctx* ctx, const wwb_weights* w) {
   // conv [32][100] -> [100][32]
   if ((rc = upload(ctx, transposed(conv_w.data(), 32, 100), &C.conv_w))) return rc;
   if ((rc = upload(ctx, conv_b, &C.conv_b))) return rc;
-  if ((rc = upload(ctx, crnn_pack_conv(conv_w.data()), &C.tc_conv))) return rc;
+  if ((rc = upload(ctx, crnn_pack_conv(conv_w.data(), w->mel_length), &C.tc_conv))) return rc;
   for (int layer = 0; layer < 2; ++layer) {
     const int in = layer == 0 ? 640 : 64;
     // both directions side by side: Wt [in][192], bias [192]
@@ -328,8 +328,8 @@ int wwb_create(int device, const wwb_weights* w, int precision, wwb_ctx** out) {
     return fail(nullptr, WWB_ERR_ARG, "filter geometry %dx%d unsupported (expected %dx%d)", w->n_mel, w->n_bins, kMel, kBins);
   if (w->kind != WWB_MODEL_CRNN && w->kind != WWB_MODEL_WAVENET && w->kind != WWB_MODEL_NONE)
     return fail(nullptr, WWB_ERR_ARG, "bad model kind");
-  if (w->kind == WWB_MODEL_CRNN && w->mel_length != 151)
-    return fail(nullptr, WWB_ERR_ARG, "CRNN window of %d frames unsupported (expected 151)", w->mel_length);
+  if (w->kind == WWB_MODEL_CRNN && (w->mel_length < kCrnnMinL || w->mel_length > kCrnnMaxL))
+    return fail(nullptr, WWB_ERR_ARG, "CRNN window of %d frames unsupported (expected %d..%d)", w->mel_length, kCrnnMinL, kCrnnMaxL);
   if (w->kind == WWB_MODEL_WAVENET && (w->mel_length < 17 || w->mel_length > 182))
     return fail(nullptr, WWB_ERR_ARG, "WaveNet window of %d frames unsupported (expected 17..182)", w->mel_length);
   if (w->kind == WWB_MODEL_CRNN && w->n_out != 1 && w->n_out != 2)

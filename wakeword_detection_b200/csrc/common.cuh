@@ -224,14 +224,45 @@ struct WinMap {
 int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* det_out,
                          float* post, cudaStream_t st);
 int crnn_simt_detect(wwb_ctx* ctx, const float* enc, int64_t B, float* out, cudaStream_t st);
-std::vector<unsigned char> crnn_pack_conv(const float* conv_w);
+// Time geometry of the CRNN conv (kernel 20, stride 8, TF SAME) over a window of L frames: T = ceil(L / 8) columns and
+// 8T + 12 - L zero frames, pad_lo of them before the window.  Column t covers window frames 8t - pad_lo .. + 19; bit t
+// of padmask is set if that touches the padding.  Columns 0 and T - 1 always do, column 1 too when pad_lo = 9
+// (L = 1, 2 mod 8) and column T - 2 when pad_hi >= 9 (L = 1, 2, 3 mod 8).  For L = 151: T = 19, pad 6 / 7, columns 0, 18.
+struct CrnnGeom {
+  int T, pad_lo;
+  uint32_t padmask;
+};
+constexpr int kCrnnMinL = 17, kCrnnMaxL = 256;   // T = 3 .. 32 (padmask holds one bit per column)
+inline CrnnGeom crnn_geom(int L) {
+  CrnnGeom g;
+  g.T = (L + 7) / 8;
+  g.pad_lo = (8 * g.T + 12 - L) / 2;
+  g.padmask = 0;
+  for (int t = 0; t < g.T; ++t)
+    if (8 * t - g.pad_lo < 0 || 8 * t - g.pad_lo + 19 >= L) g.padmask |= 1u << t;
+  return g;
+}
+// conv-weight variant of column t in the shared-column path: 0 = all taps (interior columns), 1.. = the padded columns
+// in order, each with the taps that meet the padding zeroed
+__host__ __device__ __forceinline__ int crnn_variant(uint32_t padmask, int t) {
+#ifdef __CUDA_ARCH__
+  return (padmask >> t) & 1u ? 1 + __popc(padmask & ((1u << t) - 1u)) : 0;
+#else
+  return (padmask >> t) & 1u ? 1 + __builtin_popcount(padmask & ((1u << t) - 1u)) : 0;
+#endif
+}
+std::vector<unsigned char> crnn_pack_conv(const float* conv_w, int L);
 std::vector<unsigned char> crnn_pack_w1(const float* w_nk);
 // shared-column geometry of a sliding-window batch (crnn_tc.cu)
 struct CrnnShare {
   int q, nsp, Mp, F, wps, tps;
   int64_t n_streams;
+  int T;              // conv columns per window
+  uint32_t padmask;   // padded columns (CrnnGeom); the variants are 0 (unless every column is padded) and 1 .. popc
 };
 bool crnn_share_plan(const WinMap& wm, int L, CrnnShare* out);
+int crnn_share_first_variant(const CrnnShare& g);   // 1 if every column is padded (variant 0 unused), else 0
+int crnn_share_launches(const CrnnShare& g);        // front-kernel launches: one per variant in use
 size_t crnn_share_xws_bytes(const CrnnShare& g, int64_t n_streams);
 int crnn_front_tc(wwb_ctx* ctx, const WinMap& wm, float* xw1, cudaStream_t st, int mode = 0, const CrnnShare* g = nullptr,
                   int variant = 0);
@@ -241,7 +272,7 @@ int gru_rec_tc(wwb_ctx* ctx, int layer, const float* xw, float* seq_out, float* 
                unsigned char* seq_packed = nullptr);
 std::vector<unsigned char> crnn_pack_w2(const float* w_nk);
 std::vector<float> crnn_reorder_bias2(const float* bf);
-size_t crnn_seq_packed_bytes(int64_t B);
+size_t crnn_seq_packed_bytes(int64_t B, int T);
 int gru2_fused_tc(wwb_ctx* ctx, const unsigned char* seq_packed, float* last_out, int64_t B, const int32_t* n_dev,
                   cudaStream_t st);
 int wavenet_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* det_out,

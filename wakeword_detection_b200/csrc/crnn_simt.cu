@@ -3,9 +3,9 @@
 // This is the validation path of the tensor-core kernels (crnn_tc.cu): the same
 // arithmetic as CRNN/encode.tflite + detect.tflite (SURVEY.md Appendix A2) with every
 // product and sum in fp32.  Stages (global intermediates in ctx workspaces):
-//   conv   : mel window [151,40] -> ReLU(conv 5x20, stride (2,8), SAME) -> [19, 640]
-//   proj   : [B*19, in] x [in, 192] + b_in     (both directions side by side)
-//   gru    : 19 recurrent steps per direction, gates z|r|h, reset_after
+//   conv   : mel window [L,40] -> ReLU(conv 5x20, stride (2,8), SAME) -> [T, 640], T = ceil(L / 8) (CrnnGeom)
+//   proj   : [B*T, in] x [in, 192] + b_in     (both directions side by side)
+//   gru    : T recurrent steps per direction, gates z|r|h, reset_after
 //   detect : 64 -> 64 ReLU -> n_out, sigmoid / softmax
 #include <stdlib.h>
 
@@ -13,31 +13,32 @@
 
 namespace wwb {
 
-constexpr int C_T = 19, C_F = 20, C_CH = 32, C_FEAT = 640, C_H = 32, C_G = 96;
+constexpr int C_F = 20, C_CH = 32, C_FEAT = 640, C_H = 32, C_G = 96;
 constexpr int C_KF = 5, C_KT = 20, C_TAPS = 100;
-constexpr int C_PT = 6, C_PF = 1;              // SAME padding before (time, freq)
-constexpr int C_XT = 164, C_XF = 44;           // padded window in shared memory
+constexpr int C_PF = 1;                        // SAME padding before (freq); in time it is CrnnGeom::pad_lo
+constexpr int C_XF = 44;                       // padded window in shared memory: 8T + 12 rows of C_XF
 
 __global__ void __launch_bounds__(256) crnn_conv_kernel(WinMap wm, const float* __restrict__ w,
                                                         const float* __restrict__ bias,
-                                                        float* __restrict__ out, int L) {
-  __shared__ float xs[C_XT][C_XF];
+                                                        float* __restrict__ out, int L, int T, int pad_lo) {
+  extern __shared__ float xs_raw[];
+  float(*xs)[C_XF] = reinterpret_cast<float(*)[C_XF]>(xs_raw);
   __shared__ float ws[C_TAPS][C_CH];
   const int64_t b = blockIdx.x;
   if (wm.n_win_dev && b >= *wm.n_win_dev) return;
   const int tid = threadIdx.x;
-  for (int i = tid; i < C_XT * C_XF; i += 256) (&xs[0][0])[i] = 0.f;
+  for (int i = tid; i < (8 * T + 12) * C_XF; i += 256) xs_raw[i] = 0.f;
   for (int i = tid; i < C_TAPS * C_CH; i += 256) (&ws[0][0])[i] = w[i];
   __syncthreads();
   for (int i = tid; i < L * kMel; i += 256) {
     int t = i / kMel, f = i - t * kMel;
-    xs[t + C_PT][f + C_PF] = win_row(wm, b, t)[f];
+    xs[t + pad_lo][f + C_PF] = win_row(wm, b, t)[f];
   }
   __syncthreads();
   const int c = tid & 31, grp = tid >> 5;
   const float bc = bias[c];
-  float* o = out + b * (C_T * C_FEAT);
-  for (int p = grp; p < C_T * C_F; p += 8) {
+  float* o = out + b * (T * C_FEAT);
+  for (int p = grp; p < T * C_F; p += 8) {
     const int t = p / C_F, f = p - t * C_F;
     float acc = 0.f;
 #pragma unroll
@@ -98,13 +99,13 @@ __global__ void __launch_bounds__(256) sgemm_bias_kernel(const float* __restrict
 
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.0f / (1.0f + expf(-x)); }
 
-// xw: [B, 19, 192] (fwd gates | bwd gates).  4 windows x 2 directions x 32 units per block.
-// seq_out [B,19,64] (layer 1) or last_out [B,64] (layer 2).
+// xw: [B, T, 192] (fwd gates | bwd gates).  4 windows x 2 directions x 32 units per block.
+// seq_out [B,T,64] (layer 1) or last_out [B,64] (layer 2).
 __global__ void __launch_bounds__(256) gru_rec_kernel(const float* __restrict__ xw, const float* __restrict__ u_f,
                                                       const float* __restrict__ br_f, const float* __restrict__ u_b,
                                                       const float* __restrict__ br_b, float* __restrict__ seq_out,
                                                       float* __restrict__ last_out, int64_t B,
-                                                      const int32_t* __restrict__ n_dev) {
+                                                      const int32_t* __restrict__ n_dev, int T) {
   __shared__ float us[2][C_H][C_G];
   __shared__ float hs[8][C_H];
   const int tid = threadIdx.x;
@@ -121,8 +122,8 @@ __global__ void __launch_bounds__(256) gru_rec_kernel(const float* __restrict__ 
   float h = 0.f;
   hs[tid >> 5][i] = 0.f;
   __syncthreads();
-  for (int step = 0; step < C_T; ++step) {
-    const int t = dir ? (C_T - 1 - step) : step;
+  for (int step = 0; step < T; ++step) {
+    const int t = dir ? (T - 1 - step) : step;
     float az = bz, ar = brr, ah = bh;
     const float* hrow = hs[tid >> 5];
 #pragma unroll
@@ -134,7 +135,7 @@ __global__ void __launch_bounds__(256) gru_rec_kernel(const float* __restrict__ 
     }
     float xz = 0.f, xr = 0.f, xh = 0.f;
     if (live) {
-      const float* x = xw + (b * C_T + t) * (2 * C_G) + dir * C_G;
+      const float* x = xw + (b * T + t) * (2 * C_G) + dir * C_G;
       xz = x[i]; xr = x[32 + i]; xh = x[64 + i];
     }
     float z = sigmoid_f(xz + az);
@@ -144,7 +145,7 @@ __global__ void __launch_bounds__(256) gru_rec_kernel(const float* __restrict__ 
     __syncwarp();
     hs[tid >> 5][i] = h;
     __syncwarp();
-    if (live && seq_out) seq_out[(b * C_T + t) * 64 + dir * C_H + i] = h;
+    if (live && seq_out) seq_out[(b * T + t) * 64 + dir * C_H + i] = h;
   }
   if (live && last_out) last_out[b * 64 + dir * C_H + i] = h;
 }
@@ -242,7 +243,9 @@ int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* 
   const int64_t B = wm.n_win;
   if (B == 0) return WWB_OK;
   const CrnnWeights& W = ctx->crnn;
-  // chunk the batch so the intermediates stay bounded (xw: 14.6 KB per window)
+  const CrnnGeom geo = crnn_geom(ctx->L);
+  const int T = geo.T;
+  // chunk the batch so the intermediates stay bounded (xw: 768 T bytes per window, 14.6 KB at L = 151)
   // a multiple of 128 windows x 148 SMs (the recurrence kernel's wave)
   int64_t chunk = 37888;
   if (const char* e = getenv("WWB_CRNN_CHUNK")) chunk = std::max<int64_t>(128, atoll(e));
@@ -266,11 +269,12 @@ int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* 
   void *conv = nullptr, *xw, *s1, *enc_ws, *xws = nullptr;
   int rc;
   // the 48.6 KB/window conv intermediate exists only on the fp32 validation path (1.8 GB per chunk)
-  if (ctx->precision == WWB_PREC_F32 && (rc = workspace(ctx, 1, (size_t)std::min(B, chunk) * C_T * C_FEAT * 4, &conv))) return rc;
-  if (shared && (rc = workspace(ctx, 1, 3 * crnn_share_xws_bytes(sh, chunk_streams), &xws))) return rc;
-  if ((rc = workspace(ctx, 2, shared ? 16 : (size_t)((std::min(B, chunk) + 127) / 128 * 128) * C_T * 2 * C_G * 4, &xw))) return rc;
-  // layer-1 output: fp32 [B, 19, 64] (fp32 path) or the packed fp16 hi/lo operand of the fused layer-2 kernel (same bytes per value)
-  if ((rc = workspace(ctx, 3, std::max((size_t)std::min(B, chunk) * C_T * 64 * 4, crnn_seq_packed_bytes(std::min(B, chunk))), &s1))) return rc;
+  const int n_var = 1 + __builtin_popcount(geo.padmask);   // conv-weight variants of the shared-column path
+  if (ctx->precision == WWB_PREC_F32 && (rc = workspace(ctx, 1, (size_t)std::min(B, chunk) * T * C_FEAT * 4, &conv))) return rc;
+  if (shared && (rc = workspace(ctx, 1, n_var * crnn_share_xws_bytes(sh, chunk_streams), &xws))) return rc;
+  if ((rc = workspace(ctx, 2, shared ? 16 : (size_t)((std::min(B, chunk) + 127) / 128 * 128) * T * 2 * C_G * 4, &xw))) return rc;
+  // layer-1 output: fp32 [B, T, 64] (fp32 path) or the packed fp16 hi/lo operand of the fused layer-2 kernel (same bytes per value)
+  if ((rc = workspace(ctx, 3, std::max((size_t)std::min(B, chunk) * T * 64 * 4, crnn_seq_packed_bytes(std::min(B, chunk), T)), &s1))) return rc;
   if ((rc = workspace(ctx, 4, (size_t)std::min(B, chunk) * 64 * 4, &enc_ws))) return rc;
   for (int64_t b0 = 0; b0 < B; b0 += chunk) {
     const int64_t nb = std::min(chunk, B - b0);
@@ -282,18 +286,20 @@ int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* 
       sub.b0 = 0;
     }
     float* enc = enc_out ? enc_out + b0 * 64 : (float*)enc_ws;
-    const int64_t M = nb * C_T;
+    const int64_t M = nb * T;
     // both directions of a layer share one GEMM: Wt = [in][192]
     const bool tc = ctx->precision != WWB_PREC_F32;
     if (shared) {
-      // interior columns once per position, then the padded columns t = 0 / 18 (same strips, masked conv weights)
+      // interior columns once per position, then each padded column (same strips, masked conv weights)
       const size_t vbytes = crnn_share_xws_bytes(sh, nb / sh.wps);
-      for (int v = 0; v < 3; ++v)
+      for (int v = crnn_share_first_variant(sh); v < n_var; ++v)
         if ((rc = crnn_front_tc(ctx, sub, (float*)((unsigned char*)xws + v * vbytes), st, 1, &sh, v))) return rc;
     } else if (tc) {
       if ((rc = crnn_front_tc(ctx, sub, (float*)xw, st))) return rc;
     } else {
-      crnn_conv_kernel<<<(unsigned)nb, 256, 0, st>>>(sub, W.conv_w, W.conv_b, (float*)conv, ctx->L);
+      const size_t xs_bytes = (size_t)(8 * T + 12) * C_XF * sizeof(float);
+      WWB_CUDA(ctx, cudaFuncSetAttribute(crnn_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)xs_bytes));
+      crnn_conv_kernel<<<(unsigned)nb, 256, xs_bytes, st>>>(sub, W.conv_w, W.conv_b, (float*)conv, ctx->L, T, geo.pad_lo);
       WWB_CHECK_LAUNCH(ctx);
       sgemm_bias_kernel<<<dim3((unsigned)((M + 63) / 64), 3), 256, 0, st>>>((float*)conv, W.gru_w[0], W.gru_bi[0],
                                                                             (float*)xw, M, 2 * C_G, C_FEAT);
@@ -305,13 +311,13 @@ int crnn_simt_posteriors(wwb_ctx* ctx, const WinMap& wm, float* enc_out, float* 
       if ((rc = gru2_fused_tc(ctx, (unsigned char*)s1, enc, nb, wm.n_win_dev, st))) return rc;
     } else {
       gru_rec_kernel<<<(unsigned)((nb + 3) / 4), 256, 0, st>>>((float*)xw, W.gru_u[0], W.gru_br[0], W.gru_u[1],
-                                                              W.gru_br[1], (float*)s1, nullptr, nb, wm.n_win_dev);
+                                                              W.gru_br[1], (float*)s1, nullptr, nb, wm.n_win_dev, T);
       WWB_CHECK_LAUNCH(ctx);
       sgemm_bias_kernel<<<dim3((unsigned)((M + 63) / 64), 3), 256, 0, st>>>((float*)s1, W.gru_w[2], W.gru_bi[2],
                                                                             (float*)xw, M, 2 * C_G, 64);
       WWB_CHECK_LAUNCH(ctx);
       gru_rec_kernel<<<(unsigned)((nb + 3) / 4), 256, 0, st>>>((float*)xw, W.gru_u[2], W.gru_br[2], W.gru_u[3],
-                                                              W.gru_br[3], nullptr, enc, nb, wm.n_win_dev);
+                                                              W.gru_br[3], nullptr, enc, nb, wm.n_win_dev, T);
       WWB_CHECK_LAUNCH(ctx);
     }
     if (det_out || post) {

@@ -2,22 +2,23 @@
 // (precision WWB_PREC_TC / TC_FAST).  Replaces CRNN/encode.tflite op 0 (CONV_2D 5x20,
 // stride (2,8), SAME, ReLU) and the x-side FULLY_CONNECTED of the two layer-1 WHILE
 // bodies (SURVEY.md Appendix A2) for a batch of windows:
-//     mel window [151,40]  ->  xw1[b, t, 0:192] = conv_out[b, t, 0:640] . W1^T + b_in
-// (fwd gates z|r|h then bwd gates z|r|h).  The 48.6 KB/window conv output never leaves the SM.
+//     mel window [L,40]  ->  xw1[b, t, 0:192] = conv_out[b, t, 0:640] . W1^T + b_in,   t < T = ceil(L / 8)
+// (fwd gates z|r|h then bwd gates z|r|h), L = 17..256 (CrnnGeom).  The conv output (48.6 KB per window at L = 151)
+// never leaves the SM.
 //
-// One persistent CTA per SM works on tiles of 128 GEMM rows.  For independent windows a tile is 6 windows: row
-// r = wl*21 + t (wl = window in the tile, t = conv time step; 19 of every 21 rows are real) is the M index of every
-// GEMM, so one thread owns one (window, t) pair.  For sliding-window batches a tile is a STRIP of 126 consecutive conv
-// steps of one stream (CA_MODE_STRIPS below): every column is computed once per stream position instead of once per
-// window that contains it.  Everything between the producers (which frames an element holds) and the projection
+// One persistent CTA per SM works on tiles of 128 GEMM rows.  For independent windows a tile is floor(128 / (T + 2))
+// windows: row r = wl*(T+2) + t (wl = window in the tile, t = conv time step; T of every T + 2 rows are real; 6 x 21
+// rows at L = 151) is the M index of every GEMM, so one thread owns one (window, t) pair.  For sliding-window batches
+// a tile is a STRIP of 126 consecutive conv steps of one stream (CA_MODE_STRIPS below): every column is computed once
+// per stream position instead of once per window that contains it.  Everything between the producers (which frames an element holds) and the projection
 // epilogue (where a row's xw goes) is the same code in both modes.
 //
 //  * The conv is an implicit GEMM per output frequency f: D[128,32] = A_f[128,128] . Wc^T with
 //    k = (freq tap kf, time tap kt).  A_f is never materialised: the window is kept in shared
 //    memory TRANSPOSED and fp16-split, XP[freq row p][element e] = 8 consecutive time samples
-//    (16 bytes), e = wl*21 + chunk.  Because the conv's time stride is 8 = one element, the
-//    operand "row r, k-chunk (kf, j)" is XP[2f+kf][r + j]: linear in r (16 bytes per row) — the
-//    tcgen05 shared-memory descriptor reads it in place (SBO = 128, LBO = 16 or, for the chunk
+//    (16 bytes), e = wl*(T+2) + chunk: frames 8 chunk - pad_lo .. + 7 of window wl.  Because the
+//    conv's time stride is 8 = one element, the operand "row r, k-chunk (kf, j)" is XP[2f+kf][r + j]:
+//    linear in r (16 bytes per row) — the tcgen05 shared-memory descriptor reads it in place (SBO = 128, LBO = 16 or, for the chunk
 //    pair that straddles two freq taps, row pitch - 32).
 //  * XP streams through a ring of three 8-row groups (+ one mirror row so that "next row" is
 //    always physically adjacent), filled by four producer warps from the mel windows in global
@@ -37,9 +38,11 @@ namespace wwb {
 
 using namespace tc;
 
-constexpr int CA_WPT = 6;                         // windows per tile
-constexpr int CA_TP = 21;                         // row slots per window
-constexpr int CA_T = 19, CA_F = 20;
+// Window geometry (CrnnGeom): T conv steps per window, T + 2 row slots per window and floor(128 / (T + 2)) windows per
+// tile of independent windows (6 x 21 for T = 19, 3 x 34 for T = 32).  The kernels are compiled twice: with T = 19
+// (L = 145..152, the shipped models) fixed at compile time, and with T read from the parameters for every other length.
+constexpr int CA_T_SHIPPED = 19;
+constexpr int CA_F = 20;
 constexpr int CA_PITCH = 131 * 16;                // bytes per XP row (130 elements used; odd multiple of 16)
 constexpr int CA_RING_ROWS = 25;                  // 3 groups of 8 + mirror of physical row 0
 constexpr int CA_XP_PLANE = CA_RING_ROWS * CA_PITCH;
@@ -65,15 +68,15 @@ struct CaSmem {
 };
 
 // Sliding-window batches (regular grid, hop h in {1,2,4,8}) share conv columns between windows: the conv's time stride
-// is 8 frames, so column t of window j covers frames h*j + 8t - 6 .. + 13 and depends only on the POSITION INDEX
-// m = j + q*t (q = 8/h) as long as it does not touch the window's zero padding, i.e. for t = 1..17.  Those columns (and
-// their 192-wide GRU-1 input projection) are computed once per stream and position by tiles that are STRIPS of 126
-// consecutive conv steps of one stream and phase (mode 1).  The two padded columns of a window are strips as well, with
-// the padding moved from the data into the WEIGHTS: column t = 0 of window j is the conv at position m = j with the time
-// taps 0..5 zeroed (they would meet the 6 padding frames), column t = 18 the conv at m = j + 18q with taps 13..19 zeroed.
-// Each column is the same MMA sequence as in mode 0 with zero products in the same places, so the results are
-// bit-identical.  One launch per weight variant writes its own buffer
-//   xwS[variant][stream][48 float4 columns][Mp positions]     variant 0: interior, 1: t = 0, 2: t = 18
+// is 8 frames, so column t of window j covers frames h*j + 8t - pad_lo .. + 19 and depends only on the POSITION INDEX
+// m = j + q*t (q = 8/h) as long as it does not touch the window's zero padding (at L = 151: t = 1..17).  Those columns
+// (and their 192-wide GRU-1 input projection) are computed once per stream and position by tiles that are STRIPS of 126
+// consecutive conv steps of one stream and phase (mode 1).  The padded columns of a window (CrnnGeom::padmask: two, three
+// or four of them) are strips as well, with the padding moved from the data into the WEIGHTS: padded column t of window j
+// is the conv at position m = j + q*t with the time taps that would meet padding frames zeroed (L = 151: column 0 with
+// taps 0..5 zeroed, column 18 with taps 13..19).  Each column is the same MMA sequence as in mode 0 with zero products in
+// the same places, so the results are bit-identical.  One launch per weight variant writes its own buffer
+//   xwS[variant][stream][48 float4 columns][Mp positions]     variant 0: interior, crnn_variant(padmask, t): padded t
 // and the layer-1 recurrence reads 128 consecutive positions m = j0 + q*t .. of the variant that step t needs.
 enum { CA_MODE_WINDOWS = 0, CA_MODE_STRIPS = 1 };
 constexpr int CA_STRIP_ROWS = 126;
@@ -88,8 +91,9 @@ struct CaParams {
   const unsigned char* w1;      // [20][CA_W1_SLICE]
   const float* conv_b;
   const float* b_in;            // [192]
-  float* xw1;                   // mode 0: [ceil(n_win/128), 19, 48, 128] float4 (see the projection epilogue); modes 1/2: see CaShare
+  float* xw1;                   // mode 0: [ceil(n_win/128), T, 48, 128] float4 (see the projection epilogue); mode 1: see CaShare
   int L;
+  int T, pad_lo;                // CrnnGeom
   int nsplit;
   int mode;                     // CA_MODE_*
   int64_t n_tiles;              // modes 1/2 (mode 0 derives it from the window count)
@@ -110,6 +114,7 @@ __device__ __forceinline__ void split8v(const float (&x)[8], uint4& hi, uint4& l
   split_pair(x[6], x[7], hi.w, lo.w);
 }
 
+template <int kT>   // kT > 0: T fixed at compile time; 0: T = P.T
 __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   CaSmem& sm = *reinterpret_cast<CaSmem*>(smem_raw);
@@ -117,7 +122,9 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);   // warp-uniform for the compiler: role branches are uniform branches
   const int64_t n_win = P.wm.n_win_dev ? (int64_t)*P.wm.n_win_dev : P.wm.n_win;
   const int mode = P.mode;
-  const int64_t n_tiles = mode == CA_MODE_WINDOWS ? (n_win + CA_WPT - 1) / CA_WPT : P.n_tiles;
+  const int T = kT > 0 ? kT : P.T;
+  const int TP = T + 2, WPT = 128 / TP;             // row slots per window, windows per tile (mode 0)
+  const int64_t n_tiles = mode == CA_MODE_WINDOWS ? (n_win + WPT - 1) / WPT : P.n_tiles;
 
   // ---- one-time setup ----
   for (int i = tid; i < (int)(sizeof(sm.xp) / 16); i += CA_THREADS) reinterpret_cast<uint4*>(sm.xp)[i] = make_uint4(0, 0, 0, 0);
@@ -169,7 +176,7 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
     // =========================== epilogue warps: one row each ===========================
     const int q = warp;
     const int r = q * 32 + lane;
-    const int wl = r / CA_TP, t = r - wl * CA_TP;
+    const int wl = r / TP, t = r - wl * TP;
     const uint32_t tlane = tmem + ((uint32_t)(q * 32) << 16);
     uint32_t tcount = 0;
 
@@ -198,9 +205,9 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
       int64_t b;
       bool valid;
       if (mode == CA_MODE_WINDOWS) {
-        const int64_t w = tile * CA_WPT + wl;
-        valid = (wl < CA_WPT) && (t < CA_T) && (w < n_win);
-        b = (((w >> 7) * CA_T + t) * 48) * 128 + (w & 127);
+        const int64_t w = tile * WPT + wl;
+        valid = (wl < WPT) && (t < T) && (w < n_win);
+        b = (((w >> 7) * T + t) * 48) * 128 + (w & 127);
       } else {
         const int per = P.sh.q * P.sh.nsp;
         const int64_t stream = tile / per;
@@ -395,7 +402,7 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
     // =========================== XP producers ===========================
     const int pset = (warp - (CA_EPI_WARPS + CA_ROLE_WARPS)) / CA_PROD_WARPS;       // this set fills the groups with gg % 2 == pset
     const int task = tid - (CA_EPI_WARPS + CA_ROLE_WARPS + pset * CA_PROD_WARPS) * 32;   // 0..127; element e = task
-    const bool has_task = mode == CA_MODE_WINDOWS ? task < CA_WPT * CA_TP : true;
+    const bool has_task = mode == CA_MODE_WINDOWS ? task < WPT * TP : true;
     uint32_t gg = 0;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
       // element `task` of the tile = 8 consecutive frames f0 .. f0+7 (relative to `start` of stream s), valid in [0, fhi)
@@ -403,11 +410,11 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
       int start = 0, f0, fhi;
       bool live;
       if (mode == CA_MODE_WINDOWS) {
-        const int wl = task / CA_TP, c = task - wl * CA_TP;   // window in tile, time chunk (frames 8c-6 .. 8c+1)
-        const int64_t b = tile * CA_WPT + wl;
+        const int wl = task / TP, c = task - wl * TP;   // window in tile, time chunk (frames 8c - pad_lo .. + 7)
+        const int64_t b = tile * WPT + wl;
         live = has_task && b < n_win;
         if (live) win_origin(P.wm, b, s, start);
-        f0 = 8 * c - 6;
+        f0 = 8 * c - P.pad_lo;
         fhi = P.L;
       } else {
         const int per = P.sh.q * P.sh.nsp;
@@ -415,7 +422,7 @@ __global__ void __launch_bounds__(CA_THREADS, 1) crnn_front_tc_kernel(const CaPa
         const int rem = (int)(tile - s * per);
         const int k = rem / P.sh.q, phase = rem - k * P.sh.q;
         live = true;
-        f0 = (8 / P.sh.q) * phase + 8 * (CA_STRIP_ROWS * k + task) - 6;
+        f0 = (8 / P.sh.q) * phase + 8 * (CA_STRIP_ROWS * k + task) - P.pad_lo;
         fhi = P.sh.F;
       }
       for (int g = 0; g < CA_GROUPS; ++g, ++gg) {
@@ -476,20 +483,27 @@ static void put_split16(std::vector<unsigned char>& buf, size_t hi_off, size_t l
   memcpy(&buf[lo_off], &l, 2);
 }
 
-// conv_w [32][5][20] -> 3 variants x [plane][16 chunks][32 channels][8 halves]; chunk q = kf*3 + j holds time taps 8j..8j+7.
-// Variant 0: all taps; 1: taps 0..5 zeroed (column t = 0 of a window: its first 6 frames are padding); 2: taps 13..19
-// zeroed (column t = 18: frames 151.. are padding)
-std::vector<unsigned char> crnn_pack_conv(const float* conv_w) {
-  std::vector<unsigned char> out((size_t)3 * 2 * CA_CW_PLANE, 0);
-  for (int v = 0; v < 3; ++v)
+// conv_w [32][5][20] -> 1 + popc(padmask) variants x [plane][16 chunks][32 channels][8 halves]; chunk q = kf*3 + j holds
+// time taps 8j..8j+7.  Variant 0: all taps; variant crnn_variant(padmask, t) of a padded column t: the taps kt whose
+// window frame 8t - pad_lo + kt lies outside 0..L-1 zeroed (L = 151: variant 1 = column 0 with taps 0..5 zeroed,
+// variant 2 = column 18 with taps 13..19 zeroed)
+std::vector<unsigned char> crnn_pack_conv(const float* conv_w, int L) {
+  const CrnnGeom geo = crnn_geom(L);
+  const int n_var = 1 + __builtin_popcount(geo.padmask);
+  std::vector<unsigned char> out((size_t)n_var * 2 * CA_CW_PLANE, 0);
+  for (int v = 0; v < n_var; ++v) {
+    int col = -1;   // the padded column of variant v (none for variant 0)
+    for (int t = 0; t < geo.T; ++t)
+      if (v && crnn_variant(geo.padmask, t) == v) col = t;
     for (int q = 0; q < 15; ++q)
       for (int n = 0; n < 32; ++n)
         for (int e = 0; e < 8; ++e) {
-          const int kf = q / 3, kt = (q % 3) * 8 + e;
-          if (kt >= 20 || (v == 1 && kt < 6) || (v == 2 && kt >= 13)) continue;
+          const int kf = q / 3, kt = (q % 3) * 8 + e, frame = 8 * col - geo.pad_lo + kt;
+          if (kt >= 20 || (col >= 0 && (frame < 0 || frame >= L))) continue;
           const size_t off = (size_t)v * 2 * CA_CW_PLANE + ((size_t)q * 32 + n) * 16 + e * 2;
           put_split16(out, off, off + CA_CW_PLANE, conv_w[(n * 5 + kf) * 20 + kt]);
         }
+  }
   return out;
 }
 
@@ -506,6 +520,11 @@ std::vector<unsigned char> crnn_pack_w1(const float* w_nk) {
   return out;
 }
 
+// the front-kernel launches of the shared-column path: one per conv-weight variant in use (variant 0 is not when every
+// column is padded, L = 17, 18)
+int crnn_share_first_variant(const CrnnShare& g) { return g.padmask + 1 == (1ull << g.T) ? 1 : 0; }
+int crnn_share_launches(const CrnnShare& g) { return 1 + __builtin_popcount(g.padmask) - crnn_share_first_variant(g); }
+
 // geometry of the shared-column path for a regular window grid; false if the grid does not qualify
 bool crnn_share_plan(const WinMap& wm, int L, CrnnShare* out) {
   if (wm.win_stream || wm.n_win_dev || wm.b0 != 0 || wm.win_per_stream < 2) return false;
@@ -514,18 +533,21 @@ bool crnn_share_plan(const WinMap& wm, int L, CrnnShare* out) {
   const int wps = wm.win_per_stream;
   if (wm.n_win % wps) return false;
   if ((int64_t)(wps - 1) * hop + L > wm.ring) return false;   // a window would wrap around the ring
+  const CrnnGeom geo = crnn_geom(L);
   CrnnShare g;
   g.q = 8 / hop;
   g.wps = wps;
   g.tps = (wps + 127) / 128;
   g.F = (wps - 1) * hop + L;
-  const int m_max = wps - 1 + 18 * g.q;   // column t = 18 of the last window (variant 2 strips)
+  g.T = geo.T;
+  g.padmask = geo.padmask;
+  const int m_max = wps - 1 + (geo.T - 1) * g.q;   // column T - 1 of the last window
   g.nsp = (m_max / g.q + 1 + CA_STRIP_ROWS - 1) / CA_STRIP_ROWS;
   g.Mp = g.q * CA_STRIP_ROWS * g.nsp;
   g.n_streams = wm.n_win / wps;
-  // worth it only if it is fewer tiles than 6 windows per tile
-  const int64_t tiles_shared = 3 * g.n_streams * g.q * g.nsp;
-  if (tiles_shared >= (wm.n_win + CA_WPT - 1) / CA_WPT) return false;
+  // worth it only if it is fewer tiles than the per-window tiles (128 / (T + 2) windows each)
+  const int64_t tiles_shared = crnn_share_launches(g) * g.n_streams * g.q * g.nsp;
+  if (tiles_shared >= (wm.n_win + 128 / (geo.T + 2) - 1) / (128 / (geo.T + 2))) return false;
   *out = g;
   return true;
 }
@@ -536,8 +558,12 @@ int crnn_front_tc(wwb_ctx* ctx, const WinMap& wm, float* xw1, cudaStream_t st, i
   if (wm.n_win == 0) return WWB_OK;
   CaParams P;
   memset(&P, 0, sizeof(P));
+  const CrnnGeom geo = crnn_geom(ctx->L);
   P.mode = mode;
-  int64_t n_tiles = (wm.n_win + CA_WPT - 1) / CA_WPT;
+  P.T = geo.T;
+  P.pad_lo = geo.pad_lo;
+  const int wpt = 128 / (geo.T + 2);
+  int64_t n_tiles = (wm.n_win + wpt - 1) / wpt;
   if (mode != CA_MODE_WINDOWS) {
     P.sh = *g;
     n_tiles = (wm.n_win / g->wps) * g->q * g->nsp;
@@ -553,9 +579,10 @@ int crnn_front_tc(wwb_ctx* ctx, const WinMap& wm, float* xw1, cudaStream_t st, i
   P.nsplit = ctx->precision == WWB_PREC_TC ? 3 : 1;
   P.dbg = reinterpret_cast<long long*>(ctx->debug_buf);
   const size_t smem = sizeof(CaSmem) + 128;
-  WWB_CUDA(ctx, cudaFuncSetAttribute(crnn_front_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = geo.T == CA_T_SHIPPED ? crnn_front_tc_kernel<CA_T_SHIPPED> : crnn_front_tc_kernel<0>;
+  WWB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const unsigned grid = (unsigned)std::min<int64_t>(n_tiles, ctx->sm_count);
-  crnn_front_tc_kernel<<<grid, CA_THREADS, smem, st>>>(P);
+  kernel<<<grid, CA_THREADS, smem, st>>>(P);
   WWB_CHECK_LAUNCH(ctx);
   return WWB_OK;
 }
@@ -570,13 +597,12 @@ int crnn_front_tc(wwb_ctx* ctx, const WinMap& wm, float* xw1, cudaStream_t st, i
 //                z = sig(xz + hz), r = sig(xr + hr), c = tanh(xh + r*(hh + b_h)), h = c + z*(h - c)
 // xw (the input projection incl. b_in and the z/r parts of the recurrent bias) comes from global
 // memory, one 384-byte row per (window, t, dir).  Warps 0-3 run the forward direction (t = s),
-// warps 4-7 the backward one (t = 18 - s); each thread owns one window: its h[32] stays in
+// warps 4-7 the backward one (t = T - 1 - s); each thread owns one window: its h[32] stays in
 // registers, the fp16-split copy in shared memory is the A operand of the next step.
 namespace wwb {
 
 using namespace tc;
 
-constexpr int GR_T = 19;
 constexpr int GR_H_BYTES = 2 * 4 * 128 * 16;     // hi + lo planes, K = 32
 constexpr int GR_U_BYTES = 2 * 4 * 96 * 16;
 constexpr int GR_EPI_WARPS = 16;                 // 2 directions x 4 lane quadrants x 2 unit halves: TWO threads per (window, direction),
@@ -606,15 +632,18 @@ struct GrSmem {
 };
 
 struct GrParams {
-  const float* xw;              // [ceil(B/128), 19, 48, 128] float4
-  const float* xws;             // shared-column mode (else null): [3 variants][stream][48][Mp] float4 by position (CrnnShare)
+  const float* xw;              // [ceil(B/128), T, 48, 128] float4
+  const float* xws;             // shared-column mode (else null): [variant][stream][48][Mp] float4 by position (CrnnShare)
   size_t xws_variant;           // bytes between two variants
   int q, Mp, wps;               // shared-column geometry (CrnnShare)
+  uint32_t padmask;             // padded columns: step t reads variant crnn_variant(padmask, t)
+  int ring;                     // position-ring mode (see the kernel)
+  int T;                        // steps (conv columns per window)
   const unsigned char* u;       // [2][GR_U_BYTES] packed
   const float* bh;              // [2][32]  recurrent bias of the candidate gate
-  float* seq_out;               // [B, 19, 64] or null
+  float* seq_out;               // [B, T, 64] or null
   unsigned char* seq_packed;    // or null: the layer's output sequence as the fp16 hi/lo A operand of the next layer's input
-                                // projection, [ceil(B/128)][19][plane hi, lo][8 chunks][128 windows][8 halves] (gru2_fused_tc_kernel)
+                                // projection, [ceil(B/128)][T][plane hi, lo][8 chunks][128 windows][8 halves] (gru2_fused_tc_kernel)
   float* last_out;              // [B, 64] or null
   int64_t n_win;
   const int32_t* n_win_dev;
@@ -681,6 +710,7 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8])
 // (busy-polling issuer: 2.127 vs 2.129 ms - no difference once the loader has its own warp)
 #define GR_ISS_WAIT(bar, par) mbar_wait(bar, par)
 
+template <int kT>   // kT > 0: T fixed at compile time; 0: T = P.T
 __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   GrSmem& sm = *reinterpret_cast<GrSmem*>(smem_raw);
@@ -693,14 +723,17 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
   // (4 at hop 2), so 124 of 128 positions of a step's slab are the previous step's.  Reloading whole slabs was 3.1 GB of
   // L2 -> SM traffic per launch (probe: the same kernel without the reloads 2.19 instead of 2.68 ms CRNN stage; with the
   // ring 2.53 - the three whole-slab loads a tile still needs have one step of lead time each).  In ring mode
-  // the interior steps t = 1..17 of a tile and direction share ONE stage buffer as a ring over positions: 128 positions are
+  // the interior steps t = 1..T-2 of a tile and direction share ONE stage buffer as a ring over positions: 128 positions are
   // loaded once, each later step adds q (row = position modulo the ring size; a tile that touches two streams keeps one
   // ring per stream: n_A + 4 and n_B + 4 rows of the buffer's 128, hence tiles of 120 windows).  The padded columns
-  // t = 0 / 18 come from their own variants and use the direction's other buffer, loaded while the ring steps run; the two
+  // t = 0 / T-1 come from their own variants and use the direction's other buffer, loaded while the ring steps run; the two
   // buffers swap roles from tile to tile so that every large load has a step of lead time.  The barrier protocol is
-  // unchanged: load n may be issued once step n - 2 of the direction has been consumed.
-  const bool ring = shared && P.wps >= GR_TW && P.q == 4;
+  // unchanged: load n may be issued once step n - 2 of the direction has been consumed.  The host sets P.ring only if the
+  // padded columns are exactly t = 0 and T - 1: lengths with a third or fourth padded column (L = 1, 2, 3 mod 8) read
+  // whole slabs per step instead, since a padded step 1 or T - 2 would need a third buffer role.
+  const bool ring = P.ring != 0;
   const int TW = ring ? GR_TW : 128;
+  const int T = kT > 0 ? kT : P.T;
   const int64_t n_tiles = (n_win + TW - 1) / TW;
 
   for (int i = tid; i < (int)(2 * GR_U_BYTES / 16); i += GR_THREADS)
@@ -744,13 +777,13 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
       float h[16];
 #pragma unroll
       for (int i = 0; i < 16; ++i) h[i] = 0.f;
-      for (int s = 0; s < GR_T; ++s, ++n_x) {
-        const int t = d ? GR_T - 1 - s : s;
+      for (int s = 0; s < T; ++s, ++n_x) {
+        const int t = d ? T - 1 - s : s;
         // this direction's xw slab of the step was fetched by the TMA engine one step ahead (per-thread loads could
         // prefetch only one 400-clock chunk ahead of ~1500 clocks of DRAM latency)
         const int xs = n_x % GR_XST;
         mbar_wait(&sm.x_full[d][xs], (n_x / GR_XST) & 1);
-        const bool vstep = s == 0 || s == GR_T - 1;
+        const bool vstep = s == 0 || s == T - 1;
         const int xbuf = ring ? (int)((n_tl & 1) ^ (vstep ? 0u : 1u)) : xs;
         const int xrow = ring && !vstep ? rbase + ridx : r;
         const float4* xp = reinterpret_cast<const float4*>(sm.x[d][xbuf]) + xrow + (ub / 4) * 128;
@@ -803,7 +836,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
         uint32_t hr8[8], lr8[8];
 #pragma unroll
         for (int c = 0; c < 8; ++c) split_pair(h[2 * c], h[2 * c + 1], hr8[c], lr8[c]);
-        if (s < GR_T - 1) {
+        if (s < T - 1) {
           fence_before_sync();
           tmem_st8(th, hr8);
           tmem_st8(th + 16, lr8);
@@ -813,12 +846,12 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
           if (lane == 0) mbar_arrive(&sm.h_ready[d]);
         }
         if (valid && P.seq_out) {
-          float4* dst = reinterpret_cast<float4*>(P.seq_out + (b * GR_T + t) * 64 + d * 32 + ub);
+          float4* dst = reinterpret_cast<float4*>(P.seq_out + (b * T + t) * 64 + d * 32 + ub);
 #pragma unroll
           for (int i = 0; i < 4; ++i) dst[i] = make_float4(h[4 * i], h[4 * i + 1], h[4 * i + 2], h[4 * i + 3]);
         }
         if (valid && P.seq_packed) {   // the split computed for the recurrent GEMM is the next layer's A operand: 512 contiguous bytes per warp store
-          unsigned char* dst = P.seq_packed + ((size_t)((b >> 7) * GR_T + t) * G2_A_BYTES) + (size_t)((d * 4 + half * 2) * 128 + (int)(b & 127)) * 16;
+          unsigned char* dst = P.seq_packed + ((size_t)((b >> 7) * T + t) * G2_A_BYTES) + (size_t)((d * 4 + half * 2) * 128 + (int)(b & 127)) * 16;
 #pragma unroll
           for (int u = 0; u < 2; ++u) {
             *reinterpret_cast<uint4*>(dst + u * 2048) = make_uint4(hr8[4 * u], hr8[4 * u + 1], hr8[4 * u + 2], hr8[4 * u + 3]);
@@ -847,10 +880,10 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
         if (lane == 0) ok = mbar_test_wait(&sm.x_empty[dd][xs], ((n_ld[dd] / GR_XST) & 1) ^ 1) ? 1u : 0u;
         if (!__shfl_sync(0xffffffffu, ok, 0)) return;
       }
-      const int t = dd ? GR_T - 1 - ld_s[dd] : ld_s[dd];
+      const int t = dd ? T - 1 - ld_s[dd] : ld_s[dd];
       if (ring) {
         const int s = ld_s[dd];
-        const bool vstep = s == 0 || s == GR_T - 1;
+        const bool vstep = s == 0 || s == T - 1;
         unsigned char* const buf = sm.x[dd][(ld_tl[dd] & 1) ^ (vstep ? 0u : 1u)];
         const int64_t b0 = ld_tile[dd] * TW;
         const int nrows = (int)(n_win - b0 < TW ? n_win - b0 : TW);
@@ -858,7 +891,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
         const int j0 = (int)(b0 - stream0 * P.wps);
         const int nA = nrows < P.wps - j0 ? nrows : P.wps - j0;
         const int nseg = nrows > nA ? 2 : 1;
-        const unsigned char* base = reinterpret_cast<const unsigned char*>(P.xws) + (t == 0 ? 1 : t == GR_T - 1 ? 2 : 0) * P.xws_variant;
+        const unsigned char* base = reinterpret_cast<const unsigned char*>(P.xws) + crnn_variant(P.padmask, t) * P.xws_variant;
         const bool full = vstep || s == 1;   // a whole slab: the padded column of the step, or the ring's first 128 positions
         if (full) {
           if (lane == 0) mbar_arrive_expect_tx(&sm.x_full[dd][xs], (uint32_t)nrows * 24 * 16);
@@ -902,14 +935,14 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
       } else if (shared) {
         // the tile's windows b0.. are dense over (stream, j): at step t they sit at consecutive positions m = j + q*t of
         // their stream, so a slab is one run of positions per stream the tile touches, times 24 column rows; the padded
-        // columns t = 0 / 18 come from their own variants of the strip computation
+        // columns come from their own variants of the strip computation
         const int64_t b0 = ld_tile[dd] * 128;
         const int nrows = (int)(n_win - b0 < 128 ? n_win - b0 : 128);
         if (lane == 0) mbar_arrive_expect_tx(&sm.x_full[dd][xs], (uint32_t)nrows * 24 * 16);
         __syncwarp();
         int64_t stream = b0 / P.wps;
         int j = (int)(b0 - stream * P.wps);
-        const unsigned char* base = reinterpret_cast<const unsigned char*>(P.xws) + (t == 0 ? 1 : t == GR_T - 1 ? 2 : 0) * P.xws_variant;
+        const unsigned char* base = reinterpret_cast<const unsigned char*>(P.xws) + crnn_variant(P.padmask, t) * P.xws_variant;
         for (int row = 0; row < nrows; ++stream, j = 0) {
           const int n = nrows - row < P.wps - j ? nrows - row : P.wps - j;
           if (lane < 24)
@@ -919,11 +952,11 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
         }
       } else if (lane == 0) {
         mbar_arrive_expect_tx(&sm.x_full[dd][xs], GR_X_BYTES);
-        bulk_g2s(sm.x[dd][xs], reinterpret_cast<const unsigned char*>(P.xw) + ((size_t)(ld_tile[dd] * GR_T + t) * 48 + dd * 24) * 128 * 16,
+        bulk_g2s(sm.x[dd][xs], reinterpret_cast<const unsigned char*>(P.xw) + ((size_t)(ld_tile[dd] * T + t) * 48 + dd * 24) * 128 * 16,
                  GR_X_BYTES, &sm.x_full[dd][xs]);
       }
       ++n_ld[dd];
-      if (++ld_s[dd] == GR_T) { ld_s[dd] = 0; ld_tile[dd] += gridDim.x; ++ld_tl[dd]; }
+      if (++ld_s[dd] == T) { ld_s[dd] = 0; ld_tile[dd] += gridDim.x; ++ld_tl[dd]; }
     };
     while (ld_tile[0] < n_tiles || ld_tile[1] < n_tiles) {
       const uint32_t before = n_ld[0] + n_ld[1];
@@ -938,7 +971,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru_rec_tc_kernel(const GrParam
     uint32_t n_h = 0;
     const uint64_t db0 = make_desc(smem_u32(sm.u[0]), 1536, 128), db1 = make_desc(smem_u32(sm.u[1]), 1536, 128);
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int s = 1; s < GR_T; ++s, ++n_h) {
+      for (int s = 1; s < T; ++s, ++n_h) {
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
           GR_ISS_WAIT(&sm.h_ready[d], n_h & 1);
@@ -988,12 +1021,16 @@ int gru_rec_tc(wwb_ctx* ctx, int layer, const float* xw, float* seq_out, float* 
   GrParams P;
   memset(&P, 0, sizeof(P));
   P.xw = xw;
+  const int T = crnn_geom(ctx->L).T;
+  P.T = T;
   int64_t n_tiles = (B + 127) / 128;
   if (xws) {
     P.xws = xws;
     P.q = g->q; P.Mp = g->Mp; P.wps = g->wps;
+    P.padmask = g->padmask;
     P.xws_variant = crnn_share_xws_bytes(*g, B / g->wps);
-    if (g->wps >= GR_TW && g->q == 4) n_tiles = (B + GR_TW - 1) / GR_TW;   // position-ring mode (see the kernel)
+    P.ring = g->wps >= GR_TW && g->q == 4 && g->padmask == (1u | 1u << (T - 1));
+    if (P.ring) n_tiles = (B + GR_TW - 1) / GR_TW;   // position-ring mode (see the kernel)
   }
   P.u = ctx->crnn.tc_u[layer];
   P.bh = ctx->crnn.tc_bh[layer];
@@ -1004,9 +1041,10 @@ int gru_rec_tc(wwb_ctx* ctx, int layer, const float* xw, float* seq_out, float* 
   P.n_win_dev = n_dev;
   P.nsplit = ctx->precision == WWB_PREC_TC ? 3 : 1;
   const size_t smem = sizeof(GrSmem) + 128;
-  WWB_CUDA(ctx, cudaFuncSetAttribute(gru_rec_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = T == CA_T_SHIPPED ? gru_rec_tc_kernel<CA_T_SHIPPED> : gru_rec_tc_kernel<0>;
+  WWB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const unsigned grid = (unsigned)std::min<int64_t>(n_tiles, (int64_t)ctx->sm_count);
-  gru_rec_tc_kernel<<<grid, GR_THREADS, smem, st>>>(P);
+  kernel<<<grid, GR_THREADS, smem, st>>>(P);
   WWB_CHECK_LAUNCH(ctx);
   return WWB_OK;
 }
@@ -1045,8 +1083,10 @@ struct G2Params {
   int64_t n_win;
   const int32_t* n_win_dev;
   int nsplit;
+  int T;                        // steps
 };
 
+template <int kT>   // kT > 0: T fixed at compile time; 0: T = P.T
 __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Params P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   G2Smem& sm = *reinterpret_cast<G2Smem*>(smem_raw);
@@ -1054,6 +1094,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Pa
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int64_t n_win = P.n_win_dev ? (int64_t)*P.n_win_dev : P.n_win;
   const int64_t n_tiles = (n_win + 127) / 128;
+  const int T = kT > 0 ? kT : P.T;
 
   for (int i = tid; i < (int)(2 * G2_W_BYTES / 16); i += GR_THREADS)
     reinterpret_cast<uint4*>(&sm.w[0][0])[i] = reinterpret_cast<const uint4*>(P.w2)[i];
@@ -1107,7 +1148,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Pa
       float h[16];
 #pragma unroll
       for (int i = 0; i < 16; ++i) h[i] = 0.f;
-      for (int s = 0; s < GR_T; ++s, ++n_acc) {
+      for (int s = 0; s < T; ++s, ++n_acc) {
         mbar_wait(&sm.acc_full[d], n_acc & 1);
         fence_after_sync();
 #pragma unroll
@@ -1133,7 +1174,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Pa
             gru_gates2(az[i], ar[i], hh[i] + bh[u * 8 + i], xh[i], az[i + 1], ar[i + 1], hh[i + 1] + bh[u * 8 + i + 1], xh[i + 1],
                        h[u * 8 + i], h[u * 8 + i + 1]);
         }
-        if (s < GR_T - 1) {
+        if (s < T - 1) {
           uint32_t hr8[8], lr8[8];
 #pragma unroll
           for (int c = 0; c < 8; ++c) split_pair(h[2 * c], h[2 * c + 1], hr8[c], lr8[c]);
@@ -1165,13 +1206,13 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Pa
         if (lane == 0) ok = mbar_test_wait(&sm.a_empty[dd][xs], ((n_ld[dd] / G2_AST) & 1) ^ 1) ? 1u : 0u;
         if (!__shfl_sync(0xffffffffu, ok, 0)) return;
       }
-      const int t = dd ? GR_T - 1 - ld_s[dd] : ld_s[dd];
+      const int t = dd ? T - 1 - ld_s[dd] : ld_s[dd];
       if (lane == 0) {
         mbar_arrive_expect_tx(&sm.a_full[dd][xs], G2_A_BYTES);
-        bulk_g2s(sm.a[dd][xs], P.seq + (size_t)(ld_tile[dd] * GR_T + t) * G2_A_BYTES, G2_A_BYTES, &sm.a_full[dd][xs]);
+        bulk_g2s(sm.a[dd][xs], P.seq + (size_t)(ld_tile[dd] * T + t) * G2_A_BYTES, G2_A_BYTES, &sm.a_full[dd][xs]);
       }
       ++n_ld[dd];
-      if (++ld_s[dd] == GR_T) { ld_s[dd] = 0; ld_tile[dd] += gridDim.x; }
+      if (++ld_s[dd] == T) { ld_s[dd] = 0; ld_tile[dd] += gridDim.x; }
     };
     while (ld_tile[0] < n_tiles || ld_tile[1] < n_tiles) {
       const uint32_t before = n_ld[0] + n_ld[1];
@@ -1185,7 +1226,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1) gru2_fused_tc_kernel(const G2Pa
     const int nsplit = P.nsplit;
     uint32_t n_step = 0, n_h = 0;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int s = 0; s < GR_T; ++s, ++n_step) {
+      for (int s = 0; s < T; ++s, ++n_step) {
         // input projections of this step (do not depend on h): as soon as the slab is in and the accumulator has been read
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
@@ -1267,7 +1308,7 @@ std::vector<float> crnn_reorder_bias2(const float* bf) {
     for (int n = 0; n < 96; ++n) out[d * 96 + n] = bf[d * 96 + (n < 32 ? 64 + n : n - 32)];
   return out;
 }
-size_t crnn_seq_packed_bytes(int64_t B) { return (size_t)((B + 127) / 128) * GR_T * G2_A_BYTES; }
+size_t crnn_seq_packed_bytes(int64_t B, int T) { return (size_t)((B + 127) / 128) * T * G2_A_BYTES; }
 
 int gru2_fused_tc(wwb_ctx* ctx, const unsigned char* seq_packed, float* last_out, int64_t B, const int32_t* n_dev,
                   cudaStream_t st) {
@@ -1283,11 +1324,13 @@ int gru2_fused_tc(wwb_ctx* ctx, const unsigned char* seq_packed, float* last_out
   P.n_win = B;
   P.n_win_dev = n_dev;
   P.nsplit = ctx->precision == WWB_PREC_TC ? 3 : 1;
+  P.T = crnn_geom(ctx->L).T;
   const size_t smem = sizeof(G2Smem) + 128;
-  WWB_CUDA(ctx, cudaFuncSetAttribute(gru2_fused_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = P.T == CA_T_SHIPPED ? gru2_fused_tc_kernel<CA_T_SHIPPED> : gru2_fused_tc_kernel<0>;
+  WWB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int64_t n_tiles = (B + 127) / 128;
   const unsigned grid = (unsigned)std::min<int64_t>(n_tiles, (int64_t)ctx->sm_count);
-  gru2_fused_tc_kernel<<<grid, GR_THREADS, smem, st>>>(P);
+  kernel<<<grid, GR_THREADS, smem, st>>>(P);
   WWB_CHECK_LAUNCH(ctx);
   return WWB_OK;
 }

@@ -18,7 +18,8 @@ Canonical names
            sig_w[24,16,3,16] sig_b[24,16] tanh_w[24,16,3,16] tanh_b[24,16]   (out, tap, in)
            res_w[23,16,16] res_b[23,16]  skip_w[24,32,16] skip_b[24,32]
            det1_w[32,32] det1_b[32] det2_w[2,32] det2_b[2]
-  both   : mel_length[] (encoder window length in mel frames: 151 | 182)
+  both   : mel_length[] (encoder window length in mel frames, read from the encoder's input shape: CRNN 17..256,
+           shipped 151; WaveNet 17..182, shipped 182)
 """
 from __future__ import annotations
 
