@@ -160,19 +160,23 @@ int wwb_pipeline(wwb_ctx* ctx, const void* pcm_dev, int pcm_dtype, int64_t n_str
                  float* post_dev, void* stream);
 /* same through HOST buffers - the call that replaces TFLiteModel.__call__'s copy-in / invoke /
  * copy-out (spokestack/models/tensorflow.py:33-51) for a batch of streams: H2D of the PCM in
- * three slices overlapped with the kernels, D2H of the posteriors, sync.  Host buffers that
- * are not page-locked are registered on first use (cached per address range). */
+ * three slices overlapped with the kernels, D2H of the posteriors, sync.  The caller's buffers
+ * are never page-locked by the call: pageable memory takes the driver's staged copy, memory
+ * from wwb_host_alloc the overlapped one. */
 int wwb_pipeline_host(wwb_ctx* ctx, const void* pcm_host, int pcm_dtype, int64_t n_streams,
                       int64_t n_samples, float pre_emphasis, int hop, float* post_host);
 /* Asynchronous form for sweeps (utils/evaluate_models.py:280-327 runs both model types over
  * the same audio): ONE host->device copy and ONE filter pass feed n_ctx models (ctxs[0] runs
- * the filter and owns the pipeline; all ctxs on one device).  Per model m: posteriors
+ * the filter and owns the pipeline; all ctxs on one device and with the same filter fields -
+ * mel_w, mel_b, floor, offset, scale - or WWB_ERR_ARG).  Per model m: posteriors
  * post_host[m] [n_streams, n_win_m] and, if thr_host != NULL, the FAR rising-edge counts
  * (every stream one trajectory, 30-tap smoothing) and the FRR per-stream-max counts
  * (evaluate_models.py:183-218) as int64 [n_thr] each; any output pointer may be NULL.
  * Returns once the work is enqueued; up to two jobs may be in flight (the copy of job k+1
  * overlaps the kernels of job k).  wwb_sweep_wait blocks until the OLDEST job's results
- * are in host memory.  Input and output buffers must stay valid until then. */
+ * are in host memory.  Input and output buffers must stay valid until then; they are not
+ * page-locked by the call.  Every argument is checked before any copy or launch: a refused
+ * job leaves nothing enqueued. */
 int wwb_sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, int pcm_dtype,
                      int64_t n_streams, int64_t n_samples, float pre_emphasis, int hop,
                      const double* thr_host, int n_thr, float* const* post_host,

@@ -360,6 +360,9 @@ int wwb_create(int device, const wwb_weights* w, int precision, wwb_ctx** out) {
   ctx->mel_floor = w->mel_floor;
   ctx->mel_log_offset = w->mel_log_offset;
   ctx->mel_scale = w->mel_scale;
+  ctx->mel_w_host.assign(w->mel_w, w->mel_w + (size_t)kMel * kBins);
+  ctx->mel_b_host.assign(kMel, 0.f);
+  if (w->mel_b) ctx->mel_b_host.assign(w->mel_b, w->mel_b + kMel);
   int rc = build_filter_tables(ctx, w);
   if (!rc && w->kind == WWB_MODEL_CRNN) rc = build_crnn(ctx, w);
   if (!rc && w->kind == WWB_MODEL_WAVENET) rc = build_wavenet(ctx, w);

@@ -127,6 +127,7 @@ struct wwb_ctx {
   std::string tc_refused;   // why the model has no tensor-core weights (empty: it has them)
   int sm_count = 148;
   float mel_floor = 1e-5f, mel_log_offset = 0.f, mel_scale = 0.5f;
+  std::vector<float> mel_w_host, mel_b_host;   // the filter's mel_w [40][257] and mel_b [40] as given (a sweep's models share one filter pass)
   wwb::MelTables mel;
   double* hann = nullptr;      // [512] 0.5 * np.hanning(512), fp64 (fft64.cuh)
   double2* tw256 = nullptr;    // [256] W256^k

@@ -8,10 +8,10 @@
 //
 // Three CUDA streams owned by the first ctx: copy-in, compute, copy-out.  A job's PCM goes into one of two device
 // staging buffers, so the H2D copy of job k+1 runs while the kernels of job k do; a job submitted into an idle pipe
-// is cut into three slices of streams (1/8, 2/8, 5/8) so that only the first, small copy is exposed.  Host buffers
-// that are not page-locked yet are registered once (cudaHostRegister, cached per address range) - a pageable
-// cudaMemcpyAsync is staged by the driver and blocks the calling thread; wwb_host_alloc hands out pinned memory
-// directly.
+// is cut into three slices of streams (1/8, 2/8, 5/8) so that only the first, small copy is exposed.  Caller buffers
+// are never page-locked here: pageable memory takes the driver's staged copy, which blocks the calling thread, and
+// callers that want the overlapped path pass memory from wwb_host_alloc.  Registering the caller's memory would leave
+// it page-locked after the call returns, and CUDA requires it unregistered before it is freed.
 #include <stdlib.h>
 #include <string.h>
 
@@ -57,7 +57,6 @@ struct HostPipe {
   size_t seg_bytes = 0;
   std::vector<double> thr_host;        // content of `thr` (re-uploaded only when it changes)
   std::vector<int64_t> seg_key;        // (S, n_win...) the segment table was built for
-  std::vector<std::pair<char*, size_t>> registered;   // host ranges this pipe page-locked
 };
 
 static int grow(wwb_ctx* ctx, void** p, size_t* have, size_t want) {
@@ -76,31 +75,6 @@ static int grow(wwb_ctx* ctx, void** p, size_t* have, size_t want) {
   }
   *have = want;
   return WWB_OK;
-}
-
-// page-lock a caller buffer unless it already is (cudaHostAlloc / earlier registration); failure is not an error:
-// the copy then takes the driver's pageable path
-static void pin_range(HostPipe* hp, const void* p, size_t bytes) {
-  if (!p || bytes < (1u << 16)) return;
-  char* c = (char*)p;
-  for (auto& r : hp->registered)
-    if (c >= r.first && c + bytes <= r.first + r.second) return;
-  cudaPointerAttributes at;
-  if (cudaPointerGetAttributes(&at, p) == cudaSuccess && at.type != cudaMemoryTypeUnregistered) return;
-  cudaGetLastError();
-  // drop cached ranges that overlap (the caller freed and re-allocated)
-  for (size_t i = 0; i < hp->registered.size();) {
-    auto& r = hp->registered[i];
-    if (c < r.first + r.second && r.first < c + bytes) {
-      cudaHostUnregister(r.first);
-      hp->registered.erase(hp->registered.begin() + i);
-    } else {
-      ++i;
-    }
-  }
-  cudaGetLastError();
-  if (cudaHostRegister(c, bytes, cudaHostRegisterDefault) == cudaSuccess) hp->registered.push_back({c, bytes});
-  cudaGetLastError();
 }
 
 static int pipe_get(wwb_ctx* ctx, HostPipe** out) {
@@ -125,7 +99,6 @@ void host_pipe_destroy(wwb_ctx* ctx) {
   HostPipe* hp = (HostPipe*)ctx->host_pipe;
   if (!hp) return;
   cudaDeviceSynchronize();
-  for (auto& r : hp->registered) cudaHostUnregister(r.first);
   for (auto& s : hp->slot) {
     if (s.pcm) cudaFree(s.pcm);
     for (void* p : s.post) if (p) cudaFree(p);
@@ -167,8 +140,25 @@ static int sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, i
     if (!ctxs[m] || ctxs[m]->device != ctx->device) return fail(ctx, WWB_ERR_ARG, "all models of a sweep must live on one device");
     if (ctxs[m]->kind == WWB_MODEL_NONE) return fail(ctx, WWB_ERR_STATE, "ctx %d holds a filter only (no encode/detect weights)", m);
   }
+  // ONE filter pass feeds every model: they must share the filter's fields
+  for (int m = 1; m < n_ctx; ++m)
+    if (ctxs[m]->mel_w_host != ctx->mel_w_host || ctxs[m]->mel_b_host != ctx->mel_b_host ||
+        ctxs[m]->mel_floor != ctx->mel_floor || ctxs[m]->mel_log_offset != ctx->mel_log_offset ||
+        ctxs[m]->mel_scale != ctx->mel_scale)
+      return fail(ctx, WWB_ERR_ARG, "model %d has other filter fields (mel_w, mel_b, floor, offset, scale) than model 0", m);
   const bool want_counts = thr_host && n_thr > 0 && (far_host || frr_host);
   if (want_counts && n_thr > 8192) return fail(ctx, WWB_ERR_ARG, "n_thr out of range");
+  if (want_counts)
+    for (int i = 1; i < n_thr; ++i)
+      if (thr_host[i] < thr_host[i - 1]) return fail(ctx, WWB_ERR_ARG, "thresholds must be ascending");
+  const size_t esz = dtype == WWB_PCM_I16 ? 2 : 4;
+  const int64_t F = wwb_num_frames(N);
+  std::vector<int64_t> nwin(n_ctx);
+  for (int m = 0; m < n_ctx; ++m) {
+    nwin[m] = wwb_num_windows(ctxs[m], F, hop);
+    if (want_counts && far_host && far_host[m] && nwin[m] > 0 && nwin[m] < 30)
+      return fail(ctx, WWB_ERR_ARG, "FAR trajectory of %lld posteriors is shorter than the 30-tap smoothing window", (long long)nwin[m]);
+  }
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   HostPipe* hp;
   int rc = pipe_get(ctx, &hp);
@@ -176,10 +166,6 @@ static int sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, i
   if (hp->in_flight == kPipeSlots) return fail(ctx, WWB_ERR_STATE, "two jobs are in flight already: call wwb_sweep_wait first");
   const bool overlapped = hp->in_flight > 0;
   HostPipeSlot& sl = hp->slot[hp->next];
-  const size_t esz = dtype == WWB_PCM_I16 ? 2 : 4;
-  const int64_t F = wwb_num_frames(N);
-  std::vector<int64_t> nwin(n_ctx);
-  for (int m = 0; m < n_ctx; ++m) nwin[m] = wwb_num_windows(ctxs[m], F, hop);
 
   // ---- buffers ----
   if ((rc = grow(ctx, &sl.pcm, &sl.pcm_bytes, (size_t)S * N * esz))) return rc;
@@ -206,8 +192,6 @@ static int sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, i
     for (int m = 0; m < n_ctx; ++m) key.push_back(nwin[m]);
     const bool thr_same = (int)hp->thr_host.size() == n_thr && !memcmp(hp->thr_host.data(), thr_host, n_thr * sizeof(double));
     if (!thr_same || key != hp->seg_key) {
-      for (int i = 1; i < n_thr; ++i)
-        if (thr_host[i] < thr_host[i - 1]) return fail(ctx, WWB_ERR_ARG, "thresholds must be ascending");
       WWB_CUDA(ctx, cudaStreamSynchronize(hp->compute));
       if ((rc = grow(ctx, &hp->thr, &hp->thr_bytes, (size_t)n_thr * sizeof(double)))) return rc;
       if ((rc = grow(ctx, &hp->seg, &hp->seg_bytes, (size_t)n_ctx * (S + 1) * sizeof(int64_t)))) return rc;
@@ -220,9 +204,6 @@ static int sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, i
       hp->seg_key = key;
     }
   }
-  pin_range(hp, pcm_host, (size_t)S * N * esz);
-  for (int m = 0; m < n_ctx; ++m)
-    if (post_host && post_host[m]) pin_range(hp, post_host[m], (size_t)S * nwin[m] * sizeof(float));
 
   // ---- slices of streams: 1/8, 2/8, 5/8 when nothing hides the first copy, one slice otherwise ----
   int64_t bounds[4] = {0, S, S, S};
@@ -259,8 +240,6 @@ static int sweep_submit(wwb_ctx* const* ctxs, int n_ctx, const void* pcm_host, i
     for (int m = 0; m < n_ctx; ++m) {
       int64_t* c = (int64_t*)sl.counts[m];
       const int64_t* seg = (const int64_t*)hp->seg + (size_t)m * (S + 1);
-      if (nwin[m] > 0 && nwin[m] < 30 && far_host && far_host[m])
-        return fail(ctx, WWB_ERR_ARG, "FAR trajectory of %lld posteriors is shorter than the 30-tap smoothing window", (long long)nwin[m]);
       const int64_t nseg = nwin[m] > 0 ? S : 0;
       if ((rc = wwb_eval_counts(ctxs[m], (const float*)sl.post[m], seg, nseg, nullptr, nullptr, S * nwin[m], (const double*)hp->thr,
                                 n_thr, WWB_COUNT_FAR_EDGES, 30, c, hp->compute))) return rc;
