@@ -238,6 +238,19 @@ int wwb_stream_push_indexed(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids
 int wwb_stream_max_frames(const wwb_ctx* ctx);
 /* WakewordTrigger.reset (:241-246) for the streams whose mask byte is non-zero (NULL = all). */
 int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask_dev, int64_t n_streams, void* stream);
+/* Per-slot trigger options of the slots named in ids_host (id rules of wwb_stream_export); either array may be NULL
+ * (that option unchanged), not both.  threshold_host float [n_ids]: NaN = the call's threshold, any other value
+ * (+-inf too) replaces it for that slot in the strict p > threshold test.  listening_host uint8 [n_ids]: 0 or 1.
+ * A slot with listening 0 is paused on this ctx: every push and step treats it as an entry whose is_active is 1 (no
+ * samples consumed, no frame analysed, trigger 0, post_max its running maximum; the VAD fall still resets it) without
+ * changing the is_active that later stages of a chain see.  Switched back on, it continues from its retained window
+ * (reset it for a fresh start).  Defaults after wwb_stream_alloc: NaN and 1.  The options are slot configuration:
+ * wwb_stream_reset, wwb_context_reset and wwb_stream_import keep them and the state records do not carry them.
+ * Stream-ordered: a push enqueued on `stream` after this call sees the new values.  Checked before any device work
+ * (WWB_ERR_STATE: no wwb_stream_alloc, a filter-only ctx, n_ids or an id as in wwb_stream_export; WWB_ERR_ARG: NULL
+ * ids, both arrays NULL, a listening value other than 0 or 1). */
+int wwb_stream_set_options(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const float* threshold_host,
+                           const uint8_t* listening_host, void* stream);
 
 /* ---- the pipeline stages around the trigger, per stream on the device (SpeechPipeline._dispatch,
  * spokestack/pipeline.py:25-28): VAD rise/fall debounce (spokestack/vad/webrtc.py:52-77; the raw

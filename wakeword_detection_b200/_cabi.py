@@ -71,6 +71,7 @@ PROTOTYPES = {
                                           _vp]),
     "wwb_stream_max_frames": (C.c_int, [_vp]),
     "wwb_stream_reset": (C.c_int, [_vp, _vp, _i64, _vp]),
+    "wwb_stream_set_options": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),
     "wwb_context_alloc": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "wwb_context_step": (C.c_int, [_vp, _vp, _i64, _i64, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "wwb_context_step_indexed": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp, _vp, _vp,
@@ -751,6 +752,37 @@ class Engine:
             m = self._dev(np.asarray(mask), t.uint8)
             S = m.numel()
         self._check(self.lib.wwb_stream_reset(self.ctx, m.data_ptr() if m is not None else None, S, self._stream()))
+
+    def stream_set_options(self, ids, threshold=None, listening=None) -> None:
+        """Per-slot trigger options of the slots in `ids` (distinct, any order), one value per entry or one for all;
+        None leaves that option as it is.  threshold: NaN = the threshold each push or step passes, any other value
+        replaces it for the slot.  listening: 0 pauses the slot (every push treats it as is_active: nothing consumed or
+        analysed, no trigger), 1 lets it continue from its retained window.  Stream-ordered like the pushes; kept
+        across stream_reset, context_reset and stream_import, and not part of the records."""
+        ids = self._state_ids(ids)
+        thr, lst = _stream_options(ids.size, threshold, listening)
+        self._check(self.lib.wwb_stream_set_options(self.ctx, ids.ctypes.data, ids.size,
+                                                    None if thr is None else thr.ctypes.data,
+                                                    None if lst is None else lst.ctypes.data, self._stream()))
+
+
+def _stream_options(n: int, threshold=None, listening=None):
+    """threshold / listening (None, a scalar or n values) -> (float32 [n] or None, uint8 [n] or None) host arrays; a
+    wrong shape, or a listening value that is not a whole number in [0, 255], raises ValueError (the library refuses
+    values other than 0 and 1)"""
+    def per_entry(v, name):
+        a = np.asarray(v)
+        if a.ndim > 1 or (a.ndim == 1 and a.size != n):
+            raise ValueError("%s must be a scalar or %d values, got shape %s" % (name, n, list(a.shape)))
+        return np.broadcast_to(a, (n,))
+    thr = None if threshold is None else np.ascontiguousarray(per_entry(threshold, "threshold"), np.float32)
+    lst = None
+    if listening is not None:
+        v = per_entry(listening, "listening")
+        lst = np.ascontiguousarray(v, np.uint8)
+        if not np.array_equal(lst, v):
+            raise ValueError("listening values must be 0 or 1")
+    return thr, lst
 
 
 _ENGINES: Dict[Tuple, Engine] = {}

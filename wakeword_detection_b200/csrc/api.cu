@@ -551,10 +551,15 @@ int wwb_stream_alloc(wwb_ctx* ctx, int64_t max_streams, int64_t max_chunk) {
   if ((rc = dalloc(ctx, S, &s.win_slot))) return rc;
   if ((rc = dalloc(ctx, 1, &s.n_win))) return rc;
   if ((rc = dalloc(ctx, S * s.max_frames, &s.win_post))) return rc;
-  if ((rc = dalloc(ctx, 2 * S + 1, &s.tables))) return rc;
+  if ((rc = dalloc(ctx, stage_words(S), &s.tables))) return rc;
   if ((rc = dalloc(ctx, 2, &s.import_check))) return rc;
+  // slot options: every threshold a quiet NaN (all bits set: the call's threshold), every slot listening
+  if ((rc = dalloc(ctx, S, &ctx->opt.threshold))) return rc;
+  if ((rc = dalloc(ctx, S, &ctx->opt.listening))) return rc;
+  WWB_CUDA(ctx, cudaMemset(ctx->opt.threshold, 0xFF, S * sizeof(float)));
+  WWB_CUDA(ctx, cudaMemset(ctx->opt.listening, 1, S));
   for (int k = 0; k < 2; ++k) {
-    if (!ctx->stage_host[k]) WWB_CUDA(ctx, cudaHostAlloc((void**)&ctx->stage_host[k], (2 * S + 1) * sizeof(int32_t), cudaHostAllocDefault));
+    if (!ctx->stage_host[k]) WWB_CUDA(ctx, cudaHostAlloc((void**)&ctx->stage_host[k], stage_words(S) * sizeof(int32_t), cudaHostAllocDefault));
     if (!ctx->stage_done[k]) WWB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->stage_done[k], cudaEventDisableTiming));
   }
   ctx->id_seen.assign(S, 0);
@@ -642,13 +647,27 @@ static int check_tables(wwb_ctx* ctx, int64_t cap, const int32_t* ids, int64_t n
   return WWB_OK;
 }
 
-// Copies checked slot ids (and, with `len`, the chunk offsets) to st.tables on `st` through the next page-locked staging
-// slot.  Waiting only for that slot's previous copy keeps the host from blocking behind the call before.
-static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, cudaStream_t st) {
-  StreamState& s = ctx->st;
+// The next page-locked staging slot, once its previous copy has finished: waiting only for that slot keeps the host from
+// blocking behind the call before.  stage_copy sends its first n words to st.tables on `st`.
+static int stage_slot(wwb_ctx* ctx, int32_t** h) {
+  WWB_CUDA(ctx, cudaEventSynchronize(ctx->stage_done[ctx->stage_next]));
+  *h = ctx->stage_host[ctx->stage_next];
+  return WWB_OK;
+}
+
+static int stage_copy(wwb_ctx* ctx, int64_t n, cudaStream_t st) {
   const int k = ctx->stage_next;
-  WWB_CUDA(ctx, cudaEventSynchronize(ctx->stage_done[k]));
-  int32_t* h = ctx->stage_host[k];
+  WWB_CUDA(ctx, cudaMemcpyAsync(ctx->st.tables, ctx->stage_host[k], (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  WWB_CUDA(ctx, cudaEventRecord(ctx->stage_done[k], st));
+  ctx->stage_next = 1 - k;
+  return WWB_OK;
+}
+
+// Copies checked slot ids (and, with `len`, the chunk offsets) to st.tables on `st`.
+static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const int32_t* len, cudaStream_t st) {
+  int32_t* h;
+  int rc = stage_slot(ctx, &h);
+  if (rc) return rc;
   memcpy(h, ids, (size_t)n_ids * sizeof(int32_t));
   int64_t n = n_ids;
   if (len) {
@@ -660,10 +679,7 @@ static int stage_tables(wwb_ctx* ctx, const int32_t* ids, int64_t n_ids, const i
     h[2 * n_ids] = at;
     n = 2 * n_ids + 1;
   }
-  WWB_CUDA(ctx, cudaMemcpyAsync(s.tables, h, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  WWB_CUDA(ctx, cudaEventRecord(ctx->stage_done[k], st));
-  ctx->stage_next = 1 - k;
-  return WWB_OK;
+  return stage_copy(ctx, n, st);
 }
 
 // the checks of an indexed push (`pipeline`: step) in the order of check_dense
@@ -708,6 +724,28 @@ int wwb_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, void* stream)
   if (S < 1 || S > ctx->st.max_streams) return fail(ctx, WWB_ERR_STATE, "n_streams out of range");
   WWB_CUDA(ctx, cudaSetDevice(ctx->device));
   return launch_stream_reset(ctx, mask, S, (cudaStream_t)stream);
+}
+
+int wwb_stream_set_options(wwb_ctx* ctx, const int32_t* ids_host, int64_t n_ids, const float* threshold_host,
+                           const uint8_t* listening_host, void* stream) {
+  if (!ctx) return WWB_ERR_ARG;
+  int rc = check_state(ctx, false, true);
+  if (rc) return rc;
+  if (!threshold_host && !listening_host) return fail(ctx, WWB_ERR_ARG, "threshold and listening arrays both NULL");
+  const void* values = threshold_host ? (const void*)threshold_host : (const void*)listening_host;
+  if ((rc = check_tables(ctx, ctx->st.max_streams, ids_host, n_ids, nullptr, false, values))) return rc;
+  for (int64_t i = 0; listening_host && i < n_ids; ++i)
+    if (listening_host[i] > 1)
+      return fail(ctx, WWB_ERR_ARG, "listening value %d (entry %lld) is not 0 or 1", listening_host[i], (long long)i);
+  WWB_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  int32_t* h;
+  if ((rc = stage_slot(ctx, &h))) return rc;
+  memcpy(h, ids_host, (size_t)n_ids * sizeof(int32_t));
+  if (threshold_host) memcpy(h + n_ids, threshold_host, (size_t)n_ids * sizeof(float));
+  for (int64_t i = 0; listening_host && i < n_ids; ++i) h[2 * n_ids + i] = listening_host[i];
+  if ((rc = stage_copy(ctx, (listening_host ? 3 : 2) * n_ids, st))) return rc;
+  return launch_stream_options(ctx, n_ids, threshold_host != nullptr, listening_host != nullptr, st);
 }
 
 int wwb_context_alloc(wwb_ctx* ctx, int frame_width_ms, int vad_rise_delay_ms, int vad_fall_delay_ms, int min_active_ms,

@@ -92,9 +92,9 @@ struct StreamState {
   int32_t* win_slot = nullptr;  // [S] first window slot of the stream in this push
   int32_t* n_win = nullptr;     // [1]
   float* win_post = nullptr;    // [S*max_frames]
-  // tables of an indexed push of n entries (wwb_stream_push_indexed): [0, n) slot of each entry, [n, 2n] exclusive
-  // prefix sum of the chunk lengths
-  int32_t* tables = nullptr;    // [2S+1]
+  // tables of a call over n entries: [0, n) slot of each entry, then for an indexed push [n, 2n] the exclusive prefix
+  // sum of the chunk lengths, for wwb_stream_set_options [n, 2n) the thresholds' bits and [2n, 3n) the listening flags
+  int32_t* tables = nullptr;    // [stage_words(S)]
   // wwb_stream_import's check: [0] the lowest bad entry and its reason, [1] finished blocks (both 0 between calls)
   unsigned long long* import_check = nullptr;
 };
@@ -114,6 +114,17 @@ struct ContextState {
   uint8_t* e_is_speech = nullptr;    // [S] scratch: is_speech / is_active per entry of the push (context_vad_kernel)
   uint8_t* e_is_active = nullptr;
   int8_t* activated_by = nullptr;    // [S] scratch of a trigger chain: the stage that triggered so far, -1 if none
+};
+
+// words of st.tables and of each host staging slot for S slots: room for the largest table above
+inline int64_t stage_words(int64_t S) { return 3 * S + 1; }
+
+// Per-slot trigger options (wwb_stream_set_options), allocated with the stream state.  Slot configuration, not session
+// state: resets, imports and records leave them alone.  Kept out of StreamState so that the kernels that take a
+// StreamState by value and do not read the options keep their parameter layout.
+struct SlotOptions {
+  float* threshold = nullptr;   // [S] NaN: the threshold the push or step passes
+  uint8_t* listening = nullptr; // [S] 0: every push treats the slot as is_active
 };
 
 }  // namespace wwb
@@ -136,14 +147,15 @@ struct wwb_ctx {
   wwb::WavenetWeights wn;
   wwb::StreamState st;
   wwb::ContextState cs;
+  wwb::SlotOptions opt;
   // growable workspaces
   void* ws[8] = {};
   size_t ws_bytes[8] = {};
   int64_t launches = 0;
   void* debug_buf = nullptr;   // optional device buffer for kernel timeline dumps (wwb_debug_buffer)
   void* host_pipe = nullptr;   // host-buffer pipeline state (host_pipeline.cu), created on first use
-  // host side of the indexed-push tables: two page-locked staging slots laid out like st.tables, each guarded by an event
-  // recorded after its copy, and the duplicate-id marks (all 0 between calls)
+  // host side of st.tables (indexed pushes, records, slot options): two page-locked staging slots of stage_words(S)
+  // words, each guarded by an event recorded after its copy, and the duplicate-id marks (all 0 between calls)
   int32_t* stage_host[2] = {};
   cudaEvent_t stage_done[2] = {};
   int stage_next = 0;
@@ -192,6 +204,8 @@ int launch_stream_finish(wwb_ctx* ctx, int64_t S, const int32_t* ids, const uint
                          float threshold, float* post_out, int32_t* n_post_out, uint8_t* trigger_out,
                          float* post_max_out, cudaStream_t st);
 int launch_stream_reset(wwb_ctx* ctx, const uint8_t* mask, int64_t S, cudaStream_t st);
+// wwb_stream_set_options' scatter of the n entries staged in st.tables (ids, thresholds, listening flags)
+int launch_stream_options(wwb_ctx* ctx, int64_t n, bool threshold, bool listening, cudaStream_t st);
 // stream state records (stream_state.cu): ids is the device id table of n entries
 int64_t stream_state_bytes(int L);
 int launch_stream_export(wwb_ctx* ctx, const int32_t* ids, int64_t n, void* records, cudaStream_t st);

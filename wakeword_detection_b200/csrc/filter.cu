@@ -340,11 +340,21 @@ struct StreamFilterParams {
   const double2* tw256;
   const double2* tw512;
   MelParams mp;
+  SlotOptions opt;
 };
 
 __device__ __forceinline__ int stream_total_frames(int total) { return total >= kFFT ? (total - kFFT) / kHop + 1 : 0; }
 
 __device__ __forceinline__ int64_t entry_slot(const int32_t* ids, int64_t i) { return ids ? (int64_t)ids[i] : i; }
+
+// entry i (slot s) skips this push as an active stream does ("if not context.is_active: self._sample(...)", :139-140):
+// its is_active flag is set or its slot is paused on this ctx (wwb_stream_set_options).  Both flags are read
+// unconditionally, so that the two loads are in flight together.
+__device__ __forceinline__ bool entry_active(const uint8_t* is_active, const SlotOptions& opt, int64_t i, int64_t s) {
+  const bool active = is_active ? is_active[i] != 0 : false;
+  const bool listening = opt.listening[s] != 0;
+  return active | !listening;
+}
 
 // entry i's chunk and its length
 __device__ __forceinline__ const int16_t* entry_chunk(const StreamFilterParams& P, int64_t i, int& n) {
@@ -363,7 +373,7 @@ __global__ void __launch_bounds__(128) stream_plan_kernel(const StreamFilterPara
   if (i >= P.n_streams) return;
   const int64_t s = entry_slot(P.ids, i);
   int n_new = 0;
-  const bool active = P.is_active && P.is_active[i];   // "if not context.is_active: self._sample(...)" (:139-140)
+  const bool active = entry_active(P.is_active, P.opt, i, s);
   const bool speech = P.is_speech ? (P.is_speech[i] != 0) : true;
   if (!active && speech) {
     int n;
@@ -446,8 +456,8 @@ __global__ void __launch_bounds__(128) stream_tail_kernel(const StreamFilterPara
   const StreamState& S = P.st;
   const int64_t i = blockIdx.x;
   const int tid = threadIdx.x;
-  if (P.is_active && P.is_active[i]) return;
   const int64_t s = entry_slot(P.ids, i);
+  if (entry_active(P.is_active, P.opt, i, s)) return;
   int n;
   const int16_t* chunk = entry_chunk(P, i, n);
   const int np = S.n_pending[s];
@@ -497,6 +507,7 @@ struct StreamFinishParams {
   uint8_t* trigger_out;   // [entries]
   float* post_max_out;    // [entries]
   int64_t n_streams;      // entries
+  SlotOptions opt;
 };
 
 __global__ void stream_finish_kernel(const StreamFinishParams P) {
@@ -510,13 +521,15 @@ __global__ void stream_finish_kernel(const StreamFinishParams P) {
     const int slot = n > 0 ? S.win_slot[i] : 0;
     float pm = S.post_max[s];
     bool trig = false;
-    const bool active = P.is_active && P.is_active[i];
+    const bool active = entry_active(P.is_active, P.opt, i, s);
+    const float slot_thr = P.opt.threshold[s];
+    const float thr = isnan(slot_thr) ? P.threshold : slot_thr;
     for (int q = 0; q < S.max_frames; ++q) {
       float p = nanf("");
       if (q < n) {
         p = S.win_post[slot + q];
         if (p > pm) pm = p;
-        if (p > P.threshold && !active) trig = true;
+        if (p > thr && !active) trig = true;
       }
       if (P.post_out) P.post_out[i * S.max_frames + q] = p;
     }
@@ -550,6 +563,16 @@ __global__ void stream_reset_kernel(StreamState S, const uint8_t* mask, int64_t 
     S.ring_head[s] = 0;
     S.post_max[s] = 0.0f;
   }
+}
+
+// wwb_stream_set_options: entry i of the staged table (layout at StreamState::tables) into slot tab[i], one thread each
+__global__ void stream_options_kernel(SlotOptions O, const int32_t* __restrict__ tab, int64_t n, bool threshold,
+                                      bool listening) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int32_t s = tab[i];
+  if (threshold) O.threshold[s] = __int_as_float(tab[n + i]);
+  if (listening) O.listening[s] = (uint8_t)tab[2 * n + i];
 }
 
 // filter.tflite on magnitudes: one thread per (frame, band)
@@ -590,6 +613,7 @@ int launch_stream_filter(wwb_ctx* ctx, const int16_t* pcm, int64_t S, int64_t n,
   P.st = ctx->st; P.L = ctx->L;
   P.hann_half = ctx->hann; P.tw256 = ctx->tw256; P.tw512 = ctx->tw512;
   P.mp = mel_params(ctx);
+  P.opt = ctx->opt;
   WWB_CUDA(ctx, cudaMemsetAsync(ctx->st.n_win, 0, sizeof(int32_t), st));
   stream_plan_kernel<<<(unsigned)((S + 127) / 128), 128, 0, st>>>(P);
   WWB_CHECK_LAUNCH(ctx);
@@ -610,8 +634,14 @@ int launch_stream_finish(wwb_ctx* ctx, int64_t S, const int32_t* ids, const uint
   StreamFinishParams P;
   P.st = ctx->st; P.L = ctx->L; P.ids = ids; P.is_speech = is_speech; P.is_active = is_active;
   P.threshold = threshold; P.post_out = post_out; P.n_post_out = n_post_out;
-  P.trigger_out = trigger_out; P.post_max_out = post_max_out; P.n_streams = S;
+  P.trigger_out = trigger_out; P.post_max_out = post_max_out; P.n_streams = S; P.opt = ctx->opt;
   stream_finish_kernel<<<(unsigned)S, 128, 0, st>>>(P);
+  WWB_CHECK_LAUNCH(ctx);
+  return WWB_OK;
+}
+
+int launch_stream_options(wwb_ctx* ctx, int64_t n, bool threshold, bool listening, cudaStream_t st) {
+  stream_options_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(ctx->opt, ctx->st.tables, n, threshold, listening);
   WWB_CHECK_LAUNCH(ctx);
   return WWB_OK;
 }

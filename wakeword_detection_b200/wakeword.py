@@ -46,7 +46,12 @@ class MultiStreamTrigger:
 
     export_streams(ids) -> uint8 device tensor [n_ids, record bytes]: the state of those slots, one record each.
     import_streams(ids, records) puts such records (from any context of the same model, any device) into the slots in
-    `ids`: to park and resume a session, move it to another slot, context or GPU, or rewind it."""
+    `ids`: to park and resume a session, move it to another slot, context or GPU, or rewind it.
+
+    set_stream_options(ids, threshold, listening) sets per-slot options, one value per entry of `ids` or one for all:
+    a threshold that replaces posterior_threshold for that slot (NaN: back to posterior_threshold), and listening 0 to
+    pause a slot (its pushes are treated as is_active: nothing is consumed or analysed) or 1 to resume it from its
+    retained window.  Resets and imports keep the options."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, chunk_samples: int = 320,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, device: int = 0,
@@ -75,6 +80,9 @@ class MultiStreamTrigger:
     def import_streams(self, ids, records) -> None:
         self.engine.stream_import(ids, records)
 
+    def set_stream_options(self, ids, threshold=None, listening=None) -> None:
+        self.engine.stream_set_options(ids, threshold, listening)
+
     def reset(self, mask=None) -> None:
         self.engine.stream_reset(mask)
 
@@ -91,8 +99,8 @@ class MultiStreamPipeline:
     step(pcm[S, n] int16, vad_raw[S]) -> dict of device tensors: post, n_post, post_max, is_speech, is_active,
     activated, deactivated.  step_streams(ids, frames, vad_raw) dispatches only the slots in `ids`, each with its own
     frame (list of 1-D int16 arrays or tensors); same dict, one row per entry of `ids`.  export_streams /
-    import_streams as on MultiStreamTrigger; the records carry the VAD debounce and ActivationTimeout state too (the
-    delays are the context's own)."""
+    import_streams and set_stream_options as on MultiStreamTrigger; the records carry the VAD debounce and
+    ActivationTimeout state too (the delays are the context's own).  A paused slot's VAD debounce and timeout go on."""
 
     def __init__(self, model_dir: str, model_type: str, n_streams: int, frame_width: int = 20, sample_rate: int = 16000,
                  pre_emphasis: float = 0.0, posterior_threshold: float = 0.5, vad_rise_delay: int = 0,
@@ -120,6 +128,9 @@ class MultiStreamPipeline:
     def import_streams(self, ids, records) -> None:
         self.engine.stream_import(ids, records)
 
+    def set_stream_options(self, ids, threshold=None, listening=None) -> None:
+        self.engine.stream_set_options(ids, threshold, listening)
+
     def reset(self) -> None:
         self.engine.context_reset()
 
@@ -138,7 +149,11 @@ class MultiWakewordPipeline:
     step(pcm[S, n] int16, vad_raw[S]) / step_streams(ids, frames, vad_raw) -> the dict of MultiStreamPipeline with post
     [K, S, max_frames], n_post [K, S] and post_max [K, S] per stage, plus activated_by [S] (int8: the stage that
     triggered, -1 if none).  export_streams(ids) -> one record tensor per stage (stage 0's carries the pipeline state);
-    import_streams(ids, records) puts them back, all or nothing across the stages."""
+    import_streams(ids, records) puts them back, all or nothing across the stages.
+
+    set_stream_options(ids, threshold, listening) sets the options of MultiStreamTrigger per slot and stage: arrays
+    [n_ids, K], or [n_ids] / a scalar for every stage.  A slot that listens to stage k only runs no encoder windows in
+    the other stages, and a paused stage does not change the is_active that later stages see."""
 
     def __init__(self, models, n_streams: int, frame_width: int = 20, sample_rate: int = 16000, vad_rise_delay: int = 0,
                  vad_fall_delay: int = 0, min_active: int = 500, max_active: int = 5000, device: int = 0,
@@ -175,6 +190,32 @@ class MultiWakewordPipeline:
 
     def import_streams(self, ids, records) -> None:
         self.engines[0].stream_import_chain(self.engines[1:], ids, records)
+
+    def set_stream_options(self, ids, threshold=None, listening=None) -> None:
+        ids = np.ascontiguousarray(ids, np.int32)
+        if ids.ndim != 1:
+            raise ValueError("ids must be 1-D")
+        K = len(self.engines)
+
+        def per_stage(v, name):
+            """None, a scalar, [n_ids] or [n_ids, K] -> the K stages' values"""
+            if v is None:
+                return [None] * K
+            a = np.asarray(v)
+            if a.ndim == 1:
+                a = a[:, None]
+            if a.ndim > 2 or (a.ndim == 2 and a.shape not in ((ids.size, K), (ids.size, 1))):
+                raise ValueError("%s must be a scalar, [%d] or [%d, %d], got shape %s"
+                                 % (name, ids.size, ids.size, K, list(np.shape(v))))
+            return [np.broadcast_to(a, (ids.size, K))[:, k] for k in range(K)]
+
+        # every stage's values are checked before the first stage's call: a bad argument cannot apply to some stages only
+        opts = [_cabi._stream_options(ids.size, t, l)
+                for t, l in zip(per_stage(threshold, "threshold"), per_stage(listening, "listening"))]
+        if any(l is not None and (l > 1).any() for _, l in opts):
+            raise ValueError("listening values must be 0 or 1")
+        for e, (t, l) in zip(self.engines, opts):
+            e.stream_set_options(ids, t, l)
 
     def reset(self) -> None:
         self.engines[0].context_reset()
